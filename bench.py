@@ -3,6 +3,7 @@
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W   (CPU arm: the oracle port on the host cores)
     python bench.py --config {1,2,3,4,5} ...                  (3 = default = the driver's line; see CONFIGS below)
+    python bench.py ... --dump-outputs DIR                   (+ what the last timed step returned, as DIR/<name>.npy)
 
 One step = one pass of the FULL hot path over one slab of synthetic input per GPU:
   stage 1  genotype application + reverse complement + BPE-500 for B x C CRE windows and B gene windows
@@ -38,6 +39,34 @@ os.dup2(2, 1)
 def emit(obj):
     _RESULT_OUT.write(json.dumps(obj) + "\n")
     _RESULT_OUT.flush()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write what the timed path handed its caller in its last step as out_dir/<name>.npy, so that two builds run with
+    the same arguments (hence the same seeded inputs) can be compared output for output.  float64 stays float64, every
+    other dtype is written as float32.  Above DUMP_LIMIT_BYTES in all, every array keeps the same share of its rows,
+    drawn with a fixed seed from its row count alone: arrays with as many rows (pred and emb) keep the same rows."""
+    import torch
+    host = {}
+    for name, a in arrays.items():
+        if torch.is_tensor(a):
+            a = a.detach().cpu()
+            a = a.numpy() if a.dtype == torch.float64 else a.float().numpy()
+        a = np.asarray(a)
+        host[name] = a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        share = DUMP_LIMIT_BYTES / total
+        for name, a in host.items():
+            if a.ndim and a.shape[0] > 1:
+                rows = np.random.default_rng(0).choice(a.shape[0], max(1, int(a.shape[0] * share)), replace=False)
+                host[name] = a[np.sort(rows)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -210,6 +239,8 @@ def run_reference(args):
         r = cpu_sample(sd, cfg, hp, chroms, var, gene, args.cre, CPU_SAMPLE_TISSUES[i % len(CPU_SAMPLE_TISSUES)])
         pts.append((r["T"], r["t_model"])); s1.append(r["t_stage1"])
     t_timed = time.perf_counter() - t_timed
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pred": r["pred"], "emb": r["emb"]})
     fit_pts = list(pts)
     if len({p[0] for p in fit_pts}) < 2:                     # one tissue count cannot separate base from marginal cost
         fit_pts += warm[-1:] if warm else [(lambda r: (r["T"], r["t_model"]))(
@@ -308,15 +339,17 @@ class Bench:
         -> (milliseconds, fn's result, kernel launches, clocks sampled under load)."""
         torch = self.torch
         sampler = ClockSampler(self.local); sampler.start()
-        n0 = self.ops.launch_count()                      # counted inside libvf_b200.so (vf_launch_count)
-        self.barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        res = fn()
-        e1.record()
-        self.barrier()
-        ms = self.max_over_ranks(e0.elapsed_time(e1))
-        self.last_clocks = sampler.stop()
+        try:                                              # a failing step must not leave nvidia-smi running
+            n0 = self.ops.launch_count()                  # counted inside libvf_b200.so (vf_launch_count)
+            self.barrier()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            res = fn()
+            e1.record()
+            self.barrier()
+            ms = self.max_over_ranks(e0.elapsed_time(e1))
+        finally:
+            self.last_clocks = sampler.stop()
         return ms, res, self.ops.launch_count() - n0, self.last_clocks
 
     def time_wall(self, fn):
@@ -473,6 +506,8 @@ def run_config3(args):
     elapsed_ms, (pred, emb, err), launches, clocks = b.time_device(lambda: run_steps(args.steps, False))
     assert int(err.item()) == 0, "stage-1 kernel flagged an error"
     assert bool(torch.isfinite(pred).all()) and bool(torch.isfinite(emb).all()), "non-finite outputs"
+    if args.dump_outputs and b.rank == 0:
+        dump_outputs(args.dump_outputs, {"pred": pred, "emb": emb})
     value = b.world * preds_per_step * args.steps / (elapsed_ms / 1e3)
     # ---- end-to-end leg: host window tables in, numpy results out, every step ----
     e2e_s, (p_np, e_np) = b.time_wall(lambda: run_steps(args.steps, True))
@@ -566,6 +601,8 @@ def run_config2(args):
     steps_resident(args.warmup)
     ms, pooled, launches, clocks = b.time_device(lambda: steps_resident(args.steps))
     assert bool(torch.isfinite(pooled.float()).all())
+    if args.dump_outputs and b.rank == 0:
+        dump_outputs(args.dump_outputs, {"pooled": pooled})
     value = b.world * n * args.steps / (ms / 1e3)
     e2e_s, pooled_h = b.time_wall(lambda: steps_e2e(args.steps))
     out = b.line(value, ms / args.steps, b.world * n * args.steps / e2e_s, n * 16 + n * 9, pooled_h.numel() * 2 + 4 * n,
@@ -661,6 +698,9 @@ def run_config4(args):
     steps_resident(min(args.warmup, 3))
     ms, res, launches, clocks = b.time_device(lambda: steps_resident(args.steps))
     assert all(np.isfinite(np.asarray(r["pred_gene_exp"])).all() for r in res)
+    if args.dump_outputs and b.rank == 0:                  # per pair: [ref, het, hom] stacked on the first axis
+        dump_outputs(args.dump_outputs, {f"pair{i}_{k}": np.stack(r[k]) for i, r in enumerate(res)
+                                         for k in ("pred_gene_exp", "embd", "gene_token_embedding", "cre_token_embedding")})
     value = b.world * P * args.steps / (ms / 1e3)
     e2e_s, res = b.time_wall(lambda: steps_e2e(args.steps))
     d2h = sum(np.asarray(r[k]).nbytes for r in res for k in ("pred_gene_exp", "embd", "gene_token_embedding",
@@ -768,6 +808,8 @@ def run_config5(args):
         all_ms = [t]
     all_ms = [float(x.item()) for x in all_ms]
     ms, (gp, ge, _), launches, clocks = b.time_device(lambda: [job() for _ in range(args.steps)][-1])
+    if args.dump_outputs and b.rank == 0:
+        dump_outputs(args.dump_outputs, {"pred": gp, "emb": ge})
     total_preds = sum(rows)
     value = total_preds * args.steps / (ms / 1e3)
     e2e_s, (hp_, he_) = b.time_wall(lambda: [(lambda r: (r[0].cpu().numpy(), r[1].cpu().numpy()))(job())
@@ -822,7 +864,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gather-check", action="store_true")
     ap.add_argument("--layers", type=int, default=25, help="debug only: seq2gene depth (25 = the benchmark)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (rank 0) as "
+                    "DIR/<name>.npy, float32 / float64, at most 64 MB in all (a fixed, seeded sample of rows beyond)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)

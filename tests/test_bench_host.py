@@ -1,4 +1,5 @@
-"""Host-side arithmetic of bench.py (no GPU, no model): the CPU arm's cost line and the per-config metric table."""
+"""Host-side arithmetic of bench.py (no GPU, no model): the CPU arm's cost line, the per-config metric table and the
+output dump."""
 import numpy as np
 
 import bench
@@ -26,6 +27,27 @@ def test_a_single_tissue_count_does_not_pretend_to_know_the_base_cost():
     assert base == 0.0 and abs(marginal - 8.0) < 1e-12
     rate2, _, _ = bench.fit_rate([(1, 8.0), (2, 11.0)], stage1_s=0.0, T=63)
     assert rate2 > 2 * rate1
+
+
+def test_dump_outputs_writes_float_arrays_and_a_seeded_row_sample_above_the_cap(tmp_path, monkeypatch):
+    import torch
+    pred = torch.arange(100, dtype=torch.float32)
+    emb = torch.arange(100 * 8, dtype=torch.float32).view(100, 8).bfloat16()      # bf16 has no numpy dtype
+    bench.dump_outputs(str(tmp_path / "all"), {"pred": pred, "emb": emb, "f64": np.ones(3)})
+    got = {k: np.load(tmp_path / "all" / f"{k}.npy") for k in ("pred", "emb", "f64")}
+    assert got["pred"].dtype == np.float32 and got["emb"].dtype == np.float32 and got["f64"].dtype == np.float64
+    assert (got["pred"] == pred.numpy()).all() and (got["emb"] == emb.float().numpy()).all()
+
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 1800)                          # 3600 bytes in all -> half the rows
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"pred": pred, "emb": emb})
+    a = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in ("pred", "emb")}
+    b = {k: np.load(tmp_path / "b" / f"{k}.npy") for k in ("pred", "emb")}
+    assert sum(x.nbytes for x in a.values()) <= 1800
+    assert a["pred"].shape == (50,) and a["emb"].shape == (50, 8)
+    rows = a["pred"].astype(int)                                                  # pred[i] == i: the rows it kept
+    assert (np.diff(rows) > 0).all() and (a["emb"] == emb.float().numpy()[rows]).all()
+    assert all((a[k] == b[k]).all() for k in a)
 
 
 def test_every_config_has_a_metric_and_unit():
