@@ -187,6 +187,19 @@ int vf_encode_windows(const uint8_t* genome, const int64_t* win_base, const int3
                       const uint8_t* alt_pool, int n_win, int max_window, uint8_t* out, int64_t pitch, int32_t* out_len,
                       int32_t* err, void* stream);
 /*
+ * Single-base substitution of encoded windows (in-silico saturation mutagenesis): row r of out = the source row
+ * src[row_src[r]] (src_len[row_src[r]] bytes, as vf_encode_windows wrote it) with ONE base replaced by row_base[r].
+ * row_off[r] = forward-strand offset pos0 - w0 of the base; flags[r] bit0 = the source was reverse-complemented: the base
+ * goes to len - 1 - row_off[r] as its IUPAC complement (the table vf_encode_windows applies).  The caller passes the
+ * base of the datasets/vepdataset.py:94-131 rule: the ALT base (hom) or get_iupac_code(ref, alt) (het).
+ * out: uint8 [n_rows, out_pitch]; out_len int32 [n_rows]; err: device int32 flag (1 row longer than a pitch, 3 offset
+ * outside the row; such a row gets length 0).  Pitches: multiples of 16, rows 16-byte aligned; n_rows <= 65535.
+ * The rows then go through vf_bpe_tokenize like any encoded window.
+ */
+int vf_mutate_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
+                      const int32_t* row_off, const uint8_t* row_base, const uint8_t* flags, int n_rows, uint8_t* out,
+                      int64_t out_pitch, int32_t* out_len, int32_t* err, void* stream);
+/*
  * BPE tokenisation of n_win byte sequences (upper-cased; non-IUPAC characters split words).
  * merge_a/merge_b/merge_new: uint16 [n_merges] rank-ordered merge table.  merge_batch: uint16 [n_merges] nondecreasing
  * batch ids, or NULL: consecutive ranks with one id are applied in a single sweep with a single barrier — legal when

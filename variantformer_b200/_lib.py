@@ -45,6 +45,7 @@ SIGNATURES = {
     "vf_cast_f32_to_bf16": ([_vp, _vp, _sz, _vp], _i32),
     "vf_forest_predict": ([_vp, _i32, _i32, _i32] + [_vp] * 9 + [_i32, _vp, _vp], _i32),
     "vf_encode_windows": ([_vp] * 13 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
+    "vf_mutate_windows": ([_vp, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
     "vf_bpe_tokenize": ([_vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _i64,
                          _i32, _vp], _i32),
 }

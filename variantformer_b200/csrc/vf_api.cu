@@ -116,6 +116,12 @@ int vf_encode_windows(const uint8_t* genome, const int64_t* win_base, const int3
     return encode_windows(genome, win_base, w0, w1, var_lo, var_hi, flags, v_pos, v_ref_len, v_alt_off, v_alt_len,
                           v_gt, alt_pool, n_win, max_window, out, pitch, out_len, err, ST(stream));
 }
+int vf_mutate_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
+                      const int32_t* row_off, const uint8_t* row_base, const uint8_t* flags, int n_rows, uint8_t* out,
+                      int64_t out_pitch, int32_t* out_len, int32_t* err, void* stream) {
+    return mutate_windows(src, src_pitch, src_len, row_src, row_off, row_base, flags, n_rows, out, out_pitch, out_len, err,
+                          ST(stream));
+}
 int vf_bpe_tokenize(const uint8_t* seq, int64_t pitch, const int32_t* len, int n_win, int max_len,
                     const uint16_t* merge_a, const uint16_t* merge_b, const uint16_t* merge_new,
                     const uint16_t* merge_batch, int n_merges, uint16_t* scratch, int64_t scratch_pitch, int32_t* out_tokens, int out_pitch, int out_cap,

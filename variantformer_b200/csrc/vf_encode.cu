@@ -148,6 +148,78 @@ int encode_windows(const uint8_t* genome, const int64_t* win_base, const int32_t
 }
 
 // ---------------------------------------------------------------------------------
+// mutate_windows: an encoded window with ONE base replaced (saturation mutagenesis).  Row r of `out` is the source row
+// src[row_src[r]] with the base at forward-strand offset row_off[r] set to row_base[r]; a reverse-complemented source
+// (flags bit 0) gets it at len - 1 - off as its complement, with the table encode_windows uses (comp_base).
+// One CTA per (row, 16 KB slice), 16-byte loads and stores: pure copy bandwidth.
+// ---------------------------------------------------------------------------------
+constexpr int kMutSlice = 16384;
+
+struct MutateParams {
+    const uint8_t* src; int64_t src_pitch; const int32_t* src_len;
+    const int32_t* row_src; const int32_t* row_off; const uint8_t* row_base; const uint8_t* flags;
+    uint8_t* out; int64_t out_pitch; int32_t* out_len; int32_t* err;
+};
+
+__global__ void __launch_bounds__(256)
+mutate_windows_kernel(const MutateParams p) {
+    const int r = blockIdx.y;
+    const int sr = p.row_src[r];
+    const int len = p.src_len[sr];
+    const int off = p.row_off[r];
+    // a row that cannot be built writes nothing but a zero length (and the error flag): the tokenizer then sees an
+    // empty window and never reads the unwritten row
+    const bool bad_len = len < 0 || (int64_t)len > p.out_pitch || (int64_t)len > p.src_pitch;
+    const bool bad_off = off < 0 || off >= len;
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        if (bad_len) atomicMax(p.err, 1);
+        else if (bad_off) atomicMax(p.err, 3);
+        p.out_len[r] = (bad_len || bad_off) ? 0 : len;
+    }
+    if (bad_len || bad_off) return;
+    const int b0 = blockIdx.x * kMutSlice;
+    if (b0 >= len) return;
+    const int b1 = min(len, b0 + kMutSlice);
+    const bool rc = p.flags[r] & 1;
+    const int q = rc ? len - 1 - off : off;                   // where the base lands in the stored (strand-oriented) row
+    const uint8_t base = rc ? comp_base(p.row_base[r]) : p.row_base[r];
+    const uint4* s4 = reinterpret_cast<const uint4*>(p.src + (size_t)sr * p.src_pitch);
+    uint4* o4 = reinterpret_cast<uint4*>(p.out + (size_t)r * p.out_pitch);
+    // whole 16-byte groups up to the one holding the last byte: both pitches are multiples of 16 (host check), so the
+    // last group stays inside both rows; bytes past len are copied as they are (they are never read)
+    const int g0 = b0 >> 4, g1 = (b1 + 15) >> 4;
+    for (int g = g0 + threadIdx.x; g < g1; g += blockDim.x) {
+        uint4 v = s4[g];
+        if (g == (q >> 4)) {                                  // byte q & 15 of the group (selects: no local memory)
+            const int word = (q >> 2) & 3, sh = (q & 3) * 8;
+            const uint32_t keep = ~(0xFFu << sh), put = (uint32_t)base << sh;
+            v.x = word == 0 ? (v.x & keep) | put : v.x;
+            v.y = word == 1 ? (v.y & keep) | put : v.y;
+            v.z = word == 2 ? (v.z & keep) | put : v.z;
+            v.w = word == 3 ? (v.w & keep) | put : v.w;
+        }
+        o4[g] = v;
+    }
+}
+
+int mutate_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
+                   const int32_t* row_off, const uint8_t* row_base, const uint8_t* flags, int n_rows, uint8_t* out,
+                   int64_t out_pitch, int32_t* out_len, int32_t* err, cudaStream_t s) {
+    if (n_rows == 0) return 0;
+    VF_REQUIRE(src_pitch > 0 && src_pitch % 16 == 0 && out_pitch > 0 && out_pitch % 16 == 0,
+               "mutate_windows: pitches must be positive multiples of 16 (src %lld, out %lld)", (long long)src_pitch,
+               (long long)out_pitch);
+    VF_REQUIRE(((uintptr_t)src & 15) == 0 && ((uintptr_t)out & 15) == 0, "mutate_windows: rows must be 16-byte aligned");
+    VF_REQUIRE(n_rows <= 65535, "mutate_windows: %d rows in one call (at most 65535)", n_rows);
+    const int64_t span = src_pitch < out_pitch ? src_pitch : out_pitch;   // longest row that can be valid
+    MutateParams p{src, src_pitch, src_len, row_src, row_off, row_base, flags, out, out_pitch, out_len, err};
+    dim3 grid((unsigned)((span + kMutSlice - 1) / kMutSlice), n_rows);
+    mutate_windows_kernel<<<grid, 256, 0, s>>>(p);
+    VF_LAUNCH_OK("mutate_windows_kernel launch");
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------
 // BPE-500 tokenisation by ascending-rank sweeps in the base-position domain.
 //
 // HF tokenizers merges the globally lowest-ranked adjacent pair first (leftmost first among

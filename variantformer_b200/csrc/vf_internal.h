@@ -48,6 +48,9 @@ int encode_windows(const uint8_t* genome, const int64_t* win_base, const int32_t
                    const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len, const uint8_t* v_gt,
                    const uint8_t* alt_pool, int n_win, int max_window, uint8_t* out, int64_t pitch, int32_t* out_len,
                    int32_t* err, cudaStream_t s);
+int mutate_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
+                   const int32_t* row_off, const uint8_t* row_base, const uint8_t* flags, int n_rows, uint8_t* out,
+                   int64_t out_pitch, int32_t* out_len, int32_t* err, cudaStream_t s);
 int bpe_tokenize(const uint8_t* seq, int64_t pitch, const int32_t* len, int n_win, int max_len,
                  const uint16_t* merge_a, const uint16_t* merge_b, const uint16_t* merge_new,
                  const uint16_t* merge_batch, int n_merges, uint16_t* scratch, int64_t scratch_pitch, int32_t* out_tokens, int out_pitch, int out_cap,

@@ -52,6 +52,34 @@ def get_iupac_code(ref: str, alt: str) -> str:
     return _IUPAC.get(ref + alt, "N")
 
 
+def cre_windows(gene: GeneSpec, nb: int):
+    """-> (order, windows): the gene's CRE rows in batch order (by start, descending on the minus strand) and their
+    [w0, w1) windows."""
+    order = np.argsort(gene.cre_start, kind="stable")
+    order = order[::-1] if gene.strand == "-" else order
+    return order, [cre_window(gene.cre_start[i], gene.cre_end[i], nb) for i in order]
+
+
+def window_hits(wins, minus: bool, pos: int, g0: int, g1: int):
+    """Which windows a variant at 1-based `pos` changes -> (hits, cre_hit, unreached, gene_hit).
+
+    Overlap tests use 1-based pos against 0-based half-open windows: start < pos <= end.  The reference walks the rows
+    in batch order with no break after a hit (vepdataset.py:367-407): EVERY overlapping window it reaches gets the
+    variant (`hits`), cre_token_position is the LAST of them (`cre_hit`, None without a hit), and the walk stops early
+    at the first row that starts past the variant (+ strand) / ends before it (- strand, rows descending).  Windows
+    containing the variant that the early break never reached (`unreached`) keep their background sequence.
+    `gene_hit`: g0 < pos <= g1."""
+    hits = []
+    for k, (a, b) in enumerate(wins):
+        if (not minus and a > pos) or (minus and b < pos):
+            break
+        if a < pos <= b:
+            hits.append(k)
+    cre_hit = hits[-1] if hits else None
+    unreached = [k for k, (a, b) in enumerate(wins) if a < pos <= b and k not in hits]
+    return hits, cre_hit, unreached, g0 < pos <= g1
+
+
 class VEPBatchBuilder:
     def __init__(self, genome: Genome, device="cuda", max_length=200, context_window=200, cre_neighbour_hood=50,
                  gene_upstream_neighbour_hood=1000, gene_downstream_neighbour_hood=300000):
@@ -84,24 +112,9 @@ class VEPBatchBuilder:
         """-> the reference's VEP batch dict (3 samples: ref, het, hom) with device tensors, or the empty
         "No overlap" batch.  `background` = per-chromosome variant arrays of a sample (ingest.load_vcf_sample)."""
         minus = gene.strand == "-"
-        order = np.argsort(gene.cre_start, kind="stable")
-        order = order[::-1] if minus else order
-        wins = [cre_window(gene.cre_start[i], gene.cre_end[i], self.nb) for i in order]
+        order, wins = cre_windows(gene, self.nb)
         g0, g1 = gene_window(gene.start, gene.end, gene.strand, self.up, self.down)
-        # overlap tests use 1-based pos against 0-based half-open windows: start < pos <= end
-        # The reference walks the rows in batch order with no break after a hit (vepdataset.py:367-407): EVERY
-        # overlapping window it reaches gets the variant, cre_token_position is the LAST of them, and the walk stops
-        # early at the first row that starts past the variant (+ strand) / ends before it (- strand, rows descending).
-        hits = []
-        for k, (a, b) in enumerate(wins):
-            if (not minus and a > variant.pos) or (minus and b < variant.pos):
-                break
-            if a < variant.pos <= b:
-                hits.append(k)
-        cre_hit = hits[-1] if hits else None
-        # windows containing the variant that the early break never reached keep their background sequence
-        unreached = [k for k, (a, b) in enumerate(wins) if a < variant.pos <= b and k not in hits]
-        gene_hit = g0 < variant.pos <= g1
+        _, cre_hit, unreached, gene_hit = window_hits(wins, minus, variant.pos, g0, g1)
         if cre_hit is None and not gene_hit:
             return {k: [] for k in ("cre_sequences", "cre_attention_masks", "tissue_context", "labels", "ref_labels",
                                     "gene_expression", "strand", "gene_embeddings", "gene_attention_masks")} | \

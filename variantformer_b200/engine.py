@@ -357,8 +357,6 @@ class Engine:
         dev = self.device
         B = len(cre_tokens)
         C = np.array([t.shape[0] for t in cre_tokens]); G = np.array([t.shape[0] for t in gene_tokens])
-        T = np.array([len(t) for t in tissues])
-        up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev, non_blocking=True)
 
         def stage(tok_list, mask_list, known):
             tok = torch.cat([t.reshape(-1, t.shape[-1]) for t in tok_list]).to(torch.int32)
@@ -369,18 +367,43 @@ class Engine:
             ln = known if known is not None else (msk == 0).sum(1).numpy().astype(np.int64)
             return tok.pin_memory().to(dev, non_blocking=True), msk.pin_memory().to(dev, non_blocking=True), ln
 
-        s = {"B": B, "C": C, "G": G, "T": T}
+        s = {}
         s["ctok"], s["cmsk"], s["clens"] = stage(cre_tokens, cre_masks, None if lens is None else lens[0])
         s["gtok"], s["gmsk"], s["glens"] = stage(gene_tokens, gene_masks, None if lens is None else lens[1])
         for tag, ln, W in (("c", s["clens"], self.cre_tok), ("g", s["glens"], self.gene_tok)):
             s[tag + "_cu_tok"] = ops.cu_seqlens(ln, dev)
             s[tag + "_plan_tok"] = AttnPlan(ln, dev, W.hd)
-        # gene stream layout: per (gene, tissue): [registry(tissue); the gene's chunk embeddings]
         g_off = np.concatenate([[0], np.cumsum(G)])
+        gene_rows = [np.arange(g_off[g], g_off[g + 1], dtype=np.int64) for g in range(B)]
+        return self._prepare_seq2gene(s, C, gene_rows, int(G.sum()), tissues, ref_labels, cre_token_position,
+                                      gene_token_position)
+
+    def prepare_shared(self, cre_rows, gene_rows, n_gene_chunks, tissues, ref_labels):
+        """Slab of items whose windows are encoded once and shared between items (saturation mutagenesis: every
+        mutant of a gene reuses the reference item's unchanged windows).  cre_rows / gene_rows: one int array per item,
+        the rows of the item's CRE windows / gene chunks (in batch order) in the pooled outputs of the unique windows;
+        n_gene_chunks = number of unique gene chunks.  A window's pooled vector depends on its tokens alone, so the
+        result of an item equals its result in a slab built by `prepare` from its own tokens.  -> a slab for
+        run_pooled(slab, unique CRE pooled rows, unique gene pooled rows)."""
+        C = np.array([len(r) for r in cre_rows])
+        s = {"cre_rows": torch.from_numpy(np.concatenate(cre_rows).astype(np.int64)).to(self.device, non_blocking=True)}
+        return self._prepare_seq2gene(s, C, [np.asarray(r, np.int64) for r in gene_rows], int(n_gene_chunks), tissues,
+                                      ref_labels)
+
+    def _prepare_seq2gene(self, s, C, gene_rows, n_gene_chunks, tissues, ref_labels, cre_token_position=None,
+                          gene_token_position=None):
+        """Index structures of stages 3-4: gene_rows[g] = rows of gene g's chunk embeddings in gene_map's output."""
+        dev = self.device
+        B = len(gene_rows)
+        G = np.array([len(r) for r in gene_rows])
+        T = np.array([len(t) for t in tissues])
+        up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev, non_blocking=True)
+        s.update({"B": B, "C": C, "G": G, "T": T, "n_gene_chunks": n_gene_chunks})
+        # gene stream layout: per (gene, tissue): [registry(tissue); the gene's chunk embeddings]
         idx, seq_lens = [], []
         for g in range(B):
             tis = tissues[g].detach().cpu().numpy().astype(np.int64).reshape(-1)
-            body = np.arange(g_off[g], g_off[g + 1], dtype=np.int64)
+            body = gene_rows[g]
             for t in tis:
                 idx.append(np.concatenate([[-(t + 1)], body]))
                 seq_lens.append(G[g] + 1)
@@ -434,13 +457,25 @@ class Engine:
     @torch.no_grad()
     def run(self, s):
         """-> dict(pred fp32 [sum T], emb fp32 [sum T, D], T list, optional token embeddings); device tensors."""
+        return self.run_pooled(s, *self.pool_windows(s))
+
+    @torch.no_grad()
+    def pool_windows(self, s):
+        """Stage 2 of a slab built by `prepare`: the window encoders.  -> (CRE pooled bf16 [sum C, d], gene pooled bf16
+        [sum G, d])."""
+        cre_pooled = self.seq2reg(self.cre_tok, s["ctok"], s["cmsk"], s["clens"], s["c_cu_tok"], s["c_plan_tok"])
+        gene_pooled = self.seq2reg(self.gene_tok, s["gtok"], s["gmsk"], s["glens"], s["g_cu_tok"], s["g_plan_tok"])
+        return cre_pooled, gene_pooled
+
+    @torch.no_grad()
+    def run_pooled(self, s, cre_pooled, gene_pooled):
+        """Stages 3-4 of a slab from its pooled window vectors (pool_windows, or the unique windows of a slab built by
+        prepare_shared).  -> the dict of `run`."""
         w, ws = self.w, self.ws
         D, H, hd = w.D, w.H, w.hd
         nC, Mg = int(s["C"].sum()), s["Mg"]
-
-        # ---- stage 2: window encoders ----
-        cre_pooled = self.seq2reg(self.cre_tok, s["ctok"], s["cmsk"], s["clens"], s["c_cu_tok"], s["c_plan_tok"])
-        gene_pooled = self.seq2reg(self.gene_tok, s["gtok"], s["gmsk"], s["glens"], s["g_cu_tok"], s["g_plan_tok"])
+        if "cre_rows" in s:                                  # shared windows: each item's CRE rows (1 KB per row)
+            cre_pooled = cre_pooled.index_select(0, s["cre_rows"])
         if COARSE and ops.PROFILER is None and w.cre_map is not None:
             return self._run_coarse(s, cre_pooled, gene_pooled)
         if w.cre_map is None:
@@ -557,7 +592,7 @@ class Engine:
             n_reg = s["reg_idx"].numel()
             cpos = s.get("cre_pos_idx")
             s["_abi_slab"] = _abi.Seq2GeneSlab(
-                int(s["C"].sum()), int(s["G"].sum()), s["Mg"], n_reg, s["n_need"], 0,
+                int(s["C"].sum()), s["n_gene_chunks"], s["Mg"], n_reg, s["n_need"], 0,
                 s["gene_idx"].data_ptr(), s["row_seq"].data_ptr(), s["logc"].data_ptr(), s["last_rows"].data_ptr(),
                 None if cpos is None else cpos.data_ptr(), *tab("plan_gself"), *tab("plan_gcross"), *tab("plan_cself"),
                 *tab("plan_last_self"), *tab("plan_last_cross"))

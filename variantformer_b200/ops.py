@@ -436,6 +436,29 @@ def encode_windows(genome, win_base, w0, w1, var_lo, var_hi, flags, variants, ma
     return out, out_len, err
 
 
+def mutate_windows(src, src_len, row_src, row_off, row_base, flags, err=None):
+    """Single-base substitutions of encoded windows (vf_mutate_windows): row r = src[row_src[r]] with the base at
+    forward-strand offset row_off[r] replaced by row_base[r] (complemented on reverse-complemented rows, flags bit 0).
+    src uint8 [n_src, pitch] and src_len int32 [n_src] as encode_windows returns them; row_src / row_off int32,
+    row_base / flags uint8 [n_rows] device tensors.  -> (out uint8 [n_rows, pitch], out_len int32 [n_rows], err)."""
+    n, pitch = row_src.numel(), src.shape[1]
+    dev = src.device
+    assert src.dtype == torch.uint8 and src.is_contiguous() and src_len.dtype == torch.int32
+    assert row_src.dtype == torch.int32 and row_off.dtype == torch.int32 and row_off.numel() == n
+    assert row_base.dtype == torch.uint8 and flags.dtype == torch.uint8 and row_base.numel() == n and flags.numel() == n
+    out = torch.empty((n, pitch), dtype=torch.uint8, device=dev)
+    out_len = torch.empty(n, dtype=torch.int32, device=dev)
+    if err is None:
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+    for r0 in range(0, n, 65535):                                       # grid.y limit of one launch
+        r1 = min(n, r0 + 65535)
+        with _timed("stage1_mutate", nbytes=2.0 * (r1 - r0) * pitch):  # row bytes read + written (upper bound)
+            check(_lib.lib().vf_mutate_windows(ptr(src), pitch, ptr(src_len), ptr(row_src[r0:r1]), ptr(row_off[r0:r1]),
+                                               ptr(row_base[r0:r1]), ptr(flags[r0:r1]), r1 - r0, ptr(out[r0:r1]), pitch,
+                                               ptr(out_len[r0:r1]), ptr(err), stream()))
+    return out, out_len, err
+
+
 def bpe_tokenize(seq, lens, max_len, merges, out_pitch, out_cap, want_starts=False, typical_len=None):
     """seq uint8 [n, pitch]; lens int32 [n]; merges = (a, b, new[, batch]) uint16 device tensors (viewed as int16
     storage); `batch` = per-rank batch ids (stage1.merge_batches) or absent."""

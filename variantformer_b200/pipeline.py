@@ -68,7 +68,7 @@ class HotPath:
             order = np.argsort(g.cre_start, kind="stable")
             labels.append(torch.from_numpy(np.asarray(g.cre_labels)[order[::-1] if g.strand == "-" else order].copy()))
         return dict(cre_tok=cre_tok, cre_msk=cre_msk, gene_tok=gene_tok, gene_msk=gene_msk, labels=labels,
-                    lens=(ccnt_h, glen_h), err=errs)
+                    lens=(ccnt_h, glen_h), err=errs, cre_seq=(seq, lens), gene_seq=(gseq, glens), gene_count=gcnt)
 
     def prepare(self, genes, variants: SampleVariants = None):
         """Stage 1 + all host bookkeeping for one slab -> a prepared slab for Engine.run."""

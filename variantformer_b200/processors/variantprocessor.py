@@ -60,6 +60,14 @@ class VariantProcessor:
                         np.asarray([MAP_REF_CRE_TO_IDX.get(c, 0) for c in m["cre_name"]], np.int64), tissues,
                         cre_chrom=list(m["chromosome"]))
 
+    def _load_inputs(self, vcf_path=None, sample_name=None):
+        """Genome (loaded once, HBM-resident), the optional background sample and the gene table."""
+        genes = pd.read_csv(self.model_config.dataset.gencode_v24).set_index("gene_id", drop=False)
+        if self._genome is None:
+            self._genome = Genome.from_arrays(ingest.load_fasta(self.vep_loader_config.fasta_path), "cuda")
+        self.background = ingest.load_vcf_sample(vcf_path, sample=sample_name) if vcf_path else None
+        return genes
+
     def initialize(self, var_df, output_dir, vcf_path=None, sample_name=None):
         """-> (pairs, model, trainer, checkpoint_path).  One pair per (variant row, gene)."""
         os.makedirs(output_dir, exist_ok=True)
@@ -69,10 +77,7 @@ class VariantProcessor:
         df = var_df.rename(columns={"chr": "chrom"})
         for col in ("chrom", "pos", "ref", "alt", "tissue", "gene_id"):
             assert col in df.columns, f"var_df must contain a '{col}' column"
-        genes = pd.read_csv(self.model_config.dataset.gencode_v24).set_index("gene_id", drop=False)
-        if self._genome is None:
-            self._genome = Genome.from_arrays(ingest.load_fasta(self.vep_loader_config.fasta_path), "cuda")
-        self.background = ingest.load_vcf_sample(vcf_path, sample=sample_name) if vcf_path else None
+        genes = self._load_inputs(vcf_path, sample_name)
         pairs = []
         for _, r in df.iterrows():
             names = [t.strip() for t in str(r["tissue"]).split(",") if t.strip() in self.tissue_vocab]
@@ -102,6 +107,53 @@ class VariantProcessor:
         df = self.compile_predictions(pairs, predictions)
         df.to_parquet(self.output_file)
         return df
+
+    def saturation_mutagenesis(self, gene_id, tissues, start, end, vcf_path=None, sample_name=None, zygosity=(2,)):
+        """In-silico saturation mutagenesis of [start, end] (1-based, inclusive, on the gene's chromosome): every
+        single-base substitution, scored as `predict` scores Variant(chrom, pos, ref, alt) for this gene, in batched
+        passes that encode every distinct window once (variantformer_b200.ism).  tissues: tissue names (or one name);
+        zygosity: a subset of {1 (het), 2 (hom)}.  Positions whose reference or background base is not A/C/G/T, and
+        positions that touch no window, are skipped.  Writes no file.
+        -> long format, one row per (pos, alt, zygosity, tissue): chrom, pos, ref, alt, genes, tissues, variant_type,
+        population, sample_name, zygosity, gene_exp, ref_gene_exp, log2fc = log2((gene_exp + 1e-10) /
+        (ref_gene_exp + 1e-10)) (the eqtl_scores form)."""
+        from .. import ism
+        from ..pipeline import HotPath
+        from ..stage1 import SampleVariants
+        names = [tissues] if isinstance(tissues, str) else [str(t).strip() for t in tissues]
+        unknown = [t for t in names if t not in self.tissue_vocab]
+        if unknown or not names:
+            raise ValueError(f"unknown tissue(s) {unknown}; see tissue_vocab.yaml" if unknown else "no tissue given")
+        genes = self._load_inputs(vcf_path, sample_name)
+        if gene_id not in genes.index:
+            raise KeyError(f"gene {gene_id!r} is not in the gene table")
+        tis = [self.tissue_vocab[t] for t in names]
+        gene = self._gene_spec(genes.loc[gene_id], tis)
+        model, _ = self.model_manager.load_model()
+        ds = self.model_config.dataset
+        hot = HotPath(model.engine(), self._genome, max_length=ds.max_length, max_chunks=ds.max_chunks,
+                      cre_neighbour_hood=ds.cre_neighbour_hood, gene_upstream=ds.gene_upstream_neighbour_hood,
+                      gene_downstream=ds.gene_downstream_neighbour_hood)
+        bg = None
+        if self.background:                                   # the sample contributes SNPs only (variant_type="SNP")
+            bg = SampleVariants({c: VEPBatchBuilder._snps_only(b) for c, b in self.background.items()}, "cuda")
+        res = ism.saturation_mutagenesis(hot, gene, int(start), int(end), zygosity, bg)
+        pred = res["pred"].cpu().numpy(); ref = res["ref_pred"].cpu().numpy()
+        muts = res["plan"].mutants
+        nt = len(tis)
+        rep = lambda xs: np.repeat(np.asarray(xs, dtype=object), nt)
+        gene_exp = pred.reshape(-1).astype(np.float64)
+        ref_exp = np.tile(ref.astype(np.float64), len(muts))
+        vtype = ["Gene and CRE overlap" if m.hits and m.gene_hit else "CRE overlap only" if m.hits else
+                 "Gene overlap only" for m in muts]
+        return pd.DataFrame({
+            "chrom": [gene.chrom] * (nt * len(muts)), "pos": np.repeat([m.pos for m in muts], nt).astype(np.int64),
+            "ref": rep([m.ref for m in muts]), "alt": rep([m.alt for m in muts]), "genes": [gene_id] * (nt * len(muts)),
+            "tissues": names * len(muts), "variant_type": rep(vtype),
+            "population": ["SAMPLE" if vcf_path else "REF_HG38"] * (nt * len(muts)),
+            "sample_name": [sample_name or "hg38"] * (nt * len(muts)), "zygosity": rep([str(m.zyg) for m in muts]),
+            "gene_exp": gene_exp, "ref_gene_exp": ref_exp,
+            "log2fc": np.log2((gene_exp + 1e-10) / (ref_exp + 1e-10))})
 
     def compile_predictions(self, pairs, predictions):
         """Long format, one row per (pair, zygosity, tissue): the reference's column set (variantprocessor.py:305-320)."""
