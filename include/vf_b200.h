@@ -178,6 +178,7 @@ int vf_forest_predict(const float* x, int ldx, int n_rows, int d, const int32_t*
  * hom SNP -> ALT, indel/MNP -> REF span replaced by ALT, overlapping or window-straddling records skipped;
  * flags bit0 = reverse-complement the result, bit1 = SNP-only filter.
  * out: uint8 [n_win, pitch]; out_len int32 [n_win]; err: device int32 flag (1 pitch overflow, 2 >2048 records).
+ * Any n_win: batches of more than 65535 windows are launched in chunks of 65535.
  * Replaces the `samtools faidx | bcftools consensus -H I -e 'ALT~"<.*>"'` subprocess pair per window
  * (utils/data_process.py:17-101, :367-467) and utils/functions.py:129-172 (reverse_complement).
  */

@@ -139,11 +139,17 @@ int encode_windows(const uint8_t* genome, const int64_t* win_base, const int32_t
     if (n_win == 0) return 0;
     VF_REQUIRE(max_window > 0 && pitch >= max_window, "encode_windows: pitch %lld < max window %d", (long long)pitch,
                max_window);
-    EncodeParams p{genome, win_base, w0, w1, var_lo, var_hi, flags, v_pos, v_ref_len, v_alt_off, v_alt_len, v_gt,
-                   alt_pool, out, pitch, out_len, err};
-    dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n_win);
-    encode_windows_kernel<<<grid, 256, 0, s>>>(p);
-    VF_LAUNCH_OK("encode_windows_kernel launch");
+    // the window index is blockIdx.y, capped at 65535 by the hardware: larger batches (every CRE window of a big slab)
+    // go in chunks, each launch seeing its chunk's windows from index 0
+    constexpr int kMaxWinPerLaunch = 65535;
+    for (int c0 = 0; c0 < n_win; c0 += kMaxWinPerLaunch) {
+        const int n = n_win - c0 < kMaxWinPerLaunch ? n_win - c0 : kMaxWinPerLaunch;
+        EncodeParams p{genome, win_base + c0, w0 + c0, w1 + c0, var_lo + c0, var_hi + c0, flags + c0, v_pos, v_ref_len,
+                       v_alt_off, v_alt_len, v_gt, alt_pool, out + (size_t)c0 * pitch, pitch, out_len + c0, err};
+        dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n);
+        encode_windows_kernel<<<grid, 256, 0, s>>>(p);
+        VF_LAUNCH_OK("encode_windows_kernel launch");
+    }
     return 0;
 }
 
