@@ -194,12 +194,27 @@ int vf_encode_windows(const uint8_t* genome, const int64_t* win_base, const int3
  * goes to len - 1 - row_off[r] as its IUPAC complement (the table vf_encode_windows applies).  The caller passes the
  * base of the datasets/vepdataset.py:94-131 rule: the ALT base (hom) or get_iupac_code(ref, alt) (het).
  * out: uint8 [n_rows, out_pitch]; out_len int32 [n_rows]; err: device int32 flag (1 row longer than a pitch, 3 offset
- * outside the row; such a row gets length 0).  Pitches: multiples of 16, rows 16-byte aligned; n_rows <= 65535.
- * The rows then go through vf_bpe_tokenize like any encoded window.
+ * outside the row; such a row gets length 0).  Pitches: multiples of 16, rows 16-byte aligned; any n_rows.
+ * The rows then go through vf_bpe_tokenize like any encoded window.  Same kernel as vf_splice_windows with k = 1.
  */
 int vf_mutate_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
                       const int32_t* row_off, const uint8_t* row_base, const uint8_t* flags, int n_rows, uint8_t* out,
                       int64_t out_pitch, int32_t* out_len, int32_t* err, void* stream);
+/*
+ * Allele splice of encoded windows (variant tables): row r of out = the source row src[row_src[r]] with the ONE base at
+ * forward-strand offset row_off[r] replaced by the k = allele_len[r] >= 0 bytes allele_pool[allele_off[r], + k) (a
+ * multi-base allele is an insertion, an empty one deletes the base; nothing else is deleted: the
+ * datasets/vepdataset.py:94-131 rule).  flags[r] bit0 = the
+ * source was reverse-complemented: the reverse complement of the allele (vf_encode_windows' table) replaces the byte at
+ * len - 1 - row_off[r].  out_len[r] = len + k - 1.  allele_off == allele_len == NULL: row r's allele is allele_pool[r],
+ * k = 1 (vf_mutate_windows).  err: device int32 flag (1 output row longer than out_pitch, 3 offset outside the row or
+ * k < 0; such a row gets length 0).  Pitches: multiples of 16, rows 16-byte aligned; any n_rows (launched in chunks of
+ * 65535).
+ */
+int vf_splice_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
+                      const int32_t* row_off, const uint8_t* allele_pool, const int32_t* allele_off,
+                      const int32_t* allele_len, const uint8_t* flags, int n_rows, uint8_t* out, int64_t out_pitch,
+                      int32_t* out_len, int32_t* err, void* stream);
 /*
  * BPE tokenisation of n_win byte sequences (upper-cased; non-IUPAC characters split words).
  * merge_a/merge_b/merge_new: uint16 [n_merges] rank-ordered merge table.  merge_batch: uint16 [n_merges] nondecreasing
@@ -294,6 +309,15 @@ typedef struct {
  * (Softplus applied), emb fp32 [n_reg, D]; gene_token_emb fp32 [n_need - n_reg, D] and cre_token_emb fp32 [n_reg, D]
  * may be NULL.  The CRE stack runs on a side stream owned by the library (one forward in flight per device).
  */
+/*
+ * Rows of the final CRE stream of the forward that just ran (CRE-token embeddings of arbitrary rows, e.g. several per
+ * prediction in a slab whose items share windows): out_f32 [n, D] = raw (un-centred) value of CRE row rows[r] of the
+ * slab, the same gather + un-centring as cre_token_emb.  PRECONDITION: called on the same stream right after
+ * vf_seq2gene_forward with the same weight table, slab and workspace (untouched in between): it reads the stream that
+ * call left in the workspace.  rows int32 [n], each in [0, n_cre).
+ */
+int vf_seq2gene_cre_rows(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t* slab, void* workspace,
+                         size_t workspace_bytes, const int32_t* rows, int n, float* out_f32, void* stream);
 size_t vf_seq2gene_workspace_bytes(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t* slab);
 int vf_seq2gene_forward(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t* slab, const void* cre_pooled_bf16,
                         const void* gene_pooled_bf16, void* workspace, size_t workspace_bytes, float* pred, float* emb,

@@ -25,6 +25,7 @@ SIGNATURES = {
     "vf_seq2reg_forward": ([_vp, _vp, _vp, _vp, _i32, _i32, _i64, _vp, _i32, _vp, _sz, _vp, _vp], _i32),
     "vf_seq2gene_workspace_bytes": ([_vp, _vp], _sz),
     "vf_seq2gene_forward": ([_vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp], _i32),
+    "vf_seq2gene_cre_rows": ([_vp, _vp, _vp, _sz, _vp, _i32, _vp, _vp], _i32),
     "vf_device_check": ([_vp], _i32),
     "vf_gemm_bf16": ([_vp, _i32, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _i32, _vp, _i32, _vp], _i32),
     "vf_gemm_bf16_ln": ([_vp, _i32, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32, _vp, _i32, _vp, _i32,
@@ -46,6 +47,7 @@ SIGNATURES = {
     "vf_forest_predict": ([_vp, _i32, _i32, _i32] + [_vp] * 9 + [_i32, _vp, _vp], _i32),
     "vf_encode_windows": ([_vp] * 13 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
     "vf_mutate_windows": ([_vp, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
+    "vf_splice_windows": ([_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
     "vf_bpe_tokenize": ([_vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _i64,
                          _i32, _vp], _i32),
 }

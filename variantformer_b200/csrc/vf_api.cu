@@ -122,6 +122,13 @@ int vf_mutate_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_
     return mutate_windows(src, src_pitch, src_len, row_src, row_off, row_base, flags, n_rows, out, out_pitch, out_len, err,
                           ST(stream));
 }
+int vf_splice_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
+                      const int32_t* row_off, const uint8_t* allele_pool, const int32_t* allele_off,
+                      const int32_t* allele_len, const uint8_t* flags, int n_rows, uint8_t* out, int64_t out_pitch,
+                      int32_t* out_len, int32_t* err, void* stream) {
+    return splice_windows(src, src_pitch, src_len, row_src, row_off, allele_pool, allele_off, allele_len, flags, n_rows,
+                          out, out_pitch, out_len, err, ST(stream));
+}
 int vf_bpe_tokenize(const uint8_t* seq, int64_t pitch, const int32_t* len, int n_win, int max_len,
                     const uint16_t* merge_a, const uint16_t* merge_b, const uint16_t* merge_new,
                     const uint16_t* merge_batch, int n_merges, uint16_t* scratch, int64_t scratch_pitch, int32_t* out_tokens, int out_pitch, int out_cap,

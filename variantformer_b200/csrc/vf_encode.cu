@@ -154,75 +154,131 @@ int encode_windows(const uint8_t* genome, const int64_t* win_base, const int32_t
 }
 
 // ---------------------------------------------------------------------------------
-// mutate_windows: an encoded window with ONE base replaced (saturation mutagenesis).  Row r of `out` is the source row
-// src[row_src[r]] with the base at forward-strand offset row_off[r] set to row_base[r]; a reverse-complemented source
-// (flags bit 0) gets it at len - 1 - off as its complement, with the table encode_windows uses (comp_base).
-// One CTA per (row, 16 KB slice), 16-byte loads and stores: pure copy bandwidth.
+// splice_windows: an encoded window with ONE base replaced by an allele of k >= 0 bases (variant tables: a hom ALT of
+// any length, k = 0 deleting the base; saturation mutagenesis: k = 1).  Row r of `out` is the source row src[row_src[r]] with the base at
+// forward-strand offset row_off[r] replaced by allele_pool[allele_off[r], + allele_len[r]); a reverse-complemented source
+// (flags bit 0) gets the reverse complement of the allele in place of the byte at len - 1 - off, with the table
+// encode_windows uses (comp_base).  The row grows by k - 1 bytes (shrinks by one for k = 0).
+// One CTA per (row, 16 KB output slice); each thread writes whole 16-byte output groups:
+//   head groups (before the allele)      aligned copy of the same source group;
+//   allele groups                        assembled in registers byte by byte (at most ceil(k / 16) + 1 groups);
+//   tail groups (after the allele)       source shifted by k - 1 bytes: two aligned 16-byte loads + funnel shifts.
+// k = 1 (mutate_windows) makes the tail shift zero: every group but the one holding the base is an aligned copy.
 // ---------------------------------------------------------------------------------
-constexpr int kMutSlice = 16384;
+constexpr int kSpliceSlice = 16384;
 
-struct MutateParams {
+struct SpliceParams {
     const uint8_t* src; int64_t src_pitch; const int32_t* src_len;
-    const int32_t* row_src; const int32_t* row_off; const uint8_t* row_base; const uint8_t* flags;
+    const int32_t* row_src; const int32_t* row_off;
+    const uint8_t* allele_pool; const int32_t* allele_off; const int32_t* allele_len;   // off / len NULL: pool[r], k = 1
+    const uint8_t* flags;
     uint8_t* out; int64_t out_pitch; int32_t* out_len; int32_t* err;
 };
 
+__device__ __forceinline__ uint32_t pick(uint32_t a, uint32_t b, uint32_t c, uint32_t d, uint32_t e, uint32_t f,
+                                         uint32_t g, uint32_t h, int i) {   // word i of the 8-word window (selects only)
+    return i == 0 ? a : i == 1 ? b : i == 2 ? c : i == 3 ? d : i == 4 ? e : i == 5 ? f : i == 6 ? g : h;
+}
+// bytes [b, b + 16) of the row s4 (b >= 0), from the aligned groups b >> 4 and (b >> 4) + 1; the second group is read
+// only when it holds a byte below `len` (never past the source row)
+__device__ __forceinline__ uint4 load_shifted(const uint4* s4, int b, int len) {
+    const int j = b >> 4, sh = b & 15;
+    const uint4 lo = s4[j];
+    if (sh == 0) return lo;
+    const uint4 hi = ((j + 1) << 4) < len ? s4[j + 1] : make_uint4(0, 0, 0, 0);
+    const int ws = sh >> 2, bs = 8 * (sh & 3);
+    uint32_t w[5];
+#pragma unroll
+    for (int m = 0; m < 5; ++m) w[m] = pick(lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w, m + ws < 8 ? m + ws : 7);
+    return make_uint4(__funnelshift_r(w[0], w[1], bs), __funnelshift_r(w[1], w[2], bs), __funnelshift_r(w[2], w[3], bs),
+                      __funnelshift_r(w[3], w[4], bs));
+}
+
 __global__ void __launch_bounds__(256)
-mutate_windows_kernel(const MutateParams p) {
+splice_windows_kernel(const SpliceParams p) {
     const int r = blockIdx.y;
     const int sr = p.row_src[r];
     const int len = p.src_len[sr];
     const int off = p.row_off[r];
+    const int k = p.allele_len ? p.allele_len[r] : 1;
+    const int64_t a0 = p.allele_off ? p.allele_off[r] : r;
+    const int64_t n_out = (int64_t)len + k - 1;
     // a row that cannot be built writes nothing but a zero length (and the error flag): the tokenizer then sees an
     // empty window and never reads the unwritten row
-    const bool bad_len = len < 0 || (int64_t)len > p.out_pitch || (int64_t)len > p.src_pitch;
-    const bool bad_off = off < 0 || off >= len;
+    const bool bad_len = len < 0 || (int64_t)len > p.src_pitch || n_out > p.out_pitch;
+    const bool bad_off = off < 0 || off >= len || k < 0;
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         if (bad_len) atomicMax(p.err, 1);
         else if (bad_off) atomicMax(p.err, 3);
-        p.out_len[r] = (bad_len || bad_off) ? 0 : len;
+        p.out_len[r] = (bad_len || bad_off) ? 0 : (int)n_out;
     }
     if (bad_len || bad_off) return;
-    const int b0 = blockIdx.x * kMutSlice;
-    if (b0 >= len) return;
-    const int b1 = min(len, b0 + kMutSlice);
+    const int b0 = blockIdx.x * kSpliceSlice;
+    if (b0 >= n_out) return;
+    const int b1 = (int)min(n_out, (int64_t)b0 + kSpliceSlice);
     const bool rc = p.flags[r] & 1;
-    const int q = rc ? len - 1 - off : off;                   // where the base lands in the stored (strand-oriented) row
-    const uint8_t base = rc ? comp_base(p.row_base[r]) : p.row_base[r];
+    const int q = rc ? len - 1 - off : off;                   // first allele byte in the stored (strand-oriented) row
+    const int qe = q + k;                                     // first tail byte; tail byte o = source byte o - (k - 1)
+    const uint8_t* allele = p.allele_pool + a0;
     const uint4* s4 = reinterpret_cast<const uint4*>(p.src + (size_t)sr * p.src_pitch);
     uint4* o4 = reinterpret_cast<uint4*>(p.out + (size_t)r * p.out_pitch);
-    // whole 16-byte groups up to the one holding the last byte: both pitches are multiples of 16 (host check), so the
-    // last group stays inside both rows; bytes past len are copied as they are (they are never read)
+    // whole 16-byte groups up to the one holding the last byte: the out pitch is a multiple of 16 (host check), so the
+    // last group stays inside the row; bytes past n_out are filled with whatever is at hand (they are never read)
     const int g0 = b0 >> 4, g1 = (b1 + 15) >> 4;
     for (int g = g0 + threadIdx.x; g < g1; g += blockDim.x) {
-        uint4 v = s4[g];
-        if (g == (q >> 4)) {                                  // byte q & 15 of the group (selects: no local memory)
-            const int word = (q >> 2) & 3, sh = (q & 3) * 8;
-            const uint32_t keep = ~(0xFFu << sh), put = (uint32_t)base << sh;
-            v.x = word == 0 ? (v.x & keep) | put : v.x;
-            v.y = word == 1 ? (v.y & keep) | put : v.y;
-            v.z = word == 2 ? (v.z & keep) | put : v.z;
-            v.w = word == 3 ? (v.w & keep) | put : v.w;
+        const int o = g << 4;
+        uint4 v;
+        if (o + 16 <= q) {
+            v = s4[g];                                        // head
+        } else if (o >= qe) {
+            v = load_shifted(s4, o - (k - 1), len);           // tail
+        } else {                                              // holds allele bytes (and maybe head / tail bytes)
+            const uint8_t* row = p.src + (size_t)sr * p.src_pitch;
+            uint32_t w[4] = {0, 0, 0, 0};
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+                const int x = o + i;
+                uint32_t c = 0;
+                if (x < q) c = row[x];
+                else if (x < qe) c = rc ? comp_base(allele[k - 1 - (x - q)]) : allele[x - q];
+                else if (x < n_out) c = row[x - (k - 1)];
+                w[i >> 2] |= c << (8 * (i & 3));
+            }
+            v = make_uint4(w[0], w[1], w[2], w[3]);
         }
         o4[g] = v;
     }
 }
 
+int splice_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
+                   const int32_t* row_off, const uint8_t* allele_pool, const int32_t* allele_off,
+                   const int32_t* allele_len, const uint8_t* flags, int n_rows, uint8_t* out, int64_t out_pitch,
+                   int32_t* out_len, int32_t* err, cudaStream_t s) {
+    if (n_rows == 0) return 0;
+    VF_REQUIRE(src_pitch > 0 && src_pitch % 16 == 0 && out_pitch > 0 && out_pitch % 16 == 0,
+               "splice_windows: pitches must be positive multiples of 16 (src %lld, out %lld)", (long long)src_pitch,
+               (long long)out_pitch);
+    VF_REQUIRE(((uintptr_t)src & 15) == 0 && ((uintptr_t)out & 15) == 0, "splice_windows: rows must be 16-byte aligned");
+    VF_REQUIRE((allele_off == nullptr) == (allele_len == nullptr), "splice_windows: allele_off and allele_len go together");
+    // the row index is blockIdx.y (at most 65535 per launch): larger batches go in chunks
+    constexpr int kMaxRowsPerLaunch = 65535;
+    for (int c0 = 0; c0 < n_rows; c0 += kMaxRowsPerLaunch) {
+        const int n = n_rows - c0 < kMaxRowsPerLaunch ? n_rows - c0 : kMaxRowsPerLaunch;
+        SpliceParams p{src, src_pitch, src_len, row_src + c0, row_off + c0, allele_off ? allele_pool : allele_pool + c0,
+                       allele_off ? allele_off + c0 : nullptr, allele_len ? allele_len + c0 : nullptr, flags + c0,
+                       out + (size_t)c0 * out_pitch, out_pitch, out_len + c0, err};
+        dim3 grid((unsigned)((out_pitch + kSpliceSlice - 1) / kSpliceSlice), n);
+        splice_windows_kernel<<<grid, 256, 0, s>>>(p);
+        VF_LAUNCH_OK("splice_windows_kernel launch");
+    }
+    return 0;
+}
+
 int mutate_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
                    const int32_t* row_off, const uint8_t* row_base, const uint8_t* flags, int n_rows, uint8_t* out,
                    int64_t out_pitch, int32_t* out_len, int32_t* err, cudaStream_t s) {
-    if (n_rows == 0) return 0;
-    VF_REQUIRE(src_pitch > 0 && src_pitch % 16 == 0 && out_pitch > 0 && out_pitch % 16 == 0,
-               "mutate_windows: pitches must be positive multiples of 16 (src %lld, out %lld)", (long long)src_pitch,
-               (long long)out_pitch);
-    VF_REQUIRE(((uintptr_t)src & 15) == 0 && ((uintptr_t)out & 15) == 0, "mutate_windows: rows must be 16-byte aligned");
-    VF_REQUIRE(n_rows <= 65535, "mutate_windows: %d rows in one call (at most 65535)", n_rows);
-    const int64_t span = src_pitch < out_pitch ? src_pitch : out_pitch;   // longest row that can be valid
-    MutateParams p{src, src_pitch, src_len, row_src, row_off, row_base, flags, out, out_pitch, out_len, err};
-    dim3 grid((unsigned)((span + kMutSlice - 1) / kMutSlice), n_rows);
-    mutate_windows_kernel<<<grid, 256, 0, s>>>(p);
-    VF_LAUNCH_OK("mutate_windows_kernel launch");
-    return 0;
+    return splice_windows(src, src_pitch, src_len, row_src, row_off, row_base, nullptr, nullptr, flags, n_rows, out,
+                          out_pitch, out_len, err, s);
 }
 
 // ---------------------------------------------------------------------------------

@@ -300,6 +300,18 @@ static int seq2gene_forward(const vf_seq2gene_weights_t& w, const vf_seq2gene_sl
     return 0;
 }
 
+// CRE-token rows of the forward that just ran: the final CRE stream and its pivots are still in the workspace
+static int seq2gene_cre_rows(const vf_seq2gene_weights_t& w, const vf_seq2gene_slab_t& t, void* ws, size_t ws_bytes,
+                             const int32_t* rows, int n, float* out, cudaStream_t s) {
+    if (n == 0) return 0;
+    Seq2GeneWs b = carve_seq2gene(w, t, ws);
+    VF_REQUIRE(ws && ws_bytes >= b.bytes, "seq2gene_cre_rows: workspace of %zu bytes < %zu needed", ws_bytes, b.bytes);
+    VF_REQUIRE(rows && out, "seq2gene_cre_rows: NULL rows / out");
+    int rc;
+    if ((rc = gather_rows(b.cx, w.D, nullptr, 0, rows, n, w.D, out, nullptr, w.D, s))) return rc;
+    return uncenter_rows(out, w.D, b.cpiv, rows, n, w.D, out, nullptr, w.D, s);
+}
+
 // ====================================================================================================================
 // attention work tables (host): the C counterpart of variantformer_b200.ops.SlotMap
 // ====================================================================================================================
@@ -367,6 +379,12 @@ int vf_seq2gene_forward(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t
     VF_REQUIRE(w && slab, "seq2gene_forward: NULL weight table / slab");
     return seq2gene_forward(*w, *slab, cre_pooled_bf16, gene_pooled_bf16, workspace, workspace_bytes, pred, emb, gene_token_emb,
                             cre_token_emb, ST(stream));
+}
+
+int vf_seq2gene_cre_rows(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t* slab, void* workspace,
+                         size_t workspace_bytes, const int32_t* rows, int n, float* out_f32, void* stream) {
+    VF_REQUIRE(w && slab, "seq2gene_cre_rows: NULL weight table / slab");
+    return seq2gene_cre_rows(*w, *slab, workspace, workspace_bytes, rows, n, out_f32, ST(stream));
 }
 
 }  // extern "C"

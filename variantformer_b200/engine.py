@@ -378,20 +378,30 @@ class Engine:
         return self._prepare_seq2gene(s, C, gene_rows, int(G.sum()), tissues, ref_labels, cre_token_position,
                                       gene_token_position)
 
-    def prepare_shared(self, cre_rows, gene_rows, n_gene_chunks, tissues, ref_labels):
+    def prepare_shared(self, cre_rows, gene_rows, n_gene_chunks, tissues, ref_labels, cre_token_rows=None,
+                       gene_token_positions=None):
         """Slab of items whose windows are encoded once and shared between items (saturation mutagenesis: every
-        mutant of a gene reuses the reference item's unchanged windows).  cre_rows / gene_rows: one int array per item,
-        the rows of the item's CRE windows / gene chunks (in batch order) in the pooled outputs of the unique windows;
-        n_gene_chunks = number of unique gene chunks.  A window's pooled vector depends on its tokens alone, so the
-        result of an item equals its result in a slab built by `prepare` from its own tokens.  -> a slab for
-        run_pooled(slab, unique CRE pooled rows, unique gene pooled rows)."""
+        mutant of a gene reuses the reference item's unchanged windows; variant tables: every (variant, gene) pair reuses
+        its gene's reference item).  cre_rows / gene_rows: one int array per item, the rows of the item's CRE windows /
+        gene chunks (in batch order) in the pooled outputs of the unique windows; n_gene_chunks = number of unique gene
+        chunks.  A window's pooled vector depends on its tokens alone, so the result of an item equals its result in a
+        slab built by `prepare` from its own tokens.
+        Token rows (optional, one list per item, possibly empty): cre_token_rows = CRE rows of the item (batch order)
+        whose final CRE-stream value is returned (tissue-independent: one row per (item, row)); gene_token_positions =
+        gene-token positions whose last-layer output is returned, one row per (item, position, tissue), tissues
+        innermost.  -> a slab for run_pooled(slab, unique CRE pooled rows, unique gene pooled rows)."""
         C = np.array([len(r) for r in cre_rows])
         s = {"cre_rows": torch.from_numpy(np.concatenate(cre_rows).astype(np.int64)).to(self.device, non_blocking=True)}
+        if cre_token_rows is not None:
+            c_off = np.concatenate([[0], np.cumsum(C)])[:-1]
+            rows = [c_off[b] + np.asarray(r, np.int64).reshape(-1) for b, r in enumerate(cre_token_rows)]
+            s["cre_tok_rows"] = torch.from_numpy(np.concatenate(rows + [np.zeros(0, np.int64)]).astype(np.int32)).to(
+                self.device, non_blocking=True)
         return self._prepare_seq2gene(s, C, [np.asarray(r, np.int64) for r in gene_rows], int(n_gene_chunks), tissues,
-                                      ref_labels)
+                                      ref_labels, gene_token_positions=gene_token_positions)
 
     def _prepare_seq2gene(self, s, C, gene_rows, n_gene_chunks, tissues, ref_labels, cre_token_position=None,
-                          gene_token_position=None):
+                          gene_token_position=None, gene_token_positions=None):
         """Index structures of stages 3-4: gene_rows[g] = rows of gene g's chunk embeddings in gene_map's output."""
         dev = self.device
         B = len(gene_rows)
@@ -431,6 +441,13 @@ class Engine:
         if gene_token_position is not None:
             gp = np.repeat(np.asarray([int(p) for p in gene_token_position]) + 1, T)      # +1: registry token
             need_seq = np.concatenate([need_seq, np.arange(n_seq)]); need_off = np.concatenate([need_off, gp])
+        if gene_token_positions is not None:                                # per (item, position, tissue)
+            seq0 = np.concatenate([[0], np.cumsum(T)])[:-1]
+            ts, to = [np.zeros(0, np.int64)], [np.zeros(0, np.int64)]
+            for b, ps in enumerate(gene_token_positions):
+                ps = np.asarray(ps, np.int64).reshape(-1)
+                ts.append(np.tile(seq0[b] + np.arange(T[b]), len(ps))); to.append(np.repeat(ps + 1, T[b]))
+            need_seq = np.concatenate([need_seq] + ts); need_off = np.concatenate([need_off] + to)
         s["last_rows"] = up(reg_rows[need_seq] + need_off, np.int32)
         s["n_need"] = int(len(need_seq))
         k = np.arange(len(need_seq))
@@ -446,8 +463,8 @@ class Engine:
                 units.append([start, i - start, cu_cre_np[g], C[g], 0])
                 start = i
         s["plan_last_cross"] = AttnPlan(None, dev, self.w.hd, units=np.asarray(units))
-        if gene_token_position is not None:
-            s["gene_pos_idx"] = up(reg_rows + gp, np.int32)                                 # (:665-666)
+        if gene_token_position is not None or gene_token_positions is not None:
+            s["gene_pos_idx"] = up(reg_rows[need_seq[n_seq:]] + need_off[n_seq:], np.int32)   # (:665-666)
         if cre_token_position is not None:
             c_off = np.concatenate([[0], np.cumsum(C)])[:-1]
             s["cre_pos_idx"] = up(np.repeat(c_off + np.asarray([int(p) for p in cre_token_position]), T), np.int32)
@@ -580,6 +597,11 @@ class Engine:
         if "cre_pos_idx" in s:
             t, _ = ops.gather_rows(cx, None, s["cre_pos_idx"])
             out["cre_token_embedding"], _ = ops.uncenter_rows(t, cpiv, idx=s["cre_pos_idx"])
+        if "cre_tok_rows" in s:
+            out["cre_token_embedding"] = torch.empty((0, D), dtype=torch.float32, device=cx.device)
+            if s["cre_tok_rows"].numel():
+                t, _ = ops.gather_rows(cx, None, s["cre_tok_rows"])
+                out["cre_token_embedding"], _ = ops.uncenter_rows(t, cpiv, idx=s["cre_tok_rows"])
         return out
 
     def _run_coarse(self, s, cre_pooled, gene_pooled):
@@ -604,9 +626,12 @@ class Engine:
                                                      slab.n_need - slab.n_reg, w.D, "cre_pos_idx" in s)
         out = {"pred": pred, "emb": emb, "T": s["T"].tolist()}
         if "gene_pos_idx" in s:
-            out["gene_token_embedding"] = gtok
+            out["gene_token_embedding"] = gtok if gtok is not None else torch.empty((0, w.D), device=pred.device)
         if ctok is not None:
             out["cre_token_embedding"] = ctok
+        if "cre_tok_rows" in s:                              # the final CRE stream is still in the workspace
+            ws = self.ws.get("coarse_g", (nbytes,), torch.uint8)
+            out["cre_token_embedding"] = ops.seq2gene_cre_rows(w.abi(), slab, ws, s["cre_tok_rows"], w.D)
         return out
 
     def forward_tokens(self, cre_tokens, cre_masks, gene_tokens, gene_masks, tissues, ref_labels, **kw):

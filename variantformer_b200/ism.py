@@ -5,7 +5,7 @@ The result for position p (1-based), alternative base a and zygosity z is BY DEF
 get_iupac_code(ref, a), z = 2 writes a, into every window window_hits() says the variant reaches; a background sample
 contributes SNPs only and the query base wins at its position.  What is not recomputed (DESIGN section 11):
   * the reference item is encoded and tokenized once per gene;
-  * a mutant re-encodes only its hit CRE windows (vf_mutate_windows + the fixed-row BPE) and its gene window (full BPE
+  * a mutant re-encodes only its hit CRE windows (vf_splice_windows + the fixed-row BPE) and its gene window (full BPE
     of the mutated 301 kb word: an incremental re-tokenization is not proven exact);
   * a window's pooled seq2reg vector depends on its tokens alone, so every DISTINCT token row (CRE window or 200-token
     gene chunk) is encoded once over the whole region, and items point into the pooled rows (Engine.prepare_shared).
@@ -121,7 +121,171 @@ def _raise_on_error(err, what):
     code = int(err.item())
     if code:
         raise RuntimeError(f"stage-1 kernel reported error {code} while {what} (1: pitch overflow, 2: >2048 "
-                           "variants/window, 3: substitution outside its window)")
+                           "variants/window, 3: edit outside its window)")
+
+
+@dataclass
+class Edit:
+    """One edited item of a gene: the base at 1-based `pos` replaced by `data` (one byte or more: an insertion; empty:
+    a deletion) in the CRE windows `hits` (batch order) and, if `gene_hit`, in the gene window.  `plain_cre` /
+    `plain_gene`: CRE windows / the gene window that the item reads from the reference genome WITHOUT the background
+    sample (VEPBatchBuilder.build: the het / hom samples carry the background of the variant's chromosome only)."""
+    pos: int
+    data: bytes
+    hits: List[int]
+    gene_hit: bool
+    plain_cre: List[int] = field(default_factory=list)
+    plain_gene: bool = False
+
+
+def _round16(n):
+    return (int(n) + 15) // 16 * 16
+
+
+@torch.no_grad()
+def build_edit_items(hot, gene, edits: List[Edit], variants=None, want_gene_pos=False, t=None):
+    """Stage 1 of a pass over the edits of one gene: the reference item (gene + background `variants`) and one item per
+    edit as rows of two tables of DISTINCT token rows.  Edited windows are spliced from the reference item's encoded
+    windows (vf_splice_windows), CRE windows go through the fixed-row BPE, gene windows through the full BPE of the
+    edited word, and every distinct token row is kept once.  t: the reference item's HotPath.tokenize output (computed
+    here when None).  want_gene_pos: also return, per edited gene window, the strand-oriented offset p of the edit
+    (len(seq) - p - 1 on the minus strand, with the edited length), the character there and the index of the token
+    covering it (VEPBatchBuilder.build), and the gene window bytes and token starts of the reference item and of the
+    background-free reference (the same unless `variants` is given).
+    -> dict(cre_tokens int32 [n_c, L], gene_tokens int32 [n_g, L] (distinct rows, device), cre_rows / gene_rows (per item,
+    reference item first: int64 rows of the item's CRE windows / gene chunks in those tables), labels, C, G_ref,
+    g_count (gene chunks per edit item)[, gene_pos: per edit (p, char, token index) or None, ref_gene / plain_gene:
+    (bytes, starts)])."""
+    tok, dev = hot.tok, hot.engine.device
+    L = hot.max_length
+    t = hot.tokenize([gene], variants) if t is None else t
+    ref_ctok = t["cre_tok"][0]                                      # int32 [C, L]
+    ref_gtok = t["gene_tok"][0]                                     # int32 [G_ref, L]
+    C, G_ref = ref_ctok.shape[0], ref_gtok.shape[0]
+    _, wins = cre_windows(gene, hot.nb)
+    g0, _ = gene_window(gene.start, gene.end, gene.strand, hot.up, hot.down)
+    flag = int(gene.strand == "-")
+    err = t["err"].clone()
+    pool, a_off = bytearray(), []                                  # every edit's bytes, once
+    for e in edits:
+        a_off.append(len(pool)); pool += e.data
+    pool_d = _u8(np.frombuffer(bytes(pool) or b"\0", np.uint8), dev)
+    a_len = [len(e.data) for e in edits]
+    # ---- CRE windows: one spliced row per (edit, hit window), fixed 200-token rows ----
+    c_src, c_off, c_aoff, c_alen, c_owner = [], [], [], [], []
+    for i, e in enumerate(edits):
+        for k in e.hits:
+            c_src.append(k); c_off.append(e.pos - 1 - wins[k][0]); c_aoff.append(a_off[i]); c_alen.append(a_len[i])
+            c_owner.append(i)
+    cseq, clen = t["cre_seq"]
+    if c_src:
+        n = len(c_src)
+        mseq, mlen, err = ops.splice_windows(cseq, clen, _i32(c_src, dev), _i32(c_off, dev), pool_d, _i32(c_aoff, dev),
+                                             _i32(c_alen, dev), _u8([flag] * n, dev),
+                                             cseq.shape[1] + _round16(max(c_alen)), err)
+        mtok, _, _ = tok.tokenize_fixed(mseq, mlen, mseq.shape[1], typical_len=max(b - a for a, b in wins))
+        cand_c = torch.cat([ref_ctok, mtok.to(ref_ctok.dtype)])
+    else:
+        cand_c = ref_ctok
+    # ---- gene window: splice + full BPE, keep the 200-token chunks that differ from the reference item's ----
+    gseq, glen = t["gene_seq"]
+    cap = L * hot.max_chunks
+    ref_pad = torch.zeros((hot.max_chunks, L), dtype=torch.int32, device=dev)
+    ref_pad[:G_ref] = ref_gtok
+    gene_edits = [i for i, e in enumerate(edits) if e.gene_hit]
+    g_count = np.full(len(edits), G_ref, np.int64)                 # chunks of every edit item's gene window
+    g_changed = {}                                                  # edit -> bool [G_m] changed chunks
+    gene_pos = [None] * len(edits)
+    changed_rows = []
+    glen0 = int(glen[0].item()) if want_gene_pos and gene_edits else 0
+    for a in range(0, len(gene_edits), GENE_GROUP):
+        grp = gene_edits[a:a + GENE_GROUP]
+        n = len(grp)
+        offs = [edits[i].pos - 1 - g0 for i in grp]
+        mseq, mlen, err = ops.splice_windows(gseq, glen, _i32([0] * n, dev), _i32(offs, dev), pool_d,
+                                             _i32([a_off[i] for i in grp], dev), _i32([a_len[i] for i in grp], dev),
+                                             _u8([flag] * n, dev), gseq.shape[1] + _round16(max(a_len[i] for i in grp)),
+                                             err)
+        res = ops.bpe_tokenize(mseq, mlen, mseq.shape[1], tok.merges, cap, cap, want_starts=want_gene_pos)
+        gt, gc = res[0], res[1]
+        if want_gene_pos:                                           # vepdataset.py: VEPBatchBuilder.build, gene_hit
+            p = np.asarray([glen0 + a_len[i] - 1 - o - 1 if flag else o for i, o in zip(grp, offs)], np.int64)
+            p_d = torch.from_numpy(p).to(dev)
+            ch = mseq.gather(1, p_d[:, None].clamp(0, mseq.shape[1] - 1))[:, 0].cpu().numpy()
+            st = res[2]
+            valid = torch.arange(st.shape[1], device=dev)[None, :] < gc[:, None]
+            tix = ((st <= p_d[:, None]) & valid).sum(1).cpu().numpy() - 1
+            for j, i in enumerate(grp):
+                gene_pos[i] = (int(p[j]), chr(int(ch[j])), int(tix[j]))
+            del st, res
+        del mseq
+        G_m = np.minimum(hot.max_chunks, (gc.cpu().numpy().astype(np.int64) + L - 1) // L)
+        rows = gt.view(n, hot.max_chunks, L)
+        valid = torch.arange(hot.max_chunks, device=dev)[None, :] < torch.from_numpy(G_m).to(dev)[:, None]
+        changed = valid & (rows != ref_pad[None]).any(-1)
+        changed_h = changed.cpu().numpy()
+        changed_rows.append(rows[changed])
+        for j, i in enumerate(grp):
+            g_count[i] = G_m[j]
+            g_changed[i] = changed_h[j, :G_m[j]]
+    # ---- windows read without the background: the background-free reference item ----
+    tp = None
+    if variants is not None and any(e.plain_cre or e.plain_gene for e in edits):
+        tp = hot.tokenize([gene], None)
+        err = torch.maximum(err, tp["err"])
+        c_plain = cand_c.shape[0]
+        cand_c = torch.cat([cand_c, tp["cre_tok"][0].to(cand_c.dtype)])
+        changed_rows.append(tp["gene_tok"][0])
+    cand_g = torch.cat([ref_gtok] + changed_rows) if changed_rows else ref_gtok
+    _raise_on_error(err, "building the edited windows")
+    # ---- every distinct token row once ----
+    uc, inv_c = torch.unique(cand_c, dim=0, return_inverse=True)
+    ug, inv_g = torch.unique(cand_g, dim=0, return_inverse=True)
+    inv_c = inv_c.cpu().numpy().astype(np.int64); inv_g = inv_g.cpu().numpy().astype(np.int64)
+    # ---- item -> rows of the distinct tables ----
+    ref_c, ref_g = inv_c[:C], inv_g[:G_ref]
+    cre_rows, gene_rows = [ref_c], [ref_g]
+    g_next = G_ref
+    c_of = {}                                                          # (edit, window) -> row of cand_c
+    for j, (i, k) in enumerate(zip(c_owner, c_src)):
+        c_of[(i, k)] = C + j
+    if tp is not None:
+        plain_g = inv_g[cand_g.shape[0] - tp["gene_tok"][0].shape[0]:]
+    for i, e in enumerate(edits):
+        r = ref_c.copy()
+        for k in e.hits:
+            r[k] = inv_c[c_of[(i, k)]]
+        if tp is not None:
+            r[e.plain_cre] = inv_c[c_plain + np.asarray(e.plain_cre, np.int64)]
+        cre_rows.append(r)
+        if tp is not None and e.plain_gene:                  # never together with gene_hit (other chromosome)
+            gene_rows.append(plain_g)
+            g_count[i] = len(plain_g)
+        elif e.gene_hit:
+            ch = g_changed[i]
+            gr = np.empty(len(ch), np.int64)
+            n_ch = int(ch.sum())
+            gr[ch] = inv_g[g_next:g_next + n_ch]
+            keep = np.nonzero(~ch)[0]
+            gr[keep] = ref_g[keep]
+            g_next += n_ch
+            gene_rows.append(gr)
+        else:
+            gene_rows.append(ref_g)
+    out = dict(cre_tokens=uc.to(torch.int32), gene_tokens=ug.to(torch.int32), cre_rows=cre_rows, gene_rows=gene_rows,
+               labels=t["labels"][0], C=C, G_ref=G_ref, g_count=g_count)
+    if want_gene_pos:
+        out["gene_pos"] = gene_pos
+        _, gcnt, starts = ops.bpe_tokenize(gseq, glen, gseq.shape[1], tok.merges, cap, cap, want_starts=True)
+        n_tok = int(gcnt[0].item())
+        out["ref_gene"] = (gseq[0, :int(glen[0].item())].cpu().numpy().tobytes(), starts[0, :n_tok].cpu().numpy())
+        out["plain_gene"] = out["ref_gene"]
+        if tp is not None:
+            pseq, plen = tp["gene_seq"]
+            _, pcnt, pstarts = ops.bpe_tokenize(pseq, plen, pseq.shape[1], tok.merges, cap, cap, want_starts=True)
+            out["plain_gene"] = (pseq[0, :int(plen[0].item())].cpu().numpy().tobytes(),
+                                 pstarts[0, :int(pcnt[0].item())].cpu().numpy())
+    return out
 
 
 @torch.no_grad()
@@ -130,8 +294,7 @@ def build_items(hot, gene, start: int, end: int, zygosity=(2,), variants=None):
     -> dict(plan, cre_tokens int32 [n_c, L], gene_tokens int32 [n_g, L] (distinct rows, device), cre_rows / gene_rows
     (per item, reference item first: int64 rows of the item's CRE windows / gene chunks in those tables), labels,
     counters)."""
-    tok, dev = hot.tok, hot.engine.device
-    L = hot.max_length
+    tok = hot.tok
     t = hot.tokenize([gene], variants)
     off, chrom_len = hot.genome.offsets[gene.chrom]
     if not (1 <= start <= end <= chrom_len):
@@ -144,88 +307,16 @@ def build_items(hot, gene, start: int, end: int, zygosity=(2,), variants=None):
         bg_bases = rseq[0, :end - start + 1].cpu().numpy().tobytes()
     plan = plan_mutants(gene, start, end, ref_bases, bg_bases, zygosity, hot.nb, hot.up, hot.down)
     muts = plan.mutants
-    ref_ctok = t["cre_tok"][0]                                      # int32 [C, L]
-    ref_gtok = t["gene_tok"][0]                                     # int32 [G_ref, L]
-    C, G_ref = ref_ctok.shape[0], ref_gtok.shape[0]
-    g0 = plan.gene_window[0]
-    flag = int(plan.minus)
-    err = t["err"].clone()
-    # ---- CRE windows: one mutated row per (mutant, hit window), fixed 200-token rows ----
-    c_src, c_off, c_base, c_owner = [], [], [], []
-    for m_i, m in enumerate(muts):
-        for k in m.hits:
-            c_src.append(k); c_off.append(m.pos - 1 - plan.wins[k][0]); c_base.append(ord(m.base)); c_owner.append(m_i)
-    cseq, clen = t["cre_seq"]
-    if c_src:
-        n = len(c_src)
-        mseq, mlen, err = ops.mutate_windows(cseq, clen, _i32(c_src, dev), _i32(c_off, dev), _u8(c_base, dev),
-                                             _u8([flag] * n, dev), err)
-        mtok, _, _ = tok.tokenize_fixed(mseq, mlen, mseq.shape[1], typical_len=max(b - a for a, b in plan.wins))
-        cand_c = torch.cat([ref_ctok, mtok.to(ref_ctok.dtype)])
-    else:
-        cand_c = ref_ctok
-    # ---- gene window: mutate + full BPE, keep the 200-token chunks that differ from the reference item's ----
-    gseq, glen = t["gene_seq"]
-    cap = L * hot.max_chunks
-    ref_pad = torch.zeros((hot.max_chunks, L), dtype=torch.int32, device=dev)
-    ref_pad[:G_ref] = ref_gtok
-    gene_muts = [i for i, m in enumerate(muts) if m.gene_hit]
-    g_count = np.full(len(muts), G_ref, np.int64)                  # chunks of every mutant's gene window
-    g_changed = {}                                                  # mutant -> bool [G_m] changed chunks
-    changed_rows = []
-    for a in range(0, len(gene_muts), GENE_GROUP):
-        grp = gene_muts[a:a + GENE_GROUP]
-        n = len(grp)
-        mseq, mlen, err = ops.mutate_windows(gseq, glen, _i32([0] * n, dev),
-                                             _i32([muts[i].pos - 1 - g0 for i in grp], dev),
-                                             _u8([ord(muts[i].base) for i in grp], dev), _u8([flag] * n, dev), err)
-        gt, gc = ops.bpe_tokenize(mseq, mlen, mseq.shape[1], tok.merges, cap, cap)
-        del mseq
-        G_m = np.minimum(hot.max_chunks, (gc.cpu().numpy().astype(np.int64) + L - 1) // L)
-        rows = gt.view(n, hot.max_chunks, L)
-        valid = torch.arange(hot.max_chunks, device=dev)[None, :] < torch.from_numpy(G_m).to(dev)[:, None]
-        changed = valid & (rows != ref_pad[None]).any(-1)
-        changed_h = changed.cpu().numpy()
-        changed_rows.append(rows[changed])
-        for j, i in enumerate(grp):
-            g_count[i] = G_m[j]
-            g_changed[i] = changed_h[j, :G_m[j]]
-    cand_g = torch.cat([ref_gtok] + changed_rows) if changed_rows else ref_gtok
-    _raise_on_error(err, "building the mutant windows")
-    # ---- every distinct token row once ----
-    uc, inv_c = torch.unique(cand_c, dim=0, return_inverse=True)
-    ug, inv_g = torch.unique(cand_g, dim=0, return_inverse=True)
-    inv_c = inv_c.cpu().numpy().astype(np.int64); inv_g = inv_g.cpu().numpy().astype(np.int64)
-    # ---- item -> rows of the pooled tables ----
-    ref_c, ref_g = inv_c[:C], inv_g[:G_ref]
-    cre_rows, gene_rows = [ref_c], [ref_g]
-    g_next = G_ref
-    c_of = {}                                                          # (mutant, window) -> row of cand_c
-    for j, (m_i, k) in enumerate(zip(c_owner, c_src)):
-        c_of[(m_i, k)] = C + j
-    for m_i, m in enumerate(muts):
-        r = ref_c.copy()
-        for k in m.hits:
-            r[k] = inv_c[c_of[(m_i, k)]]
-        cre_rows.append(r)
-        if m.gene_hit:
-            ch = g_changed[m_i]
-            gr = np.empty(len(ch), np.int64)
-            n_ch = int(ch.sum())
-            gr[ch] = inv_g[g_next:g_next + n_ch]
-            keep = np.nonzero(~ch)[0]
-            gr[keep] = ref_g[keep]
-            g_next += n_ch
-            gene_rows.append(gr)
-        else:
-            gene_rows.append(ref_g)
+    it = build_edit_items(hot, gene, [Edit(m.pos, m.base.encode(), m.hits, m.gene_hit) for m in muts], variants, t=t)
+    C, G_ref, g_count = it["C"], it["G_ref"], it["g_count"]
     # windows the per-variant path encodes for the same items: per variant its reference item, plus every requested
     # zygosity item (it also encodes the zygosity not asked for; not counted)
     per_variant = sum(C + int(g_count[i]) for i in range(len(muts))) + \
         len({(m.pos, m.alt) for m in muts}) * (C + G_ref)
     zyg_n = len(set(int(z) for z in zygosity))
-    return dict(plan=plan, cre_tokens=uc.to(torch.int32), gene_tokens=ug.to(torch.int32), cre_rows=cre_rows,
-                gene_rows=gene_rows, labels=t["labels"][0],
+    uc, ug = it["cre_tokens"], it["gene_tokens"]
+    return dict(plan=plan, cre_tokens=uc, gene_tokens=ug, cre_rows=it["cre_rows"], gene_rows=it["gene_rows"],
+                labels=it["labels"],
                 counters=dict(windows_encoded=int(uc.shape[0] + ug.shape[0]), cre_windows_encoded=int(uc.shape[0]),
                               gene_chunks_encoded=int(ug.shape[0]), windows_per_variant=int(per_variant),
                               skipped={k: 3 * zyg_n * len(v) for k, v in plan.skipped.items()}))

@@ -187,6 +187,17 @@ def seq2gene_forward(table, slab, cre_pooled, gene_pooled, workspace, n_reg, n_t
     return pred, emb, gtok, ctok
 
 
+def seq2gene_cre_rows(table, slab, workspace, rows, D):
+    """Rows of the final CRE stream of the seq2gene_forward call that just ran on this stream with the same slab and
+    workspace (vf_seq2gene_cre_rows).  rows int32 [n] device tensor -> fp32 [n, D] (un-centred)."""
+    import ctypes as C
+    out = torch.empty((rows.numel(), D), dtype=torch.float32, device=rows.device)
+    if rows.numel():
+        check(_lib.lib().vf_seq2gene_cre_rows(C.addressof(table), C.addressof(slab), ptr(workspace), workspace.numel(),
+                                              ptr(rows), rows.numel(), ptr(out), stream()))
+    return out
+
+
 def cu_seqlens(lens, device):
     cu = np.zeros(len(lens) + 1, np.int32)
     np.cumsum(np.asarray(lens, np.int64), out=cu[1:])
@@ -456,6 +467,31 @@ def mutate_windows(src, src_len, row_src, row_off, row_base, flags, err=None):
             check(_lib.lib().vf_mutate_windows(ptr(src), pitch, ptr(src_len), ptr(row_src[r0:r1]), ptr(row_off[r0:r1]),
                                                ptr(row_base[r0:r1]), ptr(flags[r0:r1]), r1 - r0, ptr(out[r0:r1]), pitch,
                                                ptr(out_len[r0:r1]), ptr(err), stream()))
+    return out, out_len, err
+
+
+def splice_windows(src, src_len, row_src, row_off, allele_pool, allele_off, allele_len, flags, out_pitch, err=None):
+    """Allele splices of encoded windows (vf_splice_windows): row r = src[row_src[r]] with the ONE base at forward-strand
+    offset row_off[r] replaced by allele_pool[allele_off[r], + allele_len[r]) (reverse complement of the allele on
+    reverse-complemented rows, flags bit 0); the row grows by allele_len[r] - 1 bytes.  src uint8 [n_src, pitch] and
+    src_len int32 [n_src] as encode_windows returns them; row_src / row_off / allele_off / allele_len int32, flags uint8
+    [n_rows], allele_pool uint8 device tensors; out_pitch: a multiple of 16 that holds the longest output row.
+    -> (out uint8 [n_rows, out_pitch], out_len int32 [n_rows], err)."""
+    n = row_src.numel()
+    dev = src.device
+    assert src.dtype == torch.uint8 and src.is_contiguous() and src_len.dtype == torch.int32 and out_pitch % 16 == 0
+    for t in (row_src, row_off, allele_off, allele_len):
+        assert t.dtype == torch.int32 and t.numel() == n
+    assert allele_pool.dtype == torch.uint8 and flags.dtype == torch.uint8 and flags.numel() == n
+    out = torch.empty((n, out_pitch), dtype=torch.uint8, device=dev)
+    out_len = torch.empty(n, dtype=torch.int32, device=dev)
+    if err is None:
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+    if n:
+        with _timed("stage1_splice", nbytes=2.0 * n * out_pitch):      # row bytes read + written (upper bound)
+            check(_lib.lib().vf_splice_windows(ptr(src), src.shape[1], ptr(src_len), ptr(row_src), ptr(row_off),
+                                               ptr(allele_pool), ptr(allele_off), ptr(allele_len), ptr(flags), n,
+                                               ptr(out), out_pitch, ptr(out_len), ptr(err), stream()))
     return out, out_len, err
 
 

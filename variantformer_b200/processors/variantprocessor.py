@@ -108,6 +108,28 @@ class VariantProcessor:
         df.to_parquet(self.output_file)
         return df
 
+    def predict_batched(self, var_df: pd.DataFrame, output_dir: str, vcf_path: str = None, sample_name: str = None,
+                        rows_budget=None):
+        """`predict` with the same arguments, skip rules, errors, output file and returned DataFrame, computed in shared
+        batched passes (variantformer_b200.vep_batch): each (gene, tissue list) encodes its reference item once,
+        duplicate edits are scored once, and every distinct window goes through seq2reg once.  rows_budget: CRE rows per
+        slab (default ism.ROWS_BUDGET)."""
+        from .. import ism, vep_batch
+        from ..pipeline import HotPath
+        from ..stage1 import SampleVariants
+        pairs, model, _, _ = self.initialize(var_df, output_dir, vcf_path, sample_name)
+        ds = self.model_config.dataset
+        hot = HotPath(model.engine(), self._genome, max_length=ds.max_length, max_chunks=ds.max_chunks,
+                      cre_neighbour_hood=ds.cre_neighbour_hood, gene_upstream=ds.gene_upstream_neighbour_hood,
+                      gene_downstream=ds.gene_downstream_neighbour_hood)
+        bg = None
+        if self.background:                                   # the sample contributes SNPs only (variant_type="SNP")
+            bg = SampleVariants({c: VEPBatchBuilder._snps_only(b) for c, b in self.background.items()}, "cuda")
+        predictions, _ = vep_batch.score_pairs(hot, pairs, bg, rows_budget or ism.ROWS_BUDGET)
+        df = self.compile_predictions(pairs, predictions)
+        df.to_parquet(self.output_file)
+        return df
+
     def saturation_mutagenesis(self, gene_id, tissues, start, end, vcf_path=None, sample_name=None, zygosity=(2,)):
         """In-silico saturation mutagenesis of [start, end] (1-based, inclusive, on the gene's chromosome): every
         single-base substitution, scored as `predict` scores Variant(chrom, pos, ref, alt) for this gene, in batched
