@@ -54,6 +54,11 @@ enum {
  * seq2gene/modules/layers.py:63-80 + flash_attn MHA Wqkv/Wq/Wkv/out_proj;
  * seq2gene/model_combined_modulator.py:502-507,610-612; seq2gene/modules/layers.py:1078-1087.
  * N % 8 == 0, K % 8 == 0, 16-byte aligned operands.  bias/resid/out2 may be NULL.
+ * Alignment: A, W, out, out2_bf16 and resid 16-byte aligned; lda, ldw, ldo, ldo2 multiples of 8 elements; ldr a
+ * multiple of 4 elements (fp32 residual) or of 8 (bf16 residual); stats_out and ln_stats (vf_gemm_bf16_ln) 8-byte
+ * aligned, ln_stats 16-byte aligned when ln_parts is even and at most 16.  A violation returns an error and launches
+ * nothing; the operands the epilogue writes or reads (out, out2, resid, stats_out, ln_stats) are checked even when
+ * M == 0.
  */
 int vf_gemm_bf16(const void* A, int lda, const void* W, int ldw, int M, int N, int K, int epilogue,
                  const float* bias, const float* resid, int ldr, void* out, int ldo, void* out2_bf16, int ldo2,

@@ -1079,6 +1079,21 @@ int gemm_bf16(const void* A, int lda, const void* W, int ldw, int M, int N, int 
         g_inited = true;
     }
     VF_REQUIRE(M >= 0 && N > 0 && K > 0, "gemm: bad shape M=%d N=%d K=%d", M, N, K);
+    // Every operand the epilogue writes or reads with vector accesses (uint4 / float4 rows of out, uint2 of the mirror
+    // and of a bf16 residual, float2 statistics, float4 batches of the LayerNorm partials) must be aligned for them: a
+    // misaligned view is an error here, not a misaligned-address fault in the kernel.  Checked before the M == 0 return
+    // so that a caller's bad view is reported whatever its row count.
+    const auto misaligned = [](const void* q, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(q) & (bytes - 1)) != 0; };
+    VF_REQUIRE(!misaligned(out, 16), "gemm: output must be 16-byte aligned");
+    VF_REQUIRE(!misaligned(out2, 16) && (!out2 || ldo2 % 8 == 0),
+               "gemm: bf16 mirror must be 16-byte aligned with a row stride that is a multiple of 8 elements (ldo2=%d)", ldo2);
+    VF_REQUIRE(!misaligned(resid, 16) && (!resid || ldr % (resid_bf16 ? 8 : 4) == 0),
+               "gemm: residual must be 16-byte aligned with a row stride that is a multiple of 16 bytes (ldr=%d)", ldr);
+    VF_REQUIRE(!misaligned(stats_out, 8), "gemm: stats_out must be 8-byte aligned");
+    // (the epilogue reads a row's partials as float4 batches when 2 <= ln_parts <= 16 and ln_parts is even)
+    VF_REQUIRE(!misaligned(ln_stats, ln_parts > 1 && ln_parts <= 16 && ln_parts % 2 == 0 ? 16 : 8),
+               "gemm: ln_stats must be 8-byte aligned (16-byte for an even partial count of 2 to 16: such rows are read as "
+               "float4)");
     if (M == 0) return 0;
     VF_REQUIRE(N % 8 == 0 && K % 8 == 0, "gemm: N and K must be multiples of 8 (N=%d K=%d)", N, K);
     VF_REQUIRE(epi >= 0 && epi < VF_EPI_COUNT, "gemm: unknown epilogue %d", epi);
@@ -1123,25 +1138,21 @@ int gemm_bf16(const void* A, int lda, const void* W, int ldw, int M, int N, int 
     } else {
         tr = ta;                                                       // never dereferenced
     }
-    // bf16 epilogues store through TMA (VF_GEMM_TMA_STORE=0: per-lane stores, for A/B runs); needs a 16-byte aligned
-    // output whose row stride keeps 16-byte alignment
+    // bf16 epilogues store through TMA (VF_GEMM_TMA_STORE=0: per-lane stores, for A/B runs); out and ldo were checked
+    // above for the 16-byte alignment both paths need
     CUtensorMap to = ta;
     p.tma_store = 0;
-    if (out_bf16 && g_tma_store && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (ldo % 8) == 0) {
+    if (out_bf16 && g_tma_store) {
         if (make_tmap_out_bf16(&to, out, M, n_out, ldo)) return -1;
         p.tma_store = 1;
     }
-    if (pair && (g_rt & 1) && epi == VF_EPI_BIAS_RESID_F32 && resid_bf16 && !out && out2 && N % BN == 0 &&
-        (reinterpret_cast<uintptr_t>(resid) & 15) == 0 && (ldr % 8) == 0 && (reinterpret_cast<uintptr_t>(out2) & 15) == 0 &&
-        (ldo2 % 8) == 0) {
+    if (pair && (g_rt & 1) && epi == VF_EPI_BIAS_RESID_F32 && resid_bf16 && !out && out2 && N % BN == 0) {
         // out_proj shape: bf16 residual in, bf16 mirror + row statistics out -> TMA-staged epilogue (see kGemmSmemRT)
         if (make_tmap_out_bf16(&tr, const_cast<void*>(resid), M, N, ldr)) return -1;
         if (make_tmap_out_bf16(&to, out2, M, N, ldo2)) return -1;
         return launch_tc_pair<VF_EPI_BIAS_RESID_F32, 1>(ta, tb, tr, to, p, stream);
     }
-    if (pair && (g_rt & 2) && epi == VF_EPI_BIAS_RESID_F32 && resid && !resid_bf16 && out == resid && ldo == ldr && N % BN == 0 &&
-        (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (ldo % 4) == 0 &&
-        (!out2 || ((reinterpret_cast<uintptr_t>(out2) & 15) == 0 && (ldo2 % 8) == 0))) {
+    if (pair && (g_rt & 2) && epi == VF_EPI_BIAS_RESID_F32 && resid && !resid_bf16 && out == resid && ldo == ldr && N % BN == 0) {
         // FFN2 form, in place on the fp32 stream (+ mirror, statistics)
         if (make_tmap_slab_f32(&tr, out, M, N, ldo)) return -1;
         if (out2 && make_tmap_out_bf16(&to, out2, M, N, ldo2)) return -1;
