@@ -112,6 +112,24 @@ int vf_attention_mc_varlen(const void* q, int ldq, const void* k, int ldk, const
                            int head_dim, const float* slopes, void* stream);
 
 /*
+ * Attention probabilities of a cross-attention for selected query rows (no positional bias), fp32:
+ *   out[out_off[i] + (layer * heads + h) * n_keys + c] = softmax_c( q[row_i, h] . k[first_key + c, h] / sqrt(head_dim) )
+ * for every query index i of group g (i in [group_q[2g], group_q[2g] + group_q[2g+1])), head h and key c in
+ * [0, n_keys), where (first_key, n_keys) = (group_k[2g], group_k[2g+1]) and row_i = q_rows[i] (q_rows NULL: row_i = i).
+ * Scores and softmax in fp32 over the whole key range (exact maximum, no lazy rescaling); bf16 operands as the fused
+ * kernel reads them.  Per prediction the blocks of all layers form one [n_layers, heads, n_keys] array at out_off[i].
+ * q / k: bf16, head h at columns [h*head_dim, (h+1)*head_dim) of each row (k: the K half of a packed KV buffer).
+ * Groups of any size (64 query rows share one K stream); a group with <= 0 rows or keys writes nothing.  One CTA per
+ * (group, head), CUDA cores.  Errors before any launch: head_dim not in {48, 64}, n_groups / layer < 0, heads not in
+ * [1, 65535], q or k not 16-byte aligned, ldq / ldk not multiples of 8 or < heads * head_dim, out / q_rows / group
+ * tables not 4-byte aligned, out_off not 8-byte aligned.
+ * Serves the gene -> CRE cross-attention maps (seq2gene/modules/layers.py:142-150 with the gene stream as query).
+ */
+int vf_cross_attention_probs(const void* q, int ldq, const int32_t* q_rows, const int32_t* group_q, int n_groups,
+                             const void* k, int ldk, const int32_t* group_k, int heads, int head_dim, float* out,
+                             const int64_t* out_off, int layer, void* stream);
+
+/*
  * CRE x reference-label cross-attention collapsed to the 9 cCRE classes (exact identity):
  * q bf16 [n_rows, H*HD]; kv9 fp32 [9, 2*H*HD] = Wkv·Emb9 + b ((two,h,d) order); logc fp32 [n_seq,9] =
  * log(#CREs of the class in the row's gene) (-inf when absent); row_seq int32 [n_rows].
@@ -327,6 +345,30 @@ size_t vf_seq2gene_workspace_bytes(const vf_seq2gene_weights_t* w, const vf_seq2
 int vf_seq2gene_forward(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t* slab, const void* cre_pooled_bf16,
                         const void* gene_pooled_bf16, void* workspace, size_t workspace_bytes, float* pred, float* emb,
                         float* gene_token_emb, float* cre_token_emb, void* stream);
+/*
+ * Gene -> CRE cross-attention maps of one slab (vf_cross_attention_probs layout): one group per gene, its predictions'
+ * registry rows as queries, its CREs as keys.  group_q int32 [n_groups][2] = {first prediction, predictions} (index
+ * into the n_reg predictions / the registry rows of the slab, in gene-stream order); group_k int32 [n_groups][2] =
+ * {first CRE row, CREs}; reg_rows int32 [n_reg] = gene-stream row of every prediction's registry token; out fp32,
+ * out_off int64 [n_reg] = start of each prediction's [n_layers, heads, CREs] block.
+ */
+typedef struct {
+    int n_groups;
+    const int32_t* group_q;
+    const int32_t* group_k;
+    const int32_t* reg_rows;
+    float* out;
+    const int64_t* out_off;
+} vf_cre_attention_t;
+/*
+ * vf_seq2gene_forward that also writes the maps: after the cross-attention of every gene layer, on the caller's stream,
+ * one vf_cross_attention_probs launch on the layer's queries (the registry rows of the query buffer; the pruned last
+ * layer's query rows, whose first n_reg are the registry rows).  Same workspace, same launches otherwise: pred, emb and
+ * the token embeddings are bit-identical to vf_seq2gene_forward.  attn NULL = vf_seq2gene_forward.
+ */
+int vf_seq2gene_forward_attn(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t* slab, const void* cre_pooled_bf16,
+                             const void* gene_pooled_bf16, void* workspace, size_t workspace_bytes, float* pred, float* emb,
+                             float* gene_token_emb, float* cre_token_emb, const vf_cre_attention_t* attn, void* stream);
 /*
  * HOST helper: work table of vf_attention_mc_varlen for n_seq sequences of q_lens query rows and k_lens keys (NULL =
  * self-attention), rows packed back to back.  out_table: HOST int32 [max_items][2][8] (NULL: only count).  Consecutive

@@ -1,5 +1,5 @@
 """ctypes mirrors of the weight-pointer / slab tables of the coarse entry points (include/vf_b200.h:
-vf_seq2reg_forward, vf_seq2gene_forward) and their builders from the engine's device-side weight objects."""
+vf_seq2reg_forward, vf_seq2gene_forward, vf_seq2gene_forward_attn) and their builders from the engine's device-side weight objects."""
 import ctypes as C
 
 _vp, _i, _f = C.c_void_p, C.c_int, C.c_float
@@ -37,6 +37,10 @@ class Seq2GeneSlab(C.Structure):
                 ("slots_gself", _vp), ("n_gself", _i), ("slots_gcross", _vp), ("n_gcross", _i),
                 ("slots_cself", _vp), ("n_cself", _i), ("slots_last_self", _vp), ("n_last_self", _i),
                 ("slots_last_cross", _vp), ("n_last_cross", _i)]
+
+
+class CreAttention(C.Structure):
+    _fields_ = [("n_groups", _i), ("group_q", _vp), ("group_k", _vp), ("reg_rows", _vp), ("out", _vp), ("out_off", _vp)]
 
 
 def _ptr(t):

@@ -25,6 +25,7 @@ SIGNATURES = {
     "vf_seq2reg_forward": ([_vp, _vp, _vp, _vp, _i32, _i32, _i64, _vp, _i32, _vp, _sz, _vp, _vp], _i32),
     "vf_seq2gene_workspace_bytes": ([_vp, _vp], _sz),
     "vf_seq2gene_forward": ([_vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp], _i32),
+    "vf_seq2gene_forward_attn": ([_vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp, _vp], _i32),
     "vf_seq2gene_cre_rows": ([_vp, _vp, _vp, _sz, _vp, _i32, _vp, _vp], _i32),
     "vf_device_check": ([_vp], _i32),
     "vf_gemm_bf16": ([_vp, _i32, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _i32, _vp, _i32, _vp], _i32),
@@ -33,6 +34,7 @@ SIGNATURES = {
     "vf_rowstats": ([_vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp], _i32),
     "vf_attention_mc_varlen": ([_vp, _i32, _vp, _i32, _vp, _i32, _vp, _i32, _i64, _i64, _vp, _i32, _i32, _i32, _vp,
                                 _vp], _i32),
+    "vf_cross_attention_probs": ([_vp, _i32, _vp, _vp, _i32, _vp, _i32, _vp, _i32, _i32, _vp, _vp, _i32, _vp], _i32),
     "vf_label_attention": ([_vp, _i32, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _i32, _vp], _i32),
     "vf_layernorm": ([_vp, _i32, _vp, _vp, _i32, _i32, C.c_float, _vp, _i32, _i32, _vp], _i32),
     "vf_window_lengths": ([_vp, _i32, _i32, _vp, _vp], _i32),

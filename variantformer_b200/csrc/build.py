@@ -7,7 +7,8 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["vf_api.cu", "vf_gemm.cu", "vf_attention_mc.cu", "vf_elementwise.cu", "vf_encode.cu", "vf_forward.cu"]
+SOURCES = ["vf_api.cu", "vf_gemm.cu", "vf_attention_mc.cu", "vf_elementwise.cu", "vf_encode.cu", "vf_forward.cu",
+           "vf_attn_probs.cu"]
 HEADERS = ["vf_common.cuh", "vf_internal.h", os.path.join("..", "..", "include", "vf_b200.h")]
 LIB = os.path.join(HERE, "libvf_b200.so")
 INGEST_SRC = os.path.join(HERE, "vf_ingest.cpp")

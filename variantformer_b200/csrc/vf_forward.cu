@@ -175,15 +175,28 @@ static SideStream& side_stream(int n_events) {
 
 static int seq2gene_forward(const vf_seq2gene_weights_t& w, const vf_seq2gene_slab_t& t, const void* cre_pooled,
                             const void* gene_pooled, void* ws, size_t ws_bytes, float* pred, float* emb,
-                            float* gene_token_emb, float* cre_token_emb, cudaStream_t main) {
+                            float* gene_token_emb, float* cre_token_emb, const vf_cre_attention_t* attn, cudaStream_t main) {
     VF_REQUIRE(w.cre_layers && w.gene_layers && w.n_layers >= 1 && w.D % w.heads == 0, "seq2gene_forward: incomplete weight table");
     VF_REQUIRE(t.n_need >= t.n_reg && t.n_reg > 0 && t.n_cre > 0 && t.n_gene_rows > 0, "seq2gene_forward: empty slab");
+    if (attn) {
+        VF_REQUIRE(attn->n_groups >= 0 && attn->group_q && attn->group_k && attn->reg_rows && attn->out && attn->out_off,
+                   "seq2gene_forward: incomplete CRE attention table");
+        VF_REQUIRE((reinterpret_cast<uintptr_t>(attn->out) & 3) == 0 && (reinterpret_cast<uintptr_t>(attn->out_off) & 7) == 0,
+                   "seq2gene_forward: CRE attention out / out_off misaligned");
+    }
     Seq2GeneWs b = carve_seq2gene(w, t, ws);
     VF_REQUIRE(ws && ws_bytes >= b.bytes, "seq2gene_forward: workspace of %zu bytes < %zu needed", ws_bytes, b.bytes);
     VF_REQUIRE((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "seq2gene_forward: workspace must be 256-byte aligned");
     const int D = w.D, H = w.heads, hd = D / H, P = stats_parts(D), NL = w.n_layers, F = w.ffn_hidden;
     const int nC = t.n_cre, Mg = t.n_gene_rows, R = t.n_need, n_reg = t.n_reg;
     int rc;
+    // the cross-attention maps of gene layer `layer` from the queries the attention kernel just read (q_rows NULL: the
+    // pruned last layer's query rows, registry rows first)
+    auto maps = [&](const bf16* q, int ldq, const int32_t* q_rows, const bf16* k, int layer) {
+        if (!attn) return 0;
+        return cross_attention_probs(q, ldq, q_rows, attn->group_q, attn->n_groups, k, 2 * D, attn->group_k, H, hd, attn->out,
+                                     attn->out_off, layer, main);
+    };
     // ---- stream set-up: cre_map (raw bf16 copy = context of gene layer 0), gene_map + registry gather, row centring ----
     if ((rc = linear(w.cre_map, cre_pooled, w.token_dim, nC, D, w.token_dim, VF_EPI_BIAS_F32, nullptr, 0, 0, b.cx, D, b.ctx, D,
                      nullptr, 0, 0.f, nullptr, main))) return rc;
@@ -239,8 +252,11 @@ static int seq2gene_forward(const vf_seq2gene_weights_t& w, const vf_seq2gene_sl
             if ((rc = context_layer(w.gene_layers[i], w, b.gx, b.gxb, gxs, gxs_parts, Mg, b.gs,
                 [&](bf16* qkv, bf16* o) { return attention_mc_varlen(qkv, 3 * D, qkv + D, 3 * D, qkv + 2 * D, 3 * D, o, D, Mg, Mg,
                                                                      t.slots_gself, t.n_gself, H, hd, w.slopes, main); },
-                [&](bf16* q, bf16* o) { return attention_mc_varlen(q, 3 * D, kv, 2 * D, kv + D, 2 * D, o, D, Mg, nC,
-                                                                   t.slots_gcross, t.n_gcross, H, hd, nullptr, main); },
+                [&](bf16* q, bf16* o) {
+                    int r2 = attention_mc_varlen(q, 3 * D, kv, 2 * D, kv + D, 2 * D, o, D, Mg, nC, t.slots_gcross, t.n_gcross, H,
+                                                 hd, nullptr, main);
+                    return r2 ? r2 : maps(q, 3 * D, attn ? attn->reg_rows : nullptr, kv, i);
+                },
                 &out_stats, main))) return rc;
             gxs = out_stats; gxs_parts = P;
         }
@@ -269,6 +285,7 @@ static int seq2gene_forward(const vf_seq2gene_weights_t& w, const vf_seq2gene_sl
         bf16* kv = kv_of(NL - 1);
         if ((rc = attention_mc_varlen(b.qR, D, kv, 2 * D, kv + D, 2 * D, b.aR, D, R, nC, t.slots_last_cross, t.n_last_cross, H, hd,
                                       nullptr, main))) return rc;
+        if ((rc = maps(b.qR, D, nullptr, kv, NL - 1))) return rc;
         if ((rc = linear(L.out2, b.aR, D, R, D, D, VF_EPI_BIAS_RESID_F32, b.hbR, 1, D, nullptr, 0, b.hbR, D, nullptr, 0, 0.f, b.s1R,
                          main))) return rc;
         if ((rc = linear(L.g1, b.hbR, D, R, F, D, VF_EPI_BIAS_GEGLU_BF16, nullptr, 0, 0, b.fR, F / 2, nullptr, 0, b.s1R, P, w.ln_eps,
@@ -378,7 +395,15 @@ int vf_seq2gene_forward(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t
                         float* gene_token_emb, float* cre_token_emb, void* stream) {
     VF_REQUIRE(w && slab, "seq2gene_forward: NULL weight table / slab");
     return seq2gene_forward(*w, *slab, cre_pooled_bf16, gene_pooled_bf16, workspace, workspace_bytes, pred, emb, gene_token_emb,
-                            cre_token_emb, ST(stream));
+                            cre_token_emb, nullptr, ST(stream));
+}
+
+int vf_seq2gene_forward_attn(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t* slab, const void* cre_pooled_bf16,
+                             const void* gene_pooled_bf16, void* workspace, size_t workspace_bytes, float* pred, float* emb,
+                             float* gene_token_emb, float* cre_token_emb, const vf_cre_attention_t* attn, void* stream) {
+    VF_REQUIRE(w && slab, "seq2gene_forward: NULL weight table / slab");
+    return seq2gene_forward(*w, *slab, cre_pooled_bf16, gene_pooled_bf16, workspace, workspace_bytes, pred, emb, gene_token_emb,
+                            cre_token_emb, attn, ST(stream));
 }
 
 int vf_seq2gene_cre_rows(const vf_seq2gene_weights_t* w, const vf_seq2gene_slab_t* slab, void* workspace,

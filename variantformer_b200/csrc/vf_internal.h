@@ -16,6 +16,10 @@ int attention_mc_varlen(const void* q, int ldq, const void* k, int ldk, const vo
                         long rows_q, long rows_k, const int* slots, int n_items, int heads, int head_dim,
                         const float* slopes, cudaStream_t stream);
 
+int cross_attention_probs(const void* q, int ldq, const int32_t* q_rows, const int32_t* group_q, int n_groups, const void* k,
+                          int ldk, const int32_t* group_k, int heads, int head_dim, float* out, const int64_t* out_off,
+                          int layer, cudaStream_t s);
+
 int layernorm(const float* x, int ldx, const float* gamma, const float* beta, int M, int d, float eps, void* out,
               int ldo, int act_gelu, cudaStream_t s);
 int rowstats(const float* x, int ldx, int M, int d, float* stats, void* out_bf16, int ldo, cudaStream_t s);

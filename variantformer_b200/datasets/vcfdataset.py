@@ -114,16 +114,24 @@ class VCFDataset(Dataset):
     def _get_gene_info(self, gene_id: str) -> dict:
         return self.gencode_v24[self.gencode_v24["gene_id"] == gene_id].iloc[0].to_dict()
 
+    def cre_manifest(self, gene_id, gene_info=None):
+        """The gene's CRE manifest (chromosome, start_cre, end_cre, cre_name) and its batch order: manifest row of the
+        k-th CRE window of the item (sorted by start, reversed for '-' genes)."""
+        gene_info = gene_info or self._get_gene_info(gene_id)
+        m = pd.read_csv(self.gene_cre_manifest.get_file_path(gene_id))
+        w = [cre_window(s, e, self.cre_neighbour_hood) for s, e in zip(m["start_cre"], m["end_cre"])]
+        order = np.argsort(np.asarray([x[0] for x in w]), kind="stable")      # process_subject sorts by start_cre
+        if gene_info["strand"] == "-":
+            order = order[::-1]
+        return m, order
+
     def _get_cres(self, gene_id, gene_info, vcf_path):
         """vcfdataset.py:219-283: CRE windows [start-50, end+50) sorted by start, reversed + reverse-complemented for
         '-' genes, tokenised, padded/truncated to max_length."""
-        m = pd.read_csv(self.gene_cre_manifest.get_file_path(gene_id))
+        m, order = self.cre_manifest(gene_id, gene_info)
         m = m.rename(columns={"chromosome": "chrom", "start_cre": "start", "end_cre": "end", "cre_name": "cCRE"})
         w = [cre_window(s, e, self.cre_neighbour_hood) for s, e in zip(m["start"], m["end"])]
-        order = np.argsort(np.asarray([x[0] for x in w]), kind="stable")      # process_subject sorts by start_cre
         minus = gene_info["strand"] == "-"
-        if minus:
-            order = order[::-1]
         chroms = [m["chrom"].iloc[i] for i in order]
         w0 = [w[i][0] for i in order]; w1 = [w[i][1] for i in order]
         seq, lens, err = self.tokenizer.sequences(self._genome(), chroms, w0, w1, [int(minus)] * len(order),

@@ -65,6 +65,19 @@ class AttnPlan:
         return ops.attention_mc(q, k, v, self.slots, heads, head_dim, slopes, out=out)
 
 
+def cre_attention_layout(T, C, n_layers, heads):
+    """Layout of the gene -> CRE cross-attention maps of a slab (one group per gene: its T[g] predictions, in gene-stream
+    order, against its C[g] CREs).  -> (group_q int32 [B, 2] = (first prediction, predictions), group_k int32 [B, 2] =
+    (first CRE row, CREs), out_off int64 [sum T] = start of each prediction's [n_layers, heads, C[g]] block, total
+    floats)."""
+    T = np.asarray(T, np.int64); C = np.asarray(C, np.int64)
+    group_q = np.stack([np.cumsum(T) - T, T], 1).astype(np.int32)
+    group_k = np.stack([np.cumsum(C) - C, C], 1).astype(np.int32)
+    size = np.repeat(C, T) * (n_layers * heads)
+    out_off = np.cumsum(size) - size
+    return group_q, group_k, out_off.astype(np.int64), int(size.sum())
+
+
 def sinusoidal_pe(d_model: int, length: int) -> torch.Tensor:
     """Same arithmetic as seq2reg/model.py:15-37 (computed once on the host in fp32)."""
     pe = torch.zeros(length, d_model)
@@ -319,10 +332,12 @@ class Engine:
         return xs_out
 
     # ---------------------------------------------------------------- last gene layer, needed rows only
-    def _gene_layer_last(self, L, s, x, xb, xs, kv):
+    def _gene_layer_last(self, L, s, x, xb, xs, kv, maps=None):
         """The last ContextFlashAttentionEncoderLayer of the gene stream restricted to the rows whose output is read
         (registry rows + VEP token rows): K/V of the self-attention still come from every row, all the rest runs on
-        `need` rows.  Same arithmetic as _layer on those rows.  -> fp32 [n_need, D], still row-centred."""
+        `need` rows.  Same arithmetic as _layer on those rows.  maps(q, q_rows, kv, layer): optional writer of the
+        cross-attention maps, called with the layer's queries (registry rows first).  -> fp32 [n_need, D], still
+        row-centred."""
         ws, w = self.ws, self.w
         D, H, hd = w.D, w.H, w.hd
         M, R = x.shape[0], s["n_need"]
@@ -343,6 +358,8 @@ class Engine:
                  stats_out=s1, mirror_only=True)
         ops.gemm(hb, L["q"].w, EPI_BIAS_BF16, bias=L["q"].b, out=q, ln=L["q"].ln(s1))
         s["plan_last_cross"].run(q, kv[:, :D], kv[:, D:], H, hd, None, a)
+        if maps is not None:
+            maps(q, None, kv, w.NL - 1)
         ops.gemm(a, L["out2"].w, EPI_BIAS_RESID_F32, bias=L["out2"].b, resid=hb, out2=hb, stats_out=s1, mirror_only=True)
         f = ops.gemm(hb, L["g1"].w, EPI_BIAS_GEGLU_BF16, bias=L["g1"].b, ln=L["g1"].ln(s1))
         return ops.gemm(f, L["g2"].w, EPI_BIAS_RESID_F32, bias=L["g2"].b, resid=xR, out=xR)
@@ -472,9 +489,10 @@ class Engine:
 
     # ---------------------------------------------------------------- device work for one prepared slab
     @torch.no_grad()
-    def run(self, s):
-        """-> dict(pred fp32 [sum T], emb fp32 [sum T, D], T list, optional token embeddings); device tensors."""
-        return self.run_pooled(s, *self.pool_windows(s))
+    def run(self, s, cre_attention=False):
+        """-> dict(pred fp32 [sum T], emb fp32 [sum T, D], T list, optional token embeddings); device tensors.
+        cre_attention: also return the gene -> CRE cross-attention maps (run_pooled)."""
+        return self.run_pooled(s, *self.pool_windows(s), cre_attention=cre_attention)
 
     @torch.no_grad()
     def pool_windows(self, s):
@@ -484,17 +502,31 @@ class Engine:
         gene_pooled = self.seq2reg(self.gene_tok, s["gtok"], s["gmsk"], s["glens"], s["g_cu_tok"], s["g_plan_tok"])
         return cre_pooled, gene_pooled
 
+    def _cre_attention(self, s):
+        """Device tables of the slab's cross-attention maps (built once per slab) and a fresh output buffer."""
+        if "attn_tables" not in s:
+            gq, gk, off, total = cre_attention_layout(s["T"], s["C"], self.w.NL, self.w.H)
+            up = lambda a: torch.from_numpy(a).to(self.device, non_blocking=True)
+            s["attn_tables"] = (up(gq), up(gk), up(off), off, total)
+        gq, gk, off, off_host, total = s["attn_tables"]
+        return gq, gk, off, off_host, torch.empty(total, dtype=torch.float32, device=self.device)
+
     @torch.no_grad()
-    def run_pooled(self, s, cre_pooled, gene_pooled):
+    def run_pooled(self, s, cre_pooled, gene_pooled, cre_attention=False):
         """Stages 3-4 of a slab from its pooled window vectors (pool_windows, or the unique windows of a slab built by
-        prepare_shared).  -> the dict of `run`."""
+        prepare_shared).  -> the dict of `run`.
+        cre_attention: also return the gene -> CRE cross-attention maps of every prediction r (DESIGN.md section 13):
+        out["cre_attention"] = flat fp32 device tensor, out["cre_attention_off"] = int64 numpy [sum T]; the block of r
+        at out_off[r] is [n_layers, heads, C of r's gene] = softmax over the gene's CREs (batch order) of the scaled
+        scores of r's registry-row query at every gene layer.  The other outputs are bit-identical to a run without."""
         w, ws = self.w, self.ws
         D, H, hd = w.D, w.H, w.hd
         nC, Mg = int(s["C"].sum()), s["Mg"]
         if "cre_rows" in s:                                  # shared windows: each item's CRE rows (1 KB per row)
             cre_pooled = cre_pooled.index_select(0, s["cre_rows"])
+        attn = self._cre_attention(s) if cre_attention else None
         if COARSE and ops.PROFILER is None and w.cre_map is not None:
-            return self._run_coarse(s, cre_pooled, gene_pooled)
+            return self._run_coarse(s, cre_pooled, gene_pooled, attn)
         if w.cre_map is None:
             raise NotImplementedError("token_dim == emb_dim (no cre_map) is not wired on the B200 path")
         # Both streams are row-centred (see the module docstring): cx / gx hold x - pivot_r, cxb / gxb their bf16 mirrors.
@@ -525,11 +557,18 @@ class Engine:
             L = w.gene_layers[i]
             ops.gemm(ctx, L["kv"].w, EPI_BIAS_BF16, bias=L["kv"].b, out=kvs[i])          # shared by every tissue copy
 
+        maps = None
+        if attn is not None:
+            def maps(q, q_rows, kv, layer):                  # right after the layer's cross-attention read q
+                ops.cross_attention_probs(q, kv[:, :D], q_rows, attn[0], attn[1], H, hd, attn[4], attn[2], layer)
+
         def gene_layer(i):
             L, kv = w.gene_layers[i], kvs[i]
 
             def cross(q, out):
                 s["plan_gcross"].run(q, kv[:, :D], kv[:, D:], H, hd, None, out)
+                if maps is not None:
+                    maps(q, s["reg_idx"], kv, i)
             st["g"] = self._layer(L, gx, gxb, st["g"], Mg, gene_self, cross, "g")
 
         def cre_layer(i):
@@ -574,7 +613,7 @@ class Engine:
                 gene_layer(i)
         n_reg = s["reg_idx"].numel()
         if prune_last:
-            last = self._gene_layer_last(w.gene_layers[w.NL - 1], s, gx, gxb, st["g"], kvs[w.NL - 1])
+            last = self._gene_layer_last(w.gene_layers[w.NL - 1], s, gx, gxb, st["g"], kvs[w.NL - 1], maps)
             last, last_bf = ops.uncenter_rows(last, gpiv, idx=s["last_rows"], want_bf16=True)
             emb, emb_bf = last[:n_reg], last_bf[:n_reg]
         else:
@@ -602,10 +641,13 @@ class Engine:
             if s["cre_tok_rows"].numel():
                 t, _ = ops.gather_rows(cx, None, s["cre_tok_rows"])
                 out["cre_token_embedding"], _ = ops.uncenter_rows(t, cpiv, idx=s["cre_tok_rows"])
+        if attn is not None:
+            out["cre_attention"], out["cre_attention_off"] = attn[4], attn[3]
         return out
 
-    def _run_coarse(self, s, cre_pooled, gene_pooled):
-        """Stages 3-4 of a prepared slab through vf_seq2gene_forward (layer loop in the library)."""
+    def _run_coarse(self, s, cre_pooled, gene_pooled, attn=None):
+        """Stages 3-4 of a prepared slab through vf_seq2gene_forward (layer loop in the library); with attn (the tables
+        of _cre_attention) through vf_seq2gene_forward_attn."""
         import ctypes as C
         from . import _abi, _lib
         w = self.w
@@ -621,10 +663,17 @@ class Engine:
         slab = s["_abi_slab"]
         slab.single_stream = 0 if (CRE_STREAM and self.device.type == "cuda") else 1
         nbytes = int(_lib.lib().vf_seq2gene_workspace_bytes(C.addressof(w.abi()), C.addressof(slab)))
+        tab = None
+        if attn is not None:
+            gq, gk, off, _, maps = attn
+            tab = _abi.CreAttention(gq.shape[0], gq.data_ptr(), gk.data_ptr(), s["reg_idx"].data_ptr(), maps.data_ptr(),
+                                    off.data_ptr())
         pred, emb, gtok, ctok = ops.seq2gene_forward(w.abi(), slab, cre_pooled, gene_pooled,
                                                      self.ws.get("coarse_g", (nbytes,), torch.uint8), slab.n_reg,
-                                                     slab.n_need - slab.n_reg, w.D, "cre_pos_idx" in s)
+                                                     slab.n_need - slab.n_reg, w.D, "cre_pos_idx" in s, attn=tab)
         out = {"pred": pred, "emb": emb, "T": s["T"].tolist()}
+        if attn is not None:
+            out["cre_attention"], out["cre_attention_off"] = attn[4], attn[3]
         if "gene_pos_idx" in s:
             out["gene_token_embedding"] = gtok if gtok is not None else torch.empty((0, w.D), device=pred.device)
         if ctok is not None:
@@ -634,5 +683,7 @@ class Engine:
             out["cre_token_embedding"] = ops.seq2gene_cre_rows(w.abi(), slab, ws, s["cre_tok_rows"], w.D)
         return out
 
-    def forward_tokens(self, cre_tokens, cre_masks, gene_tokens, gene_masks, tissues, ref_labels, **kw):
-        return self.run(self.prepare(cre_tokens, cre_masks, gene_tokens, gene_masks, tissues, ref_labels, **kw))
+    def forward_tokens(self, cre_tokens, cre_masks, gene_tokens, gene_masks, tissues, ref_labels, cre_attention=False,
+                       **kw):
+        return self.run(self.prepare(cre_tokens, cre_masks, gene_tokens, gene_masks, tissues, ref_labels, **kw),
+                        cre_attention=cre_attention)

@@ -171,8 +171,9 @@ def seq2reg_forward(table, tokens_i32, pad_mask_u8, cu, n_tok, slots, workspace,
     return out
 
 
-def seq2gene_forward(table, slab, cre_pooled, gene_pooled, workspace, n_reg, n_tok_rows, D, want_cre_tok):
-    """Whole seq2gene forward of one slab in one call (vf_seq2gene_forward).
+def seq2gene_forward(table, slab, cre_pooled, gene_pooled, workspace, n_reg, n_tok_rows, D, want_cre_tok, attn=None):
+    """Whole seq2gene forward of one slab in one call (vf_seq2gene_forward; with attn, an _abi.CreAttention table,
+    vf_seq2gene_forward_attn, which also writes the gene -> CRE cross-attention maps).
     -> (pred fp32 [n_reg], emb fp32 [n_reg, D], gene token embeddings or None, CRE token embeddings or None)."""
     import ctypes as C
     dev = cre_pooled.device
@@ -180,10 +181,13 @@ def seq2gene_forward(table, slab, cre_pooled, gene_pooled, workspace, n_reg, n_t
     emb = torch.empty((n_reg, D), dtype=torch.float32, device=dev)
     gtok = torch.empty((n_tok_rows, D), dtype=torch.float32, device=dev) if n_tok_rows else None
     ctok = torch.empty((n_reg, D), dtype=torch.float32, device=dev) if want_cre_tok else None
+    args = (C.addressof(table), C.addressof(slab), ptr(cre_pooled), ptr(gene_pooled), ptr(workspace), workspace.numel(),
+            ptr(pred), ptr(emb), ptr(gtok), ptr(ctok))
     with _timed("seq2gene_forward"):
-        check(_lib.lib().vf_seq2gene_forward(C.addressof(table), C.addressof(slab), ptr(cre_pooled), ptr(gene_pooled),
-                                             ptr(workspace), workspace.numel(), ptr(pred), ptr(emb), ptr(gtok), ptr(ctok),
-                                             stream()))
+        if attn is None:
+            check(_lib.lib().vf_seq2gene_forward(*args, stream()))
+        else:
+            check(_lib.lib().vf_seq2gene_forward_attn(*args, C.addressof(attn), stream()))
     return pred, emb, gtok, ctok
 
 
@@ -296,6 +300,23 @@ def attention_mc(q, k, v, slots: SlotMap, heads, head_dim, slopes=None, out=None
         check(_lib.lib().vf_attention_mc_varlen(ptr(q), q.stride(0), ptr(k), k.stride(0), ptr(v), v.stride(0),
                                                 ptr(out), out.stride(0), q.shape[0], k.shape[0], ptr(slots.table),
                                                 slots.n_items, heads, head_dim, ptr(slopes), stream()))
+    return out
+
+
+def cross_attention_probs(q, k, q_rows, group_q, group_k, heads, head_dim, out, out_off, layer):
+    """Softmax probabilities of the cross-attention of selected query rows (vf_cross_attention_probs): q / k bf16 row
+    views (k = the K half of a packed KV buffer); q_rows int32 (None: query index = row); group_q / group_k int32
+    [n_groups, 2] = (first query index, count) / (first key row, count); out fp32 flat, out_off int64 [n_queries] = start
+    of each query's [n_layers, heads, keys] block; writes the block of `layer`."""
+    for t in (q, k):
+        assert t.is_cuda and t.dtype == torch.bfloat16 and t.stride(1) == 1
+    assert group_q.dtype == torch.int32 and group_k.dtype == torch.int32 and out_off.dtype == torch.int64
+    assert out.dtype == torch.float32 and (q_rows is None or q_rows.dtype == torch.int32)
+    n_groups = group_q.shape[0]
+    with _timed("attention_probs"):
+        check(_lib.lib().vf_cross_attention_probs(ptr(q), q.stride(0), ptr(q_rows), ptr(group_q), n_groups, ptr(k),
+                                                  k.stride(0), ptr(group_k), heads, head_dim, ptr(out), ptr(out_off),
+                                                  layer, stream()))
     return out
 
 

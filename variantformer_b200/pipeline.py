@@ -171,17 +171,22 @@ class HotPath:
         writer.flush()                                   # when this returns, every slab of the call is on disk
         return len(todo)
 
-    def predict(self, genes, variants: SampleVariants = None, to_host=True):
-        """-> (pred [sum T], emb [sum T, D]) as numpy (to_host) or device tensors."""
+    def predict(self, genes, variants: SampleVariants = None, to_host=True, cre_attention=False):
+        """-> (pred [sum T], emb [sum T, D]) as numpy (to_host) or device tensors (+ the stage-1 error flag).
+        cre_attention: one more element, (maps, offsets): the gene -> CRE cross-attention maps of every prediction
+        (Engine.run_pooled), CREs in batch order (sorted by start, reversed on the minus strand)."""
         t = self.tokenize(genes, variants)
         tissues = [torch.as_tensor(g.tissues, dtype=torch.long) for g in genes]
         slab = self.engine.prepare(t["cre_tok"], t["cre_msk"], t["gene_tok"], t["gene_msk"], tissues, t["labels"],
                                    lens=t["lens"])
-        out = self.engine.run(slab)
+        out = self.engine.run(slab, cre_attention=cre_attention)
+        maps = (out["cre_attention"], out["cre_attention_off"]) if cre_attention else None
         if not to_host:
-            return out["pred"], out["emb"], t["err"]
+            return (out["pred"], out["emb"], t["err"]) + ((maps,) if cre_attention else ())
         pred = out["pred"].cpu().numpy(); emb = out["emb"].cpu().numpy()
         self._raise_on_stage1_error(t["err"])
+        if cre_attention:
+            return pred, emb, (maps[0].cpu().numpy(), maps[1])
         return pred, emb
 
     @staticmethod

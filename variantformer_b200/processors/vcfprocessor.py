@@ -3,6 +3,7 @@
 import logging
 import os
 
+import numpy as np
 import pandas as pd
 import torch
 from torch.utils.data import DataLoader
@@ -85,6 +86,26 @@ class VCFProcessor:
         predictions = trainer.predict(model, dataloader, ckpt_path=checkpoint_path)
         return self.format_output(vcf_dataset.query_df, predictions)
 
+    def cre_attention(self, vcf_path: str, query_df: pd.DataFrame, **kwargs):
+        """Which CREs each prediction reads: the gene -> CRE cross-attention of the registry (tissue) token at every
+        gene layer (DESIGN.md section 13), for the query rows of create_data / predict.  Writes no file.
+        -> (df, maps): maps[(gene_id, tissue)] = fp32 [num_layers, num_heads, C] in manifest row order; df = one row per
+        (gene_id, tissue, layer, CRE) with the CRE's manifest columns, the head-mean `attention` and the prediction's
+        `predicted_expression`."""
+        dataset, dataloader = self.create_data(vcf_path, query_df, **kwargs)
+        model, _, trainer = self.load_model()
+        model.trainer = trainer
+        frames, maps, i = [], {}, 0
+        for batch in dataloader:
+            out = model.predict_cre_attention(batch)
+            for pred, a in zip(out["pred_gene_exp"], out["cre_attention"]):
+                row = dataset.query_df.iloc[i]
+                i += 1
+                manifest, order = dataset.cre_manifest(row["gene_id"])
+                df, m = cre_attention_frame(row["gene_id"], row["tissue_names"], manifest, order, a, pred)
+                frames.append(df); maps.update(m)
+        return pd.concat(frames, ignore_index=True), maps
+
     def format_output(self, df, predictions):
         pred_exp, embd = [], []
         for p in predictions:
@@ -93,3 +114,22 @@ class VCFProcessor:
         df["predicted_expression"] = pd.Series(pred_exp, index=df.index)
         df["embeddings"] = pd.Series(embd, index=df.index)
         return df
+
+
+def cre_attention_frame(gene_id, tissues, manifest, order, maps_batch, pred):
+    """One gene's maps in manifest order and long format.  manifest: DataFrame (chromosome, start_cre, end_cre,
+    cre_name); order: manifest row of every CRE in batch order; maps_batch: [T, layers, heads, C] in batch order; pred:
+    [T, 1].  -> (df, {(gene_id, tissue): [layers, heads, C]})."""
+    maps_batch = np.asarray(maps_batch)
+    T, L, H, C = maps_batch.shape
+    assert len(manifest) == C and len(order) == C and len(tissues) == T
+    m = np.empty_like(maps_batch)
+    m[..., np.asarray(order)] = maps_batch                   # batch position k holds manifest row order[k]
+    att = m.mean(axis=2)                                    # [T, L, C]
+    rep = lambda col: np.tile(manifest[col].to_numpy(), T * L)
+    df = pd.DataFrame({"gene_id": gene_id, "tissue": np.repeat(np.asarray(tissues, object), L * C),
+                       "layer": np.tile(np.repeat(np.arange(L), C), T), "chromosome": rep("chromosome"),
+                       "start_cre": rep("start_cre"), "end_cre": rep("end_cre"), "cre_name": rep("cre_name"),
+                       "attention": att.reshape(-1),
+                       "predicted_expression": np.repeat(np.asarray(pred, np.float32).reshape(T), L * C)})
+    return df, {(gene_id, t): m[k] for k, t in enumerate(tissues)}

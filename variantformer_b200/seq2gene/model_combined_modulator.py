@@ -5,6 +5,7 @@ reference's signatures (seq2gene/model_combined_modulator.py:411-435 ctor, :540-
 import logging
 from types import SimpleNamespace
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -271,6 +272,29 @@ class Seq2GenePredictorCombinedModulator(nn.Module):
             e = s + len(batch["tissue_context"][i])
             preds.append(pred[s:e]); embs.append(embd[s:e]); s = e
         return {"pred_gene_exp": preds, "embeddings": embs, "batch_idx": batch_idx, "dataloader_idx": dataloader_idx}
+
+    @torch.no_grad()
+    def predict_cre_attention(self, batch):
+        """predict_step with the gene -> CRE cross-attention maps of every prediction (Engine.run_pooled):
+        -> {"pred_gene_exp": [np (T_i, 1)], "cre_attention": [np fp32 (T_i, num_layers, num_heads, C_i)]}, CREs in
+        the batch order of the item.  Predictions are bit-identical to predict_step's."""
+        self._check_precision()
+        if not self._engine_variant():
+            raise NotImplementedError("cross-attention maps are implemented for the configs/vf_model.yaml architecture")
+        sq = lambda xs: [x[:, 0, :] if x.dim() == 3 else x for x in xs]
+        out = self.engine().forward_tokens(sq(batch["cre_sequences"]), sq(batch["cre_attention_masks"]),
+                                           sq(batch["gene_embeddings"]), sq(batch["gene_attention_masks"]),
+                                           list(batch["tissue_context"]), list(batch["ref_cre_labels"]),
+                                           cre_attention=True)
+        pred = out["pred"].cpu().numpy(); flat = out["cre_attention"].cpu().numpy(); off = out["cre_attention_off"]
+        L, H = self.combined_modulator.num_layers, self.combined_modulator.num_heads
+        preds, maps, r = [], [], 0
+        for g, tis in enumerate(batch["tissue_context"]):
+            T, C = len(tis), batch["cre_sequences"][g].shape[0]
+            preds.append(pred[r:r + T, None])
+            maps.append(np.stack([flat[off[r + t]:off[r + t] + L * H * C].reshape(L, H, C) for t in range(T)]))
+            r += T
+        return {"pred_gene_exp": preds, "cre_attention": maps}
 
     def variant_prediction(self, batch):
         """:909-1004 — (ref, het, hom) triplet; the three samples run as ONE batched pass instead of three
