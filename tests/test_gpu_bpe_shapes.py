@@ -5,8 +5,6 @@ clusters otherwise (vf_encode.cu: bpe_tokenize), so every slab of 5 or more gene
 CTA holds one segment of the window; merges, look-aheads and self-pair run scans cross segment boundaries through
 distributed shared memory.  Every comparison checks the tokens, out_count (the count before truncation), the token
 starts and the zero padding after the kept tokens, with no tolerance."""
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -25,14 +23,6 @@ DEV = "cuda"
 SMEM_SYMS = 8192              # longest window of the shared-memory kernel (kBpeSmemSyms)
 GENE_CAP = 200 * 200          # max_length * max_chunks: tokens kept per gene window
 SEP = b"N"
-
-
-@pytest.fixture(autouse=True)
-def _cluster_size_from_window_count():
-    # the kernel reads VF_BPE_CLUSTER once per process and it overrides the 8/16 choice: every case below would then
-    # run one instantiation while claiming to test the other
-    if os.environ.get("VF_BPE_CLUSTER"):
-        pytest.fail("VF_BPE_CLUSTER is set: it overrides the 8/16-CTA cluster choice these cases rely on; unset it")
 
 
 @pytest.fixture(scope="module")

@@ -1,8 +1,8 @@
 """vf_gemm_bf16 / vf_gemm_bf16_ln across the whole contract of include/vf_b200.h (GPU box): K tails (the partial last
 k-block and K < 64, TMA zero fill), N tails with the row statistics of partly empty tiles, ragged row counts on the
 single-CTA kernel and on CTA pairs whose peer CTA has 0, 1 or 127 live rows, strided operands and outputs, element
-offsets past 2^31, batch invariance of every epilogue form, bit-identical A/B switches (child processes: the library
-reads its VF_GEMM_* switches once per process), and contract violations that must return an error without a launch.
+offsets past 2^31, batch invariance of every epilogue form, the debug SIMT path against float64 (a child process: the
+library reads VF_GEMM_DEBUG_SIMT once per process), and contract violations that must return an error without a launch.
 
 The reference is float64 on the same bf16-rounded operands.  Per-element bound of an fp32 output:
     C_F32 * 2^-23 * (|A| @ |W|^T + |bias| + |resid|)
@@ -453,7 +453,7 @@ def test_rows_do_not_depend_on_how_many_rows_are_batched(K, N):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# g. A/B switches (read once per process: every run is a child process) compute the same bits as the default
+# g. The debug SIMT path (read once per process: it runs in a child process) agrees with float64
 def _ab_cases():
     """name -> (a, w, epi, bias, resid, ln, Run keywords): each form of (f), the out_proj and FFN2 residual forms at
     M >= 1024, a K-tail case and an N-tail case."""
@@ -470,8 +470,7 @@ def _ab_cases():
     cases["k tail"] = (a, w, EPI_BIAS_RESID_F32, bias, resid, None, dict(mirror=True, stats=True))
     a, w, bias, resid = _operands(1100, 328, 512, 7)
     cases["n tail"] = (a, w, EPI_BIAS_F32, bias, None, None, dict(mirror=True, stats=True))
-    # M >= 1024 with K < 512: the single-CTA kernel by default, CTA pairs under VF_GEMM_PAIR_MIN_K=0 (one to seven
-    # k-blocks, K < 64 included)
+    # M >= 1024 with K < 512 (one to seven k-blocks, K < 64 included)
     a, w, bias, resid = _operands(1100, 512, 200, 8)
     cases["k tail K=200"] = (a, w, EPI_BIAS_RESID_F32, bias, resid, None, dict(mirror=True, stats=True))
     a, w, bias, resid = _operands(1100, 512, 40, 9)
@@ -486,7 +485,7 @@ def _ab_cases():
 
 
 def _ab_child(out_path):
-    """Runs every _ab_cases() GEMM under this process's VF_GEMM_* switches and saves the outputs (CPU tensors)."""
+    """Runs every _ab_cases() GEMM under this process's VF_GEMM_DEBUG_SIMT setting and saves the outputs (CPU tensors)."""
     torch.cuda.set_device(0)
     res = {}
     for name, (a, w, epi, bias, resid, ln, kw) in _ab_cases().items():
@@ -505,23 +504,6 @@ def _child(tmp_path, tag, switch):
     p = subprocess.run([sys.executable, "-c", code, path], cwd=ROOT, env=env, timeout=600, capture_output=True, text=True)
     assert p.returncode == 0, f"{switch}: child failed ({p.returncode})\n{p.stdout[-2000:]}\n{p.stderr[-4000:]}"
     return torch.load(path)
-
-
-SWITCHES = [{"VF_GEMM_RT": "0"}, {"VF_GEMM_TMA_STORE": "0"}, {"VF_GEMM_TILE_ORDER": "strided"},
-            {"VF_GEMM_TILE_ORDER": "chunked"}, {"VF_GEMM_PAIR_MIN_ROWS": "0"}, {"VF_GEMM_PAIR_MIN_K": "0"},
-            {"VF_GEMM_RESID_PREFETCH": "1"}]
-
-
-def test_ab_switches_are_bit_identical(tmp_path):
-    base = _child(tmp_path, "base", {})
-    bad = []
-    for i, sw in enumerate(SWITCHES):
-        got = _child(tmp_path, f"v{i}", sw)
-        for name, outs in base.items():
-            for j, (b, v) in enumerate(zip(outs, got[name])):
-                if not torch.equal(b, v):
-                    bad.append(f"{sw} {name} output {j}: {int((b != v).sum())} elements differ")
-    assert not bad, "\n".join(bad)
 
 
 def test_debug_simt_path_agrees_with_float64(tmp_path):

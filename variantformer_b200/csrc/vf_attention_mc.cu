@@ -62,69 +62,13 @@ struct Params {
     float scale_log2;
 };
 
-// producer waits (a stage to be released): optionally polled with a short sleep, see vf_gemm.cu (measured: no gain)
-#ifndef VF_RELAXED_WAITS
-#define VF_RELAXED_WAITS 0
-#endif
-#if VF_RELAXED_WAITS
-#define VF_IDLE_WAIT mbar_wait_relaxed
-#else
-#define VF_IDLE_WAIT mbar_wait
-#endif
-// Which lane of a softmax warp arrives on the warp's behalf: `elect.sync` needs no register and no S2R (the compiler does
-// not keep `lane` alive across the tile loop at 104 registers: it re-read SR_TID at every arrive).
-#ifndef VF_ATTN_ELECT
-#define VF_ATTN_ELECT 1
-#endif
-#if VF_ATTN_ELECT
-#define VF_ATTN_LEADER elect_one()
-#else
-#define VF_ATTN_LEADER (lane == 0)
-#endif
-#ifndef VF_ATTN_OPAQUE_SADDR
-#define VF_ATTN_OPAQUE_SADDR 1
-#endif
-#ifndef VF_ATTN_REGS_LO
-#define VF_ATTN_REGS_LO 32        // producer / MMA issuer warpgroup; 128 * LO + 256 * HI <= 384 * 80
-#define VF_ATTN_REGS_HI 104       // softmax warpgroups
-#endif
-#ifndef VF_ATTN_NARROW
-#define VF_ATTN_NARROW 1          // tail block: softmax on whole 16-key groups up to the last key only (0: all 64 keys)
-#endif
-#ifndef VF_ATTN_ABLATE
-#define VF_ATTN_ABLATE 0          // timing experiments only (results are wrong): 1 no MUFU, 2 no P stores, 3 no TMEM loads
-#endif
-// 2^x for a PAIR of exponents (x <= ~0) on the FMA / ALU pipes instead of the MUFU: round(x) by the magic-number add,
-// 2^r on r = x - round(x) in [-0.5, 0.5] by a degree-3 minimax polynomial (7.5e-5 relative: 1/25 of the bf16 rounding P
-// gets right after), the integer part added into the exponent field.  10 instructions per pair (2 FMNMX clamps, 2 FADD2,
-// 4 FFMA2, 2 LEA) against 2 MUFU.EX2: used for every VF_ATTN_POLY_EVERY-th pair, because the softmax warps of an SM
-// sub-partition queue on the MUFU pipe (16 results/clk/SM) while their issue slots are half idle (ncu, DESIGN.md 5).
-#ifndef VF_ATTN_POLY_EVERY
-#define VF_ATTN_POLY_EVERY 0
-#endif
-__device__ __forceinline__ void ex2_poly_pair(float x0, float x1, float& p0, float& p1) {
-    const uint64_t x = f2_pack(fmaxf(x0, -126.f), fmaxf(x1, -126.f));
-    const uint64_t t = f2_add(x, f2_bcast(12582912.f));                      // 1.5 * 2^23 + round(x)
-    const uint64_t jf = f2_add(t, f2_bcast(-12582912.f));                    // round(x)
-    const uint64_t r = f2_fma(jf, f2_bcast(-1.f), x);
-    uint64_t q = f2_fma(f2_bcast(0.0551716685295105f), r, f2_bcast(0.2426111251115799f));
-    q = f2_fma(q, r, f2_bcast(0.6932609677314758f));
-    q = f2_fma(q, r, f2_bcast(0.9999280571937561f));
-    uint32_t t0, t1, q0, q1;
-    f2_unpack(t, t0, t1);
-    f2_unpack(q, q0, q1);
-    p0 = __uint_as_float(q0 + (t0 << 23));
-    p1 = __uint_as_float(q1 + (t1 << 23));
-}
+constexpr uint32_t kRegsLo = 32;    // producer / MMA issuer warpgroup; 128 * kRegsLo + 256 * kRegsHi <= 384 * 80
+constexpr uint32_t kRegsHi = 104;   // softmax warpgroups
 
 __device__ __forceinline__ float ex2_approx(float x) {
-#if VF_ATTN_ABLATE == 1
-    return x * 0.001f;
-#else
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
-#endif
 }
 
 // O_s row *= corr, in tensor memory, 8 columns at a time (few live registers: the caller holds a whole score row).
@@ -193,7 +137,7 @@ __device__ __forceinline__ float exponents(uint32_t (&r)[64], float scale, float
         }
 #pragma unroll
         for (int i = 0; i < 32; ++i) {
-            if (VF_ATTN_NARROW && MODE == 3 && (i & 7) == 0 && 2 * i >= nvalid) break;   // whole groups past the end
+            if (MODE == 3 && (i & 7) == 0 && 2 * i >= nvalid) break;   // whole groups past the end
             uint64_t bias2;
             if constexpr (MODE == 1) {
                 bias2 = f2_fma(kKeyPair[i], sl2, c2);
@@ -255,7 +199,7 @@ __device__ __forceinline__ void softmax_rest(uint32_t (&r)[64], float mx, float 
             const uint64_t nd2 = f2_pack(-delta, -delta);
 #pragma unroll
             for (int i = 0; i < 32; ++i) {
-                if (VF_ATTN_NARROW && KIND == 3 && (i & 7) == 0 && 2 * i >= nvalid) break;
+                if (KIND == 3 && (i & 7) == 0 && 2 * i >= nvalid) break;
                 f2_unpack(f2_add(f2_pack(r[2 * i], r[2 * i + 1]), nd2), r[2 * i], r[2 * i + 1]);
             }
         }
@@ -269,17 +213,11 @@ __device__ __forceinline__ void softmax_rest(uint32_t (&r)[64], float mx, float 
     int ndone = 32;
 #pragma unroll
     for (int i = 0; i < 32; ++i) {                            // r[i] <- bf16x2(p[2i], p[2i+1]); i <= 2i: in place
-        if (VF_ATTN_NARROW && KIND == 3 && (i & 7) == 0 && 2 * i >= nvalid) { ndone = i; break; }
+        if (KIND == 3 && (i & 7) == 0 && 2 * i >= nvalid) { ndone = i; break; }
         float x0, x1;
         if constexpr (KIND == 0) f2_unpack(f2_fma(f2_pack(r[2 * i], r[2 * i + 1]), scale2, c2), x0, x1);
         else { x0 = __uint_as_float(r[2 * i]); x1 = __uint_as_float(r[2 * i + 1]); }
-        float p0, p1;
-        if (VF_ATTN_POLY_EVERY > 0 && (i % (VF_ATTN_POLY_EVERY > 0 ? VF_ATTN_POLY_EVERY : 1)) == (VF_ATTN_POLY_EVERY - 1)) {
-            ex2_poly_pair(x0, x1, p0, p1);
-        } else {
-            p0 = ex2_approx(x0);
-            p1 = ex2_approx(x1);
-        }
+        const float p0 = ex2_approx(x0), p1 = ex2_approx(x1);
         if (i & 1) acc1 = f2_add(acc1, f2_pack(p0, p1));
         else acc0 = f2_add(acc0, f2_pack(p0, p1));
         r[i] = pack_bf16x2(p0, p1);
@@ -288,9 +226,6 @@ __device__ __forceinline__ void softmax_rest(uint32_t (&r)[64], float mx, float 
         mbar_wait(p_empty_bar, p_empty_parity);
         tc_fence_after();
     }
-#if VF_ATTN_ABLATE == 2
-    if (row == 1000)
-#endif
 #pragma unroll
     for (int q8 = 0; q8 < 8; ++q8) {                          // 8 probabilities -> one 16-byte chunk of the P row
         // PRESWZ: p_row already carries the row's swizzle term (see the caller)
@@ -412,7 +347,7 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
     const int4* recs = reinterpret_cast<const int4*>(p.slots);         // 4 int4 per item: {s0.lo, s0.hi, s1.lo, s1.hi}
 
     if (warp < kFirstSoftmaxWarp) {
-        reg_dealloc<VF_ATTN_REGS_LO>();
+        reg_dealloc<kRegsLo>();
         if (warp == 0 && elect_one()) {
             // ============================ TMA producer ============================
             uint32_t ring = 0;                               // K / V blocks loaded so far (same count for both rings)
@@ -428,7 +363,7 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
                 for (int s = 0; s < 2; ++s) {
                     if (nk[s] == 0) continue;
                     const uint32_t m = nq[s]++;
-                    VF_IDLE_WAIT(q_empty[s], (m & 1) ^ 1);
+                    mbar_wait(q_empty[s], (m & 1) ^ 1);
                     mbar_arrive_expect_tx(q_full[s], kQBytes);
                     tma_load_2d(sm_q + s * kQBytes, &tmQ, q_full[s], col, qrow[s]);
                 }
@@ -438,8 +373,8 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
                 auto load_k = [&](int j, int s) {
                     const uint32_t idx = base + ring_offset(j, s, same, nk[0], nk[1]);
                     const uint32_t st = idx % kKStages;
-                    VF_IDLE_WAIT(k_empty[2 * st], ((idx / kKStages) & 1) ^ 1);
-                    VF_IDLE_WAIT(k_empty[2 * st + 1], ((idx / kKStages) & 1) ^ 1);
+                    mbar_wait(k_empty[2 * st], ((idx / kKStages) & 1) ^ 1);
+                    mbar_wait(k_empty[2 * st + 1], ((idx / kKStages) & 1) ^ 1);
                     mbar_arrive_expect_tx(k_full[st], kKvBytes);
                     tma_load_2d(sm_k + st * kKvBytes, &tmK, k_full[st], col, krow[s] + j * kKB);
                     sts_release(k_issued, idx + 1);
@@ -447,8 +382,8 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
                 auto load_v = [&](int j, int s) {
                     const uint32_t idx = base + ring_offset(j, s, same, nk[0], nk[1]);
                     const uint32_t st = idx % kVStages;
-                    VF_IDLE_WAIT(v_empty[2 * st], ((idx / kVStages) & 1) ^ 1);
-                    VF_IDLE_WAIT(v_empty[2 * st + 1], ((idx / kVStages) & 1) ^ 1);
+                    mbar_wait(v_empty[2 * st], ((idx / kVStages) & 1) ^ 1);
+                    mbar_wait(v_empty[2 * st + 1], ((idx / kVStages) & 1) ^ 1);
                     mbar_arrive_expect_tx(v_full[st], kKvBytes);
                     tma_load_2d(sm_v + st * kKvBytes, &tmV, v_full[st], col, krow[s] + j * kKB);
                     sts_release(v_issued, idx + 1);
@@ -530,9 +465,6 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
             // Blocking mode: every lane polls for itself (each one's own later parity test is then sound); non-blocking
             // mode: one lane's answer for the warp, the lanes must agree on whether the early Q K^T went out.
             auto issued = [&](uint32_t ctr, uint32_t idx, uint32_t stages, bool blocking) -> bool {
-#ifdef VF_ATTN_NO_ISSUED_CHECK                                         // A/B timing only: NOT safe (see lds_acquire)
-                return true;
-#endif
                 if (idx >= run0 + stages) return true;
                 if (!blocking) return __shfl_sync(0xffffffffu, lds_acquire(ctr), 0) > idx;
                 uint32_t spins = 0;
@@ -584,7 +516,6 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
                     mbar_wait(v_full[st], (idx / kVStages) & 1);
                     const uint32_t vb = sm_v + st * kKvBytes;
                     int nkk = kKB / 16;                          // 16-key steps of this block's P V
-#ifndef VF_ATTN_NO_VTAIL                                               // A/B timing only
                     if (j + 1 == cur.my_nk() && cur.tail() < kKB) {
                         // The last block of a sequence over-fetches rows of whatever follows it in the K/V tensors.  Their
                         // probabilities are exactly 0, but 0 x NaN/Inf would still poison O.  Whole 16-key groups past the
@@ -595,13 +526,10 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
                         if (cur.tail() & 15) {
                             for (int r = cur.tail() + (lane >> 3); r < nkk * 16; r += 4)
                                 asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(vb + r * 128 + (lane & 7) * 16), "r"(0u) : "memory");
-#ifndef VF_ATTN_VTAIL_NOFENCE                                          // A/B timing only
                             fence_proxy_async_smem();
-#endif
                             __syncwarp();
                         }
                     }
-#endif
                     mbar_wait(p_full[s], (cur.tile0 + j) & 1);
                     tc_fence_after();
                     if (elect_one()) {
@@ -622,18 +550,16 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         }
     } else {
         // ============================ softmax warps (fully independent of each other) ============================
-        reg_alloc<VF_ATTN_REGS_HI>();
+        reg_alloc<kRegsHi>();
         const int s = (warp - kFirstSoftmaxWarp) >> 2;        // slot owned by this warpgroup
         const int quad = warp & 3;                            // TMEM lane quadrant of this warp
         const int row = quad * 32 + lane;                     // row inside the 128-row query tile
         const uint32_t t_lane = tmem_base + ((uint32_t)(quad * 32) << 16);
         uint32_t s_addr = t_lane + s * kKB;
         const uint32_t o_addr = t_lane + 128 + s * 64;
-#if VF_ATTN_OPAQUE_SADDR
         // opaque: otherwise the address is REBUILT from SR_TID and the (spilled) TMEM base at every tile — S2R + LDL + 8
         // integer instructions whose scoreboard waits were 6 % of the softmax warps' samples
         asm volatile("mov.b32 %0, %0;" : "+r"(s_addr));
-#endif
         // this row of the P tile (shared-space address, 128-byte aligned) with the row's SWIZZLE_128B term folded in:
         // chunk q8 of the row lives at my_p ^ (q8 * 16)
         // (not in the ALiBi kernels: measured 3 % slower there, 0.6 % faster without the bias)
@@ -662,23 +588,21 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
                 tc_fence_after();
                 // ---- scores of this row -> registers; then the score buffer is free for the next Q K^T ----
                 uint32_t r[64];
-#if VF_ATTN_ABLATE == 3
-#pragma unroll
-                for (int e = 0; e < 64; ++e) r[e] = __float_as_uint(0.01f * (float)(e + row + j));
-#else
                 tmem_ld_32x32(s_addr, *reinterpret_cast<uint32_t(*)[32]>(&r[0]));
-                if (!VF_ATTN_NARROW || me.w - j * kKB > 32) tmem_ld_32x32(s_addr + 32, *reinterpret_cast<uint32_t(*)[32]>(&r[32]));
+                if (me.w - j * kKB > 32)                      // (a tail block's softmax reads only its groups of keys)
+                    tmem_ld_32x32(s_addr + 32, *reinterpret_cast<uint32_t(*)[32]>(&r[32]));
                 tmem_ld_wait();
-#endif
                 tc_fence_before();
                 __syncwarp();
-                if (VF_ATTN_LEADER) mbar_arrive(my_s_empty);
+                // one lane arrives on the warp's behalf: `elect.sync` needs no register and no S2R (the compiler does not
+                // keep `lane` alive across the tile loop at 104 registers: it re-read SR_TID at every arrive)
+                if (elect_one()) mbar_arrive(my_s_empty);
                 softmax_tile<HD, ALIBI>(r, o_addr, j == 0, my_p_empty, (m & 1) ^ 1, p.scale_log2, slope, qpos, j * kKB,
                                         me.w, m_ref, l_run, my_p, row, lane, gate);
                 fence_proxy_async_smem();                     // generic-proxy P writes -> visible to the UMMA (async proxy)
                 tc_fence_before();                            // orders a possible tcgen05.st rescale before the PV
                 __syncwarp();
-                if (VF_ATTN_LEADER) mbar_arrive(my_p_full);
+                if (elect_one()) mbar_arrive(my_p_full);
             }
             // ---- epilogue: O_s / l -> bf16 -> global ----
             mbar_wait(my_o_full, n_mine & 1);
@@ -691,7 +615,7 @@ attention_mc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
             tmem_ld_wait();
             tc_fence_before();
             __syncwarp();
-            if (VF_ATTN_LEADER) mbar_arrive(my_o_empty);          // O_s may be overwritten by the next item's first P V
+            if (elect_one()) mbar_arrive(my_o_empty);          // O_s may be overwritten by the next item's first P V
             if (row < me.y) {
                 const float inv = 1.0f / l_run;
                 __nv_bfloat16* dst = p.o + (size_t)(me.x + row) * p.ldo + head * HD;

@@ -177,30 +177,6 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(SmemBar bar, uint32_t byte
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
     mbar_arrive_expect_tx(smem_bar(bar), bytes);
 }
-// Potentially blocking test (the hardware may suspend the thread for a short, implementation-defined time).  An
-// explicit long suspend-time hint was measured: it saves issue slots but wakes the waiter late (attention and the
-// K=512 GEMMs 5-15 % slower), so the default stays.
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-#ifdef VF_MBAR_HINT_NS
-    asm volatile(
-        "{\n\t.reg .pred P1;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2, %3;\n\t"
-        "selp.b32 %0, 1, 0, P1;\n\t}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)VF_MBAR_HINT_NS)
-        : "memory");
-#else
-    asm volatile(
-        "{\n\t.reg .pred P1;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, P1;\n\t}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-#endif
-    return ok != 0;
-}
 // Non-blocking test of a phase.
 __device__ __forceinline__ bool mbar_test_wait(SmemBar bar, uint32_t parity) {
     uint32_t ok;
@@ -226,13 +202,11 @@ __device__ __forceinline__ uint64_t global_timer_ns() {
 // pipeline bug cannot hang the GPU.  The loop must not contain a call: a printf here (even on the cold path) gives
 // every kernel that waits on a barrier an ABI stack frame and cost the attention kernels the whole 31 % again; build
 // with -DVF_WATCHDOG_VERBOSE to get the message (block, thread, barrier, parity) when chasing a deadlock.
-template <int SLEEP_NS>
-__device__ __forceinline__ void mbar_wait_impl(SmemBar bar, uint32_t parity) {
+__device__ __forceinline__ void mbar_wait(SmemBar bar, uint32_t parity) {
     uint32_t spins = 0;
     uint64_t t0 = 0;
     while (!mbar_test_wait(bar, parity)) {
-        if constexpr (SLEEP_NS > 0) __nanosleep(SLEEP_NS);
-        if ((++spins & (SLEEP_NS > 0 ? 0x3FFFu : 0xFFFFFu)) == 0) {
+        if ((++spins & 0xFFFFFu) == 0) {
             const uint64_t now = global_timer_ns();
             if (t0 == 0) t0 = now;
             if (now - t0 > VF_WATCHDOG_NS) {
@@ -249,14 +223,7 @@ __device__ __forceinline__ void mbar_wait_impl(SmemBar bar, uint32_t parity) {
         }
     }
 }
-__device__ __forceinline__ void mbar_wait(SmemBar bar, uint32_t parity) { mbar_wait_impl<0>(bar, parity); }
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) { mbar_wait_impl<0>(smem_bar(bar), parity); }
-// The same wait for warps that share a scheduler with working warps (TMA producers, MMA issuers): a tight spin loop
-// is always ready to issue and takes up to a third of the scheduler's issue slots from the warps doing arithmetic
-// (in-kernel clock stamps: the 64-key softmax tile of the attention kernel is issue bound).  Sleeping ~30 ns between
-// polls costs far less than the microsecond wake-up of mbarrier.try_wait.
-__device__ __forceinline__ void mbar_wait_relaxed(SmemBar bar, uint32_t parity) { mbar_wait_impl<32>(bar, parity); }
-__device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) { mbar_wait_impl<32>(smem_bar(bar), parity); }
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) { mbar_wait(smem_bar(bar), parity); }
 
 // ---- TMA (cp.async.bulk.tensor) -----------------------------------------------
 __device__ __forceinline__ void tma_prefetch_desc(const void* tmap) {
@@ -273,8 +240,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const void* tmap, ui
     tma_load_2d(smem_u32(smem_dst), tmap, smem_bar(bar), c0, c1);
 }
 
-// L2 prefetch of a 2-D tile (no shared-memory destination, no barrier): the tile is resident in L2 when ordinary
-// loads ask for it later.
 // TMA store of one box from shared memory (bulk async group): smem -> global, rows / columns past the tensor's extent
 // are clipped by the hardware.  The writer must make its generic-proxy shared-memory writes visible to the async proxy
 // first (fence_proxy_async_smem) and may overwrite the buffer only after tma_store_wait_read<N>().
@@ -285,12 +250,6 @@ __device__ __forceinline__ void tma_store_2d(const void* tmap, uint32_t smem_src
 __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-
-__device__ __forceinline__ void tma_prefetch_l2_2d(const void* tmap, int c0, int c1) {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
-                 ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1)
-                 : "memory");
-}
 
 // ---- warpgroup register reallocation (all 4 warps of a warpgroup must execute the same one) ----
 template <uint32_t R>

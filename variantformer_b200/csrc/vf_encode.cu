@@ -731,16 +731,11 @@ int bpe_tokenize(const uint8_t* seq, int64_t pitch, const int32_t* len, int n_wi
                 (int)(pitch < (int64_t)max_len ? pitch : (int64_t)max_len)};
     if (max_len > kBpeSmemSyms) {
         // cluster path: CL CTAs per window, segment of the symbol array per CTA in shared memory.  16-CTA clusters (non
-        // portable size, VF_BPE_CLUSTER=16) put a slab's 8 gene windows on 128 SMs instead of 64 but the cluster barrier
-        // grows faster than the sweep shrinks: 3.1 ms against 2.6-2.8 ms per slab with the portable size (the default).
-        // A call with few windows (single-gene latency) cannot fill the machine either way: there the larger cluster wins
-        // (one 301 k-symbol window: 1.1 ms against 1.8 ms).
-        static int cl_env = -1;
-        if (cl_env < 0) {
-            const char* e = getenv("VF_BPE_CLUSTER");
-            cl_env = e ? atoi(e) : 0;
-        }
-        const int cl = (cl_env == 8 || cl_env == 16) ? cl_env : (n_win <= 4 ? 16 : 8);
+        // portable size) put a slab's 8 gene windows on 128 SMs instead of 64 but the cluster barrier grows faster than
+        // the sweep shrinks: 3.1 ms against 2.6-2.8 ms per slab with the portable size of 8.  A call with few windows
+        // (single-gene latency) cannot fill the machine either way: there the larger cluster wins (one 301 k-symbol
+        // window: 1.1 ms against 1.8 ms).
+        const int cl = n_win <= 4 ? 16 : 8;
         auto launch = [&](auto kern, int CL) -> int {
             const int seg_cap = (max_len + CL - 1) / CL + 32;
             const size_t smem = (size_t)seg_cap * sizeof(uint16_t);

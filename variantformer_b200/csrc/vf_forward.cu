@@ -34,12 +34,6 @@ struct Carver {
     }
 };
 static inline int stats_parts(int n) { return 2 * ((n + 255) / 256); }
-// out_proj reads its residual from the bf16 mirror of the stream (see engine.py: OUT_PROJ_RESID16); env switch for A/B runs
-static bool resid16_outproj() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("VF_RESID16_OUTPROJ"); v = !(e && e[0] == '0'); }
-    return v != 0;
-}
 using bf16 = uint16_t;
 
 // ---- one LayerNorm-folded or plain linear ---------------------------------------------------------------------------
@@ -86,10 +80,10 @@ static int seq2reg_forward(const vf_seq2reg_weights_t& w, const int32_t* tokens,
                          l == 0 ? b.xs0 : b.xs, l == 0 ? 1 : P, w.ln_eps, nullptr, s))) return rc;
         if ((rc = attention_mc_varlen(b.qkv, 3 * d, b.qkv + d, 3 * d, b.qkv + 2 * d, 3 * d, b.a, d, n, n, slots, n_items, H, hd,
                                       w.slopes, s))) return rc;
-        // x1 = x + MHA(..): bf16 mirror + row statistics only (the layer's residual is its INPUT, modules.py:189)
-        const bool r16 = resid16_outproj();
-        if ((rc = linear(Lr.out, b.a, d, n, d, d, VF_EPI_BIAS_RESID_F32, r16 ? (const void*)b.xb : (const void*)b.x, r16, d,
-                         nullptr, 0, b.xb, d, nullptr, 0, 0.f, b.s1, s))) return rc;
+        // x1 = x + MHA(..): bf16 mirror + row statistics only (the layer's residual is its INPUT, modules.py:189); its
+        // residual is read from the bf16 mirror of x (see engine.py: Engine.seq2reg)
+        if ((rc = linear(Lr.out, b.a, d, n, d, d, VF_EPI_BIAS_RESID_F32, b.xb, 1, d, nullptr, 0, b.xb, d, nullptr, 0, 0.f, b.s1,
+                         s))) return rc;
         if ((rc = linear(Lr.g1, b.xb, d, n, F, d, VF_EPI_BIAS_GEGLU_BF16, nullptr, 0, 0, b.f, F / 2, nullptr, 0, b.s1, P,
                          w.ln_eps, nullptr, s))) return rc;
         if ((rc = linear(Lr.g2, b.f, F / 2, n, d, F / 2, VF_EPI_BIAS_RESID_F32, b.x, 0, d, b.x, d, b.xb, d, nullptr, 0, 0.f,
@@ -143,9 +137,8 @@ static int context_layer(const vf_context_layer_t& L, const vf_seq2gene_weights_
     if ((rc = linear(L.qkv, xb, D, M, 3 * D, D, VF_EPI_BIAS_BF16, nullptr, 0, 0, b.qkv, 3 * D, nullptr, 0, xs, xs_parts,
                      w.ln_eps, nullptr, s))) return rc;
     if ((rc = self_attn(b.qkv, b.a))) return rc;
-    const bool r16 = resid16_outproj();
-    if ((rc = linear(L.out, b.a, D, M, D, D, VF_EPI_BIAS_RESID_F32, r16 ? (const void*)xb : (const void*)x, r16, D, nullptr, 0,
-                     b.hb, D, nullptr, 0, 0.f, b.s1, s))) return rc;
+    if ((rc = linear(L.out, b.a, D, M, D, D, VF_EPI_BIAS_RESID_F32, xb, 1, D, nullptr, 0, b.hb, D, nullptr, 0, 0.f, b.s1, s)))
+        return rc;
     if ((rc = linear(L.q, b.hb, D, M, D, D, VF_EPI_BIAS_BF16, nullptr, 0, 0, b.qkv, 3 * D, nullptr, 0, b.s1, P, w.ln_eps,
                      nullptr, s))) return rc;
     if ((rc = cross_attn(b.qkv, b.a))) return rc;
@@ -277,9 +270,8 @@ static int seq2gene_forward(const vf_seq2gene_weights_t& w, const vf_seq2gene_sl
                             qw.cs, D, w.ln_eps, nullptr, main))) return rc;
         if ((rc = attention_mc_varlen(b.qR, D, kvs, 3 * D, kvs + D, 3 * D, b.aR, D, R, Mg, t.slots_last_self, t.n_last_self, H, hd,
                                       w.slopes, main))) return rc;
-        const bool r16 = resid16_outproj();
-        if ((rc = linear(L.out, b.aR, D, R, D, D, VF_EPI_BIAS_RESID_F32, r16 ? (const void*)b.xbR : (const void*)b.xR, r16, D,
-                         nullptr, 0, b.hbR, D, nullptr, 0, 0.f, b.s1R, main))) return rc;
+        if ((rc = linear(L.out, b.aR, D, R, D, D, VF_EPI_BIAS_RESID_F32, b.xbR, 1, D, nullptr, 0, b.hbR, D, nullptr, 0, 0.f, b.s1R,
+                         main))) return rc;
         if ((rc = linear(L.q, b.hbR, D, R, D, D, VF_EPI_BIAS_BF16, nullptr, 0, 0, b.qR, D, nullptr, 0, b.s1R, P, w.ln_eps, nullptr,
                          main))) return rc;
         bf16* kv = kv_of(NL - 1);

@@ -30,23 +30,6 @@
 #include "vf_common.cuh"
 #include "vf_internal.h"
 
-// Waits of warps that are idle most of the time (producer, MMA issuer, epilogue warps waiting for a whole mainloop) can
-// poll with a ~30 ns sleep instead of a tight spin (-DVF_RELAXED_WAITS=1).  The step runs power capped, so the idea was
-// to leave issue slots and power to the working warps; measured on the whole step (same box, alternating): 218.2 ms
-// relaxed vs 216.2 ms tight, clocks unchanged — the late wake-ups cost more than the spinning.  Default: tight.
-#ifndef VF_RELAXED_WAITS
-#define VF_RELAXED_WAITS 0
-#endif
-#if VF_RELAXED_WAITS
-#define VF_IDLE_WAIT mbar_wait_relaxed
-#else
-#define VF_IDLE_WAIT mbar_wait
-#endif
-
-#ifndef VF_GEMM_INTERIOR_FAST
-#define VF_GEMM_INTERIOR_FAST 1
-#endif
-
 namespace vf {
 
 constexpr int BM = 128, BN = 256, BK = 64, kStages = 4;
@@ -86,9 +69,6 @@ struct GemmParams {
     float ln_inv_d, ln_eps;  //                 1 / normalised width, eps
     float* stats_out;        // fp32 outputs: partial (sum, sum of squares) of every output row -> [M, 2*n_tiles, 2], or nullptr
     int tile_chunked;        // tile schedule: 1 = each unit walks a contiguous run of tiles (n fastest), 0 = round-robin
-    int tma_store;           // bf16 epilogues: slabs leave through cp.async.bulk.tensor stores (tmO) instead of per-lane stores
-    int prefetch_resid;      // producer warp bulk-prefetches the residual tile into L2 (VF_GEMM_RESID_PREFETCH=1; off by
-                             // default: measured 5-10 % slower than the epilogue's own one-slab-ahead register prefetch)
 };
 
 template <int EPI>
@@ -103,10 +83,9 @@ constexpr bool epi_is_bf16() {
 // 16-byte chunks are XOR-swizzled inside the tile so both the row-wise writes and the column-wise reads are
 // bank-conflict free.
 // Residual slab prefetch: the 8 float4 this lane will add in the coalesced phase (4 rows x 128 B per warp request).
-// Issued as one batch well before they are needed so the (L2, see the producer's bulk prefetch) latency overlaps the
-// TMEM load and the staging writes (loads cannot be hoisted by the compiler itself: `out` may alias `resid`).
+// Issued as one batch well before they are needed so the memory latency overlaps the TMEM load and the staging writes
+// (loads cannot be hoisted by the compiler itself: `out` may alias `resid`).
 __device__ __forceinline__ void load_resid_slab(const GemmParams& p, int row0, int col0, int lane, float4 (&rr4)[8]) {
-#if VF_GEMM_INTERIOR_FAST
     // interior slab (warp-uniform test): one base pointer, constant row stride, no per-row predicates — the bounds
     // checks, 64-bit address products and the branches around them were ~45 % of the residual epilogue's instructions
     if (row0 + 32 <= p.M && col0 + 32 <= p.N) {
@@ -129,7 +108,6 @@ __device__ __forceinline__ void load_resid_slab(const GemmParams& p, int row0, i
             return;
         }
     }
-#endif
 #pragma unroll
     for (int it = 0; it < 8; ++it) {
         const int grow = row0 + it * 4 + (lane >> 3), gcol = col0 + (lane & 7) * 4;
@@ -183,50 +161,25 @@ template <int EPI>
 __device__ __forceinline__ void epilogue_store_slab(const GemmParams& p, uint32_t stage, int row0, int col0, int n_out,
                                                     const float (&v)[32], int lane, const float4 (&rr4)[8],
                                                     RowStats& rs, const CUtensorMap* tmO = nullptr, int half_buf = 0) {
-    // `stage` = shared-space address of the warp's 4 KB tile.  All reads of the transposed tile are issued as one batch
-    // (no branch in between), then the global stores follow.
+    // `stage` = shared-space address of the warp's 4 KB tile.
     if constexpr (epi_is_bf16<EPI>()) {
-        if (p.tma_store) {
-            // The slab leaves through ONE bulk tensor store: the staging layout ([32 rows][4 chunks of 16 B], chunk index
-            // XOR (row >> 1) & 3) is exactly SWIZZLE_64B, so the TMA unit reads it as it lies; rows / columns past M / N
-            // are clipped by the hardware.  The warp's 4 KB tile holds two bf16 slabs: while one is being read out by the
-            // TMA unit the next is written (at most one store group outstanding when a half is rewritten).
-            stage += half_buf * 2048;
-            if (lane == 0) tma_store_wait_read<1>();
-            __syncwarp();
+        // The slab leaves through ONE bulk tensor store: the staging layout ([32 rows][4 chunks of 16 B], chunk index
+        // XOR (row >> 1) & 3) is exactly SWIZZLE_64B, so the TMA unit reads it as it lies; rows / columns past M / N
+        // are clipped by the hardware.  The warp's 4 KB tile holds two bf16 slabs: while one is being read out by the
+        // TMA unit the next is written (at most one store group outstanding when a half is rewritten).
+        stage += half_buf * 2048;
+        if (lane == 0) tma_store_wait_read<1>();
+        __syncwarp();
 #pragma unroll
-            for (int j = 0; j < 4; ++j)
-                sts128(stage + (lane * 4 + (j ^ ((lane >> 1) & 3))) * 16, pack_bf16x2(v[j * 8 + 0], v[j * 8 + 1]),
-                       pack_bf16x2(v[j * 8 + 2], v[j * 8 + 3]), pack_bf16x2(v[j * 8 + 4], v[j * 8 + 5]),
-                       pack_bf16x2(v[j * 8 + 6], v[j * 8 + 7]));
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) { tma_store_2d(tmO, stage, col0, row0); tma_store_commit(); }
-            return;
-        }
-#pragma unroll
-        for (int j = 0; j < 4; ++j)                                     // [32 rows][4 chunks of 16 B]
+        for (int j = 0; j < 4; ++j)
             sts128(stage + (lane * 4 + (j ^ ((lane >> 1) & 3))) * 16, pack_bf16x2(v[j * 8 + 0], v[j * 8 + 1]),
                    pack_bf16x2(v[j * 8 + 2], v[j * 8 + 3]), pack_bf16x2(v[j * 8 + 4], v[j * 8 + 5]),
                    pack_bf16x2(v[j * 8 + 6], v[j * 8 + 7]));
+        fence_proxy_async_smem();
         __syncwarp();
-        uint4 q[4];
-#pragma unroll
-        for (int it = 0; it < 4; ++it) {
-            const int rr = it * 8 + (lane >> 2), jj = lane & 3;
-            q[it] = lds128(stage + (rr * 4 + (jj ^ ((rr >> 1) & 3))) * 16);
-        }
-        __syncwarp();
-        __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(p.out);
-        const int gcol = col0 + (lane & 3) * 8;
-        if (gcol + 8 <= n_out) {
-#pragma unroll
-            for (int it = 0; it < 4; ++it) {
-                const int grow = row0 + it * 8 + (lane >> 2);
-                if (grow < p.M) *reinterpret_cast<uint4*>(o + (size_t)grow * p.ldo + gcol) = q[it];
-            }
-        }
+        if (lane == 0) { tma_store_2d(tmO, stage, col0, row0); tma_store_commit(); }
     } else {
+        // All reads of the transposed tile are issued as one batch (no branch in between), then the global stores follow.
 #pragma unroll
         for (int j = 0; j < 8; ++j)                                     // [32 rows][8 chunks of 16 B]
             sts128(stage + (lane * 8 + (j ^ (lane & 7))) * 16, __float_as_uint(v[j * 4]), __float_as_uint(v[j * 4 + 1]),
@@ -241,7 +194,6 @@ __device__ __forceinline__ void epilogue_store_slab(const GemmParams& p, uint32_
         __syncwarp();
         float* o = reinterpret_cast<float*>(p.out);
         const int gcol = col0 + (lane & 7) * 4;
-#if VF_GEMM_INTERIOR_FAST
         if (row0 + 32 <= p.M && col0 + 32 <= n_out) {                   // interior slab (warp-uniform): see load_resid_slab
             const int r = row0 + (lane >> 3);
             float* op = o ? o + (size_t)r * p.ldo + gcol : nullptr;
@@ -270,7 +222,6 @@ __device__ __forceinline__ void epilogue_store_slab(const GemmParams& p, uint32_
             }
             return;
         }
-#endif
         if (gcol + 4 <= n_out) {
 #pragma unroll
             for (int it = 0; it < 8; ++it) {
@@ -312,11 +263,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     // Local copy: the fields live in registers.  Read through the parameter itself they are re-fetched from the
     // constant bank (LDCU, a scoreboard wait each) after every asm statement with a memory clobber — in the epilogue
     // that is several times per slab.
-#ifndef VF_GEMM_NO_PARAM_COPY
     const GemmParams p = p_in;
-#else
-    const GemmParams& p = p_in;
-#endif
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw;
     if (smem_u32(smem_raw) & 1023u) __trap();                // SWIZZLE_128B tiles need 1 KB alignment
@@ -359,8 +306,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     if (warp == 0 && elect_one()) {
         tma_prefetch_desc(&tmA);
         tma_prefetch_desc(&tmB);
-        if constexpr (EPI == VF_EPI_BIAS_RESID_F32) tma_prefetch_desc(&tmR);
-        if constexpr (RT != 0) tma_prefetch_desc(&tmO);
+        if constexpr (RT != 0) { tma_prefetch_desc(&tmR); tma_prefetch_desc(&tmO); }
         if constexpr (epi_is_bf16<EPI>()) tma_prefetch_desc(&tmO);
         for (int s = 0; s < kStg; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
         // the leader's tmem_empty collects the epilogue warps of BOTH CTAs of a pair
@@ -387,16 +333,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 for (int ti = 0; ti < t_count; ++ti) {
                     const int t = t_first + ti * t_step;
                     const int m0 = (t / n_tiles) * BM * CTAS + rank * BM, n0 = (t % n_tiles) * BN;
-                    if constexpr (EPI == VF_EPI_BIAS_RESID_F32) {
-                        // the epilogue of this tile runs one mainloop from now: pull its residual into L2 meanwhile
-                        if (p.resid && p.prefetch_resid) {   // (fp32 residual only)
-#pragma unroll
-                            for (int c = 0; c < BN; c += 64)
-                                if (n0 + c < p.N) tma_prefetch_l2_2d(&tmR, n0 + c, m0);
-                        }
-                    }
                     for (int kb = 0; kb < k_blocks; ++kb) {
-                        VF_IDLE_WAIT(&empty[stage], phase ^ 1);
+                        mbar_wait(&empty[stage], phase ^ 1);
                         if constexpr (CTAS == 2) {
                             // all four loads of the pair complete on the LEADER's barrier, which expects their total
                             if (rank == 0) mbar_arrive_expect_tx(&full[stage], 2 * kStageBytesC);
@@ -419,11 +357,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 int stage = 0; uint32_t phase = 0; int it = 0;
                 for (; it < t_count; ++it) {
                     const int acc = it & 1; const uint32_t acc_phase = (it >> 1) & 1;
-                    VF_IDLE_WAIT(&tmem_empty[acc], acc_phase ^ 1);
+                    mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
                     tc_fence_after();
                     const uint32_t d_tmem = tmem_base + acc * BN;
                     for (int kb = 0; kb < k_blocks; ++kb) {
-                        VF_IDLE_WAIT(&full[stage], phase);
+                        mbar_wait(&full[stage], phase);
                         tc_fence_after();
                         const uint64_t da = umma_desc_kmajor_sw128(smem_u32(smem_a + stage * kABytes));
                         const uint64_t db = umma_desc_kmajor_sw128(smem_u32(smem_b + stage * kBBytesC));
@@ -546,7 +484,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             }
             last_m0 = m0;
             rs.clear();
-            VF_IDLE_WAIT(&tmem_full[acc], acc_phase);
+            mbar_wait(&tmem_full[acc], acc_phase);
             tc_fence_after();
             const uint32_t t_row = tmem_base + ((uint32_t)(quad * 32) << 16) + acc * BN;
             if constexpr (EPI == VF_EPI_BIAS_GEGLU_BF16) {
@@ -958,40 +896,15 @@ static int make_tmap_out_bf16(CUtensorMap* tm, void* base, int rows, int cols, i
     return 0;
 }
 
-// fp32 residual [rows, cols] -> plain (unswizzled) map with box {64, 128}, used for L2 prefetch only.
-static int make_tmap_resid(CUtensorMap* tm, const float* base, int rows, int cols, int ld) {
-    PFN_encodeTiled enc = get_encode_fn();
-    VF_REQUIRE(enc, "cuTensorMapEncodeTiled entry point not available (driver too old?)");
-    VF_REQUIRE((reinterpret_cast<uintptr_t>(base) & 15) == 0 && (ld % 4) == 0,
-               "GEMM residual must be 16-byte aligned with a row stride that is a multiple of 4 elements");
-    cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)ld * 4};
-    cuuint32_t box[2] = {(cuuint32_t)(cols < 64 ? cols : 64), (cuuint32_t)BM};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    VF_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (residual) failed with CUresult %d (rows=%d cols=%d ld=%d)",
-               (int)r, rows, cols, ld);
-    return 0;
-}
-
 static int g_num_sms = 0;
 static bool g_debug_simt = false;
-static int g_resid_prefetch = 0;
-// Tile schedule: -1 = by shape (chunked for LayerNorm-folded epilogues with K <= 512, whose epilogue is the critical
-// path: +5-10 % there; round-robin otherwise: concurrently running CTAs then share A tiles in L2, worth 15 % at
-// K = 1536).  VF_GEMM_TILE_ORDER=strided|chunked forces one (A/B timing).
-static int g_tile_chunked = -1;
-// CTA-pair kernel for M >= g_pair_min_rows (VF_GEMM_PAIR_MIN_ROWS; 0 = never) and K >= g_pair_min_k: measured 6-12 %
-// faster than the single-CTA kernel at K = 1024 / 1536 (Wqkv 101k x 4608 x 1536: 1.03 -> 0.90 ms = 1590 TFLOP/s, cuBLAS
-// 0.91).  Round 1 kept K = 512 on the single-CTA kernel (its epilogue was the limit then); with the leaner epilogues of
-// round 2 (shared-memory column vectors, packed GeGLU, TMA stores) the operand traffic is the limit there too: 48 KB of
-// operands per 512-cycle k-step and SM against 32 KB for a pair — LN-folded Wqkv 1.11 M x 1536 x 512 1.61 -> 1.49 ms,
-// GeGLU1 x 2048 2.11-2.24 -> 1.95 ms (cuBLAS 1.44-1.64 / 2.02-2.31).
-static int g_pair_min_rows = 1024, g_pair_min_k = 512;
-static int g_tma_store = 1;
-static int g_rt = 3;                                    // TMA-staged residual epilogues: bit 0 out_proj form, bit 1 in-place FFN2 form (VF_GEMM_RT)
+// CTA-pair kernel for M >= kPairMinRows and K >= kPairMinK: measured 6-12 % faster than the single-CTA kernel at
+// K = 1024 / 1536 (Wqkv 101k x 4608 x 1536: 1.03 -> 0.90 ms = 1590 TFLOP/s, cuBLAS 0.91).  Round 1 kept K = 512 on the
+// single-CTA kernel (its epilogue was the limit then); with the leaner epilogues of round 2 (shared-memory column
+// vectors, packed GeGLU, TMA stores) the operand traffic is the limit there too: 48 KB of operands per 512-cycle k-step
+// and SM against 32 KB for a pair — LN-folded Wqkv 1.11 M x 1536 x 512 1.61 -> 1.49 ms, GeGLU1 x 2048 2.11-2.24 ->
+// 1.95 ms (cuBLAS 1.44-1.64 / 2.02-2.31).
+constexpr int kPairMinRows = 1024, kPairMinK = 512;
 static bool g_inited = false;
 
 template <int EPI>
@@ -1064,18 +977,6 @@ int gemm_bf16(const void* A, int lda, const void* W, int ldw, int M, int N, int 
         VF_CUDA_OK(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
         const char* e = getenv("VF_GEMM_DEBUG_SIMT");
         g_debug_simt = e && e[0] == '1';
-        const char* e2 = getenv("VF_GEMM_RESID_PREFETCH");
-        g_resid_prefetch = e2 && e2[0] == '1';
-        const char* e5 = getenv("VF_GEMM_TILE_ORDER");
-        if (e5) g_tile_chunked = e5[0] == 'c' ? 1 : e5[0] == 's' ? 0 : -1;
-        const char* e7 = getenv("VF_GEMM_TMA_STORE");
-        if (e7) g_tma_store = atoi(e7);
-        const char* e8 = getenv("VF_GEMM_RT");
-        if (e8) g_rt = atoi(e8);
-        const char* e3 = getenv("VF_GEMM_PAIR_MIN_ROWS");
-        if (e3) g_pair_min_rows = atoi(e3);
-        const char* e4 = getenv("VF_GEMM_PAIR_MIN_K");
-        if (e4) g_pair_min_k = atoi(e4);
         g_inited = true;
     }
     VF_REQUIRE(M >= 0 && N > 0 && K > 0, "gemm: bad shape M=%d N=%d K=%d", M, N, K);
@@ -1114,8 +1015,9 @@ int gemm_bf16(const void* A, int lda, const void* W, int ldw, int M, int N, int 
     VF_REQUIRE(!stats_out || !out_bf16, "gemm: row statistics are produced by the fp32 epilogues only");
     p.ln_stats = ln_stats; p.ln_parts = ln_parts; p.ln_colsum = ln_colsum;
     p.ln_inv_d = ln_dim > 0 ? 1.0f / (float)ln_dim : 0.f; p.ln_eps = ln_eps; p.stats_out = stats_out;
-    p.tile_chunked = g_tile_chunked >= 0 ? g_tile_chunked : (ln_stats != nullptr && K <= 512);
-    p.prefetch_resid = g_resid_prefetch && epi == VF_EPI_BIAS_RESID_F32 && resid && !resid_bf16;
+    // Tile schedule: chunked for LayerNorm-folded epilogues with K <= 512, whose epilogue is the critical path (+5-10 %
+    // there); round-robin otherwise: concurrently running CTAs then share A tiles in L2, worth 15 % at K = 1536.
+    p.tile_chunked = ln_stats != nullptr && K <= 512;
     if (g_debug_simt) {
         if (stats_out)
             VF_CUDA_OK(cudaMemsetAsync(stats_out, 0, (size_t)M * 2 * ((N + BN - 1) / BN) * 2 * sizeof(float), stream));
@@ -1129,30 +1031,21 @@ int gemm_bf16(const void* A, int lda, const void* W, int ldw, int M, int N, int 
             default: return launch_simt<VF_EPI_BIAS_F32>(a, lda, w, ldw, p, stream);
         }
     }
-    const bool pair = g_pair_min_rows > 0 && M >= g_pair_min_rows && K >= g_pair_min_k;
-    CUtensorMap ta, tb, tr;
+    const bool pair = M >= kPairMinRows && K >= kPairMinK;
+    CUtensorMap ta, tb;
     if (make_tmap_kmajor(&ta, A, M, K, lda, BM)) return -1;
     if (make_tmap_kmajor(&tb, W, N, K, ldw, pair ? BN / 2 : BN)) return -1;
-    if (epi == VF_EPI_BIAS_RESID_F32 && resid && !resid_bf16 && g_resid_prefetch) {
-        if (make_tmap_resid(&tr, reinterpret_cast<const float*>(resid), M, N, ldr)) return -1;
-    } else {
-        tr = ta;                                                       // never dereferenced
-    }
-    // bf16 epilogues store through TMA (VF_GEMM_TMA_STORE=0: per-lane stores, for A/B runs); out and ldo were checked
-    // above for the 16-byte alignment both paths need
-    CUtensorMap to = ta;
-    p.tma_store = 0;
-    if (out_bf16 && g_tma_store) {
-        if (make_tmap_out_bf16(&to, out, M, n_out, ldo)) return -1;
-        p.tma_store = 1;
-    }
-    if (pair && (g_rt & 1) && epi == VF_EPI_BIAS_RESID_F32 && resid_bf16 && !out && out2 && N % BN == 0) {
+    CUtensorMap tr = ta, to = ta;                                      // (placeholders where a kernel reads neither)
+    // bf16 epilogues store through TMA: out (always given for them) and ldo were checked above for the alignment the
+    // tensor map needs
+    if (out_bf16 && make_tmap_out_bf16(&to, out, M, n_out, ldo)) return -1;
+    if (pair && epi == VF_EPI_BIAS_RESID_F32 && resid_bf16 && !out && out2 && N % BN == 0) {
         // out_proj shape: bf16 residual in, bf16 mirror + row statistics out -> TMA-staged epilogue (see kGemmSmemRT)
         if (make_tmap_out_bf16(&tr, const_cast<void*>(resid), M, N, ldr)) return -1;
         if (make_tmap_out_bf16(&to, out2, M, N, ldo2)) return -1;
         return launch_tc_pair<VF_EPI_BIAS_RESID_F32, 1>(ta, tb, tr, to, p, stream);
     }
-    if (pair && (g_rt & 2) && epi == VF_EPI_BIAS_RESID_F32 && resid && !resid_bf16 && out == resid && ldo == ldr && N % BN == 0) {
+    if (pair && epi == VF_EPI_BIAS_RESID_F32 && resid && !resid_bf16 && out == resid && ldo == ldr && N % BN == 0) {
         // FFN2 form, in place on the fp32 stream (+ mirror, statistics)
         if (make_tmap_slab_f32(&tr, out, M, N, ldo)) return -1;
         if (out2 && make_tmap_out_bf16(&to, out2, M, N, ldo2)) return -1;

@@ -23,7 +23,6 @@ Schedule differences from the reference (results identical, oracle/model_fp32.py
 Numerics: bf16 GEMM/attention operands, fp32 accumulation, fp32 residual stream and LayerNorm statistics.
 """
 import math
-import os
 
 import numpy as np
 import torch
@@ -33,17 +32,12 @@ from ._lib import EPI_BIAS_BF16, EPI_BIAS_F32, EPI_BIAS_GEGLU_BF16, EPI_BIAS_GEL
 from .utils.alibi import alibi_slopes
 
 NUM_REF_CRES = 9
-# "coarse" (default): the forward of a slab is three calls into the library (vf_seq2reg_forward x2, vf_seq2gene_forward)
-# with the layer loop in C++; "fine": one Python call per kernel — the same kernels in the same order, bit-identical
-# results; used when a launch profiler is attached (bench.py's per-kernel pass) and for A/B runs (VF_ENGINE=fine).
-COARSE = os.environ.get("VF_ENGINE", "coarse") != "fine"
-# x1 = x + MHA(..) exists only as a bf16 mirror (its consumers are a LayerNorm-folded GEMM and the next residual add), so
-# the out_proj epilogue may read its residual from the bf16 mirror of x instead of the fp32 stream: half the residual
-# bytes of the most HBM-bound GEMMs of the layer.  The fp32 stream itself is untouched (the layer's own residual add reads
-# it in full precision).  VF_RESID16_OUTPROJ=0: fp32 residual there too (A/B).
-OUT_PROJ_RESID16 = os.environ.get("VF_RESID16_OUTPROJ", "1") != "0"
-# run the CRE stack on its own CUDA stream, concurrently with the gene stack ("0": one stream, for A/B and debugging)
-CRE_STREAM = os.environ.get("VF_CRE_STREAM", "1") != "0"
+# True: the forward of a slab is three calls into the library (vf_seq2reg_forward x2, vf_seq2gene_forward) with the layer
+# loop in C++; False: one Python call per kernel — the same kernels in the same order, bit-identical results; used when a
+# launch profiler is attached (bench.py's per-kernel pass).
+COARSE = True
+# run the CRE stack on its own CUDA stream, concurrently with the gene stack (False: one stream)
+CRE_STREAM = True
 
 
 class AttnPlan:
@@ -298,8 +292,10 @@ class Engine:
                      ln=L["qkv"].ln(xs0 if li == 0 else xs))                                           # Wqkv(norm1(x))
             plan.run(qkv[:, :d], qkv[:, d:2 * d], qkv[:, 2 * d:], H, hd, W.slopes, a)
             # x1 = x + MHA(..) is consumed only through norm2 -> linear_geglu_1 (the layer's residual is its INPUT,
-            # modules.py:189): it exists as a bf16 mirror + row statistics only
-            ops.gemm(a, L["out"].w, EPI_BIAS_RESID_F32, bias=L["out"].b, resid=xb if OUT_PROJ_RESID16 else x, out2=xb,
+            # modules.py:189): it exists as a bf16 mirror + row statistics only.  So out_proj reads its residual from the
+            # bf16 mirror of x too: half the residual bytes of the most HBM-bound GEMMs of the layer (the fp32 stream
+            # itself is untouched: the layer's own residual add reads it in full precision)
+            ops.gemm(a, L["out"].w, EPI_BIAS_RESID_F32, bias=L["out"].b, resid=xb, out2=xb,
                      stats_out=s1, mirror_only=True)
             ops.gemm(xb, L["g1"].w, EPI_BIAS_GEGLU_BF16, bias=L["g1"].b, out=f, ln=L["g1"].ln(s1))      # GeGLU(norm2(x1))
             ops.gemm(f, L["g2"].w, EPI_BIAS_RESID_F32, bias=L["g2"].b, resid=x, out=x, out2=xb, stats_out=xs)  # + layer input
@@ -319,8 +315,9 @@ class Engine:
         ops.gemm(xb, L["qkv"].w, EPI_BIAS_BF16, bias=L["qkv"].b, out=qkv, ln=L["qkv"].ln(xs))          # Wqkv(norm1(x))
         self_attn(qkv, a)
         # x1 = x + selfMHA(..) and x1' = x1 + crossMHA(..) are consumed only through norm2 / norm3 -> bf16 GEMM and as
-        # each other's residual (the layer's own residual is its INPUT, layers.py:163): bf16 mirror + statistics only
-        ops.gemm(a, L["out"].w, EPI_BIAS_RESID_F32, bias=L["out"].b, resid=xb if OUT_PROJ_RESID16 else x, out2=hb,
+        # each other's residual (the layer's own residual is its INPUT, layers.py:163): bf16 mirror + statistics only;
+        # out_proj reads the bf16 mirror of x as its residual (see seq2reg)
+        ops.gemm(a, L["out"].w, EPI_BIAS_RESID_F32, bias=L["out"].b, resid=xb, out2=hb,
                  stats_out=s1, mirror_only=True)
         q = qkv[:, :D]                                                  # reuse the qkv buffer for the cross query
         ops.gemm(hb, L["q"].w, EPI_BIAS_BF16, bias=L["q"].b, out=q, ln=L["q"].ln(s1))                  # Wq(norm2(x1))
@@ -354,7 +351,7 @@ class Engine:
         s["plan_last_self"].run(q, kvs[:, :D], kvs[:, D:], H, hd, w.slopes, a)
         hb = torch.empty((R, D), dtype=torch.bfloat16, device=x.device)
         s1 = torch.empty((R, ops.stats_parts(D), 2), dtype=torch.float32, device=x.device)
-        ops.gemm(a, L["out"].w, EPI_BIAS_RESID_F32, bias=L["out"].b, resid=xbR if OUT_PROJ_RESID16 else xR, out2=hb,
+        ops.gemm(a, L["out"].w, EPI_BIAS_RESID_F32, bias=L["out"].b, resid=xbR, out2=hb,
                  stats_out=s1, mirror_only=True)
         ops.gemm(hb, L["q"].w, EPI_BIAS_BF16, bias=L["q"].b, out=q, ln=L["q"].ln(s1))
         s["plan_last_cross"].run(q, kv[:, :D], kv[:, D:], H, hd, None, a)

@@ -3,7 +3,6 @@
 for slabs of genes; per-item access with the reference's tuple layout lives in datasets/vcfdataset.py."""
 from dataclasses import dataclass, field
 
-import os
 import numpy as np
 import torch
 
@@ -86,8 +85,7 @@ class HotPath:
         main = torch.cuda.current_stream(self.engine.device)
         if not hasattr(self, "_side"):
             self._side = torch.cuda.Stream(self.engine.device)
-        # VF_STAGE1_STREAM=main: no side stream (timing experiments: what the overlap is worth)
-        side = main if os.environ.get("VF_STAGE1_STREAM") == "main" else self._side
+        side = self._side
         side.wait_stream(main)                          # genome / variants / merge tables were uploaded on `main`
 
         def stage(genes):

@@ -153,12 +153,8 @@ class WindowTokenizer:
                                (load_merge_table_from_hf_json(merges_path) if merges_path.endswith(".json")
                                 else load_merge_table(merges_path)))
         self.device = torch.device(device)
-        # VF_BPE_BATCH=0: every rank its own sweep (A/B timing and the bit-identity test of the batching)
-        if os.environ.get("VF_BPE_BATCH", "1") != "0":
-            order, batch = merge_batches(a, b, c)
-            a, b, c = a[order], b[order], c[order]           # the kernel walks the table in this (equivalent) order
-        else:
-            batch = np.arange(len(a), dtype=np.uint16)
+        order, batch = merge_batches(a, b, c)
+        a, b, c = a[order], b[order], c[order]               # the kernel walks the table in this (equivalent) order
         self.merges = tuple(torch.from_numpy(np.ascontiguousarray(x).view(np.int16)).to(self.device) for x in (a, b, c, batch))
         self.max_length, self.max_chunks = max_length, max_chunks
         self._no_var = SampleVariants({}, device=self.device)
