@@ -211,6 +211,28 @@ int vf_encode_windows(const uint8_t* genome, const int64_t* win_base, const int3
                       const uint8_t* alt_pool, int n_win, int max_window, uint8_t* out, int64_t pitch, int32_t* out_len,
                       int32_t* err, void* stream);
 /*
+ * Which rows of a cohort encode to the same bytes.  Row r = one (window, sample): w0/w1/flags/var_lo/var_hi as in
+ * vf_encode_windows (flags bit1 = SNP-only), the variant arrays those of vf_encode_windows (one concatenated table may
+ * hold every sample's records; each row's [var_lo, var_hi) points at its sample's).  The applied records of a row are
+ * selected with exactly vf_encode_windows' rule (one device function serves both).
+ * vf_window_genotype_keys: keys uint64 [n_rows, 2] = a 128-bit hash of the applied records' (pos, ref_len, gt, alt_len,
+ *   ALT bytes), 0 for a row with none (the reference window); count int32 [n_rows] = the number applied, or -1 where a
+ *   2049th record would apply: such a row sets *err to 2, exactly where vf_encode_windows does; out_len int32
+ *   [n_rows] or NULL = the length vf_encode_windows gives the row, (w1 - w0) + sum(alt_len - ref_len) over the applied
+ *   records (over the first 2048 on a capped row): the row overflows a pitch iff out_len > pitch.
+ * vf_window_genotype_equal: equal int32 [n_rows] = 1 iff row r and row rep[r] (same w0, w1, flags bits 0-1) apply equal
+ *   record lists, element by element; rows of equal lists encode to identical bytes.
+ * One thread per row; any n_rows >= 0; NULL arrays for n_rows > 0 fail before any launch.
+ */
+int vf_window_genotype_keys(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                            const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_off,
+                            const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, int n_rows,
+                            unsigned long long* keys, int32_t* count, int32_t* out_len, int32_t* err, void* stream);
+int vf_window_genotype_equal(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                             const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_off,
+                             const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, int n_rows,
+                             const int32_t* rep, int32_t* equal, void* stream);
+/*
  * Single-base substitution of encoded windows (in-silico saturation mutagenesis): row r of out = the source row
  * src[row_src[r]] (src_len[row_src[r]] bytes, as vf_encode_windows wrote it) with ONE base replaced by row_base[r].
  * row_off[r] = forward-strand offset pos0 - w0 of the base; flags[r] bit0 = the source was reverse-complemented: the base

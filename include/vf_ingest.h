@@ -52,6 +52,27 @@ int vf_vcf_copy(const vf_vcf* v, int c, int64_t* pos, int32_t* ref_len, int32_t*
                 uint8_t* gt, uint8_t* alt_pool);
 void vf_vcf_close(vf_vcf* v);
 
+typedef struct vf_vcf_cohort vf_vcf_cohort;
+/* Parse many samples of a VCF in one pass: each data line is split once and every requested sample column decoded
+ * from it with vf_vcf_open's genotype rules, so sample s's arrays of a chromosome equal what vf_vcf_open(path,
+ * samples[s]) + vf_vcf_copy give (a chromosome where s keeps no record has 0 records).
+ * samples == NULL: every sample column of the '#CHROM' line, in file order (n_samples is ignored).  An unknown or a
+ * twice-requested sample fails, and so does a file without sample columns (a sites-only VCF).  regions_bed: NULL, or BED text ("chrom<TAB>start<TAB>end" lines, 0-based half-open;
+ * '#', 'track' and 'browser' lines skipped): only records whose REF span [pos, pos + max(ref_len, 1)) intersects an
+ * interval are kept, before any genotype is decoded. */
+vf_vcf_cohort* vf_vcf_open_cohort(const char* path, const char* const* samples, int n_samples, const char* regions_bed,
+                                  int n_threads);
+int vf_vcf_cohort_num_samples(const vf_vcf_cohort* v);
+const char* vf_vcf_cohort_sample_name(const vf_vcf_cohort* v, int s);
+int vf_vcf_cohort_num_chroms(const vf_vcf_cohort* v);           /* chromosomes with a kept record of any sample */
+const char* vf_vcf_cohort_chrom(const vf_vcf_cohort* v, int c);
+int64_t vf_vcf_cohort_num_records(const vf_vcf_cohort* v, int s, int c);
+int64_t vf_vcf_cohort_alt_bytes(const vf_vcf_cohort* v, int s, int c);
+/* vf_vcf_copy's arrays of sample s, chromosome c.  Returns 0 or -1. */
+int vf_vcf_cohort_copy(const vf_vcf_cohort* v, int s, int c, int64_t* pos, int32_t* ref_len, int32_t* alt_off,
+                       int32_t* alt_len, uint8_t* gt, uint8_t* alt_pool);
+void vf_vcf_cohort_close(vf_vcf_cohort* v);
+
 #ifdef __cplusplus
 }
 #endif

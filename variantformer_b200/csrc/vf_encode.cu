@@ -42,6 +42,30 @@ __device__ __forceinline__ uint8_t iupac_het(uint8_t ref, uint8_t alt) {   // ve
     return (uint8_t)tbl[r * 4 + a];
 }
 
+// The genotype-application rule of a window [w0, w1), shared by encode_windows and the genotype-key kernels so that
+// grouping rows by key can never drift from what the encoder writes: walk the candidate records [lo, hi) in order and
+// apply a record iff its genotype is not 0, it starts at or after the end of the last applied record, its REF span ends
+// inside the window and, in SNP-only windows, it is a single-base substitution.  next() -> the next applied record's
+// index, or -1.  (The 2048-record cap is the caller's: it is where the encoder's shared-memory table ends.)
+struct AppliedScan {
+    int i, hi, cur, w1;
+    bool snp_only;
+    __device__ __forceinline__ AppliedScan(int lo, int hi_, int w0, int w1_, bool snp)
+        : i(lo), hi(hi_), cur(w0), w1(w1_), snp_only(snp) {}
+    __device__ __forceinline__ int next(const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_len,
+                                        const uint8_t* v_gt) {
+        for (; i < hi; ++i) {
+            if (v_gt[i] == 0) continue;
+            const int pos = v_pos[i], rl = v_ref_len[i], al = v_alt_len[i];
+            if (pos < cur || pos + rl > w1) continue;
+            if (snp_only && !(rl == 1 && al == 1)) continue;
+            cur = pos + rl;
+            return i++;
+        }
+        return -1;
+    }
+};
+
 struct EncodeParams {
     const uint8_t* genome;            // concatenated chromosomes, 1 byte/base as in the FASTA (case kept)
     const int64_t* win_base;          // [n_win] offset of the window's chromosome in `genome`
@@ -69,16 +93,12 @@ encode_windows_kernel(const EncodeParams p) {
     const bool rc = fl & 1, snp_only = fl & 2;
     if (threadIdx.x == 0) {
         // sequential scan: which records are applied (overlap rule needs order) and where they land
-        int n = 0, cur = w0, shift = 0, bad = 0;
-        for (int i = p.var_lo[w]; i < p.var_hi[w]; ++i) {
-            if (p.v_gt[i] == 0) continue;
-            const int pos = p.v_pos[i], rl = p.v_ref_len[i], al = p.v_alt_len[i];
-            if (pos < cur || pos + rl > w1) continue;
-            if (snp_only && !(rl == 1 && al == 1)) continue;
+        int n = 0, shift = 0, bad = 0;
+        AppliedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only);
+        for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)) >= 0;) {
             if (n == kMaxApplied) { bad = 2; break; }
             s_vidx[n] = i; s_shift[n] = shift; ++n;
-            shift += al - rl;
-            cur = pos + rl;
+            shift += p.v_alt_len[i] - p.v_ref_len[i];
         }
         s_n = n; s_total = (w1 - w0) + shift;
         if (bad) atomicMax(p.err, bad);
@@ -150,6 +170,120 @@ int encode_windows(const uint8_t* genome, const int64_t* win_base, const int32_t
         encode_windows_kernel<<<grid, 256, 0, s>>>(p);
         VF_LAUNCH_OK("encode_windows_kernel launch");
     }
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------
+// window_genotype_keys / window_genotype_equal: which (window, sample) rows encode to the same bytes.  Two rows of one
+// window encode identically iff their applied record lists (AppliedScan) are equal, so a 128-bit hash of the list
+// proposes groups and the element-by-element comparison against each group's representative confirms them.  A row's
+// list is a sequential scan (the overlap rule needs order), so one thread owns one row: a cohort's rows are many and
+// short (a CRE window holds 0-2 records of a sample, a gene window a few hundred), and the kernels read only the records
+// in the rows' ranges, never the genome.
+// ---------------------------------------------------------------------------------
+struct GenotypeRows {
+    const int32_t* w0; const int32_t* w1; const int32_t* var_lo; const int32_t* var_hi; const uint8_t* flags;
+    const int32_t* v_pos; const int32_t* v_ref_len; const int32_t* v_alt_off; const int32_t* v_alt_len;
+    const uint8_t* v_gt; const uint8_t* alt_pool;
+    int n_rows;
+    __device__ __forceinline__ AppliedScan scan(int r) const {
+        return AppliedScan(var_lo[r], var_hi[r], w0[r], w1[r], flags[r] & 2);
+    }
+};
+
+__device__ __forceinline__ uint64_t mix64(uint64_t h, uint64_t x, uint64_t mul) {
+    h ^= x;
+    h *= mul;
+    return h ^ (h >> 31);
+}
+
+__global__ void __launch_bounds__(128)
+window_genotype_keys_kernel(const GenotypeRows p, unsigned long long* keys, int32_t* count, int32_t* out_len, int32_t* err) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= p.n_rows) return;
+    constexpr uint64_t kMul0 = 0x9E3779B97F4A7C15ull, kMul1 = 0xC2B2AE3D27D4EB4Full;
+    uint64_t h0 = 0x243F6A8885A308D3ull, h1 = 0x13198A2E03707344ull;
+    int n = 0, shift = 0;
+    bool bad = false;
+    AppliedScan sc = p.scan(r);
+    for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)) >= 0;) {
+        if (n == kMaxApplied) { bad = true; break; }     // the encoder's cap: err 2 on exactly the rows it flags
+        ++n;
+        const int al = p.v_alt_len[i];
+        shift += al - p.v_ref_len[i];
+        const uint64_t a = ((uint64_t)(uint32_t)p.v_pos[i] << 32) | (uint32_t)p.v_ref_len[i];
+        const uint64_t b = ((uint64_t)p.v_gt[i] << 32) | (uint32_t)al;
+        h0 = mix64(mix64(h0, a, kMul0), b, kMul0);
+        h1 = mix64(mix64(h1, b, kMul1), a, kMul1);
+        const uint8_t* s = p.alt_pool + p.v_alt_off[i];
+        for (int j = 0; j < al; j += 8) {
+            uint64_t w = 0;
+            for (int k = 0; k < 8 && j + k < al; ++k) w |= (uint64_t)s[j + k] << (8 * k);
+            h0 = mix64(h0, w, kMul0);
+            h1 = mix64(h1, w ^ 0x5555555555555555ull, kMul1);
+        }
+    }
+    if (bad) atomicMax(err, 2);
+    count[r] = bad ? -1 : n;
+    if (out_len) out_len[r] = (p.w1[r] - p.w0[r]) + shift;   // what encode_windows checks against its pitch
+    keys[2 * r] = n ? h0 : 0ull;                         // the empty list (the reference window) is key 0
+    keys[2 * r + 1] = n ? h1 : 0ull;
+}
+
+__global__ void __launch_bounds__(128)
+window_genotype_equal_kernel(const GenotypeRows p, const int32_t* rep, int32_t* equal) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= p.n_rows) return;
+    const int q = rep[r];
+    if (q == r) { equal[r] = 1; return; }
+    int eq = p.w0[r] == p.w0[q] && p.w1[r] == p.w1[q] && ((p.flags[r] ^ p.flags[q]) & 3) == 0;
+    AppliedScan a = p.scan(r), b = p.scan(q);
+    while (eq) {
+        const int i = a.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt);
+        const int j = b.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt);
+        if (i < 0 || j < 0) { eq = i == j; break; }
+        const int al = p.v_alt_len[i];
+        if (p.v_pos[i] != p.v_pos[j] || p.v_ref_len[i] != p.v_ref_len[j] || p.v_gt[i] != p.v_gt[j] ||
+            al != p.v_alt_len[j]) { eq = 0; break; }
+        const uint8_t* x = p.alt_pool + p.v_alt_off[i];
+        const uint8_t* y = p.alt_pool + p.v_alt_off[j];
+        for (int k = 0; k < al; ++k)
+            if (x[k] != y[k]) { eq = 0; break; }
+    }
+    equal[r] = eq;
+}
+
+static int genotype_rows_check(const GenotypeRows& g, const char* what) {
+    VF_REQUIRE(g.n_rows >= 0, "%s: n_rows %d < 0", what, g.n_rows);
+    if (g.n_rows == 0) return 0;
+    VF_REQUIRE(g.w0 && g.w1 && g.var_lo && g.var_hi && g.flags && g.v_pos && g.v_ref_len && g.v_alt_off && g.v_alt_len &&
+               g.v_gt && g.alt_pool, "%s: a row or variant array is NULL", what);
+    return 0;
+}
+
+int window_genotype_keys(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                         const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_off,
+                         const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, int n_rows,
+                         unsigned long long* keys, int32_t* count, int32_t* out_len, int32_t* err, cudaStream_t s) {
+    const GenotypeRows g{w0, w1, var_lo, var_hi, flags, v_pos, v_ref_len, v_alt_off, v_alt_len, v_gt, alt_pool, n_rows};
+    if (const int rc = genotype_rows_check(g, "window_genotype_keys")) return rc;
+    if (n_rows == 0) return 0;
+    VF_REQUIRE(keys && count && err, "window_genotype_keys: keys, count and err are required");
+    window_genotype_keys_kernel<<<(n_rows + 127) / 128, 128, 0, s>>>(g, keys, count, out_len, err);
+    VF_LAUNCH_OK("window_genotype_keys_kernel launch");
+    return 0;
+}
+
+int window_genotype_equal(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                          const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_off,
+                          const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, int n_rows,
+                          const int32_t* rep, int32_t* equal, cudaStream_t s) {
+    const GenotypeRows g{w0, w1, var_lo, var_hi, flags, v_pos, v_ref_len, v_alt_off, v_alt_len, v_gt, alt_pool, n_rows};
+    if (const int rc = genotype_rows_check(g, "window_genotype_equal")) return rc;
+    if (n_rows == 0) return 0;
+    VF_REQUIRE(rep && equal, "window_genotype_equal: rep and equal are required");
+    window_genotype_equal_kernel<<<(n_rows + 127) / 128, 128, 0, s>>>(g, rep, equal);
+    VF_LAUNCH_OK("window_genotype_equal_kernel launch");
     return 0;
 }
 

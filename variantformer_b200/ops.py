@@ -468,6 +468,50 @@ def encode_windows(genome, win_base, w0, w1, var_lo, var_hi, flags, variants, ma
     return out, out_len, err
 
 
+def _genotype_rows(w0, w1, var_lo, var_hi, flags, variants):
+    n = w0.numel()
+    for t in (w0, w1, var_lo, var_hi):
+        assert t.dtype == torch.int32 and t.numel() == n and t.is_contiguous()
+    assert flags.dtype == torch.uint8 and flags.numel() == n
+    v = variants
+    return n, [ptr(w0), ptr(w1), ptr(var_lo), ptr(var_hi), ptr(flags), ptr(v["pos"]), ptr(v["ref_len"]), ptr(v["alt_off"]),
+               ptr(v["alt_len"]), ptr(v["gt"]), ptr(v["alt_pool"]), n]
+
+
+def window_genotype_keys(w0, w1, var_lo, var_hi, flags, variants, key_bits=128, err=None):
+    """Genotype keys of (window, sample) rows (vf_window_genotype_keys): rows as encode_windows takes them, variants
+    the dict of device arrays (stage1.SampleVariants.dev / CohortVariants.dev).  -> (keys int64 [n, 2] (the 128-bit key
+    as two words, 0 for the reference window), count int32 [n] (applied records; -1 past the 2048-record cap, which
+    sets err to 2), lens int32 [n] (the encoded length encode_windows checks against its pitch), err).  key_bits < 128 keeps only the low bits of the key (tests: forces collisions, which
+    window_genotype_equal then separates)."""
+    n, args = _genotype_rows(w0, w1, var_lo, var_hi, flags, variants)
+    dev = w0.device
+    keys = torch.empty((n, 2), dtype=torch.int64, device=dev)
+    count = torch.empty(n, dtype=torch.int32, device=dev)
+    lens = torch.empty(n, dtype=torch.int32, device=dev)
+    if err is None:
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+    with _timed("stage1_keys"):
+        check(_lib.lib().vf_window_genotype_keys(*args, ptr(keys), ptr(count), ptr(lens), ptr(err), stream()))
+    if key_bits < 64:
+        keys[:, 0] &= (1 << key_bits) - 1
+        keys[:, 1] = 0
+    elif key_bits < 128:
+        keys[:, 1] &= (1 << (key_bits - 64)) - 1
+    return keys, count, lens, err
+
+
+def window_genotype_equal(w0, w1, var_lo, var_hi, flags, variants, rep):
+    """1 where row r applies the same record list as row rep[r] (int32 [n] device), element by element
+    (vf_window_genotype_equal).  -> int32 [n]."""
+    n, args = _genotype_rows(w0, w1, var_lo, var_hi, flags, variants)
+    assert rep.dtype == torch.int32 and rep.numel() == n
+    equal = torch.empty(n, dtype=torch.int32, device=w0.device)
+    with _timed("stage1_keys"):
+        check(_lib.lib().vf_window_genotype_equal(*args, ptr(rep), ptr(equal), stream()))
+    return equal
+
+
 def mutate_windows(src, src_len, row_src, row_off, row_base, flags, err=None):
     """Single-base substitutions of encoded windows (vf_mutate_windows): row r = src[row_src[r]] with the base at
     forward-strand offset row_off[r] replaced by row_base[r] (complemented on reverse-complemented rows, flags bit 0).

@@ -187,6 +187,14 @@ class HotPath:
             return pred, emb, (maps[0].cpu().numpy(), maps[1])
         return pred, emb
 
+    def predict_cohort(self, genes, cohort, sample_idx=None, to_host=True, **kw):
+        """Every (sample, gene) of a cohort (stage1.CohortVariants; sample_idx: which of its samples, default all) with
+        each distinct window encoded once across samples (cohort.predict_cohort).  -> (pred [S, sum T], emb [S, sum T,
+        D]) in (sample, gene, tissue) order, numpy (to_host) or device tensors; row s is bit-identical to
+        predict(genes, that sample's SampleVariants)."""
+        from .cohort import predict_cohort
+        return predict_cohort(self, genes, cohort, sample_idx, to_host=to_host, **kw)
+
     @staticmethod
     def _raise_on_stage1_error(err):
         """The encode kernel flags windows it could not build (their tokens are then all padding): never hand out

@@ -106,6 +106,103 @@ class VCFProcessor:
                 frames.append(df); maps.update(m)
         return pd.concat(frames, ignore_index=True), maps
 
+    def predict_cohort(self, vcf_path: str, query_df: pd.DataFrame, output_dir=None, samples=None, embeddings=True,
+                       genes_per_slab=8, samples_per_slab=256):
+        """Every (sample, gene, tissue) of the query for the samples of one multi-sample VCF (samples: names, default
+        every sample column), with one region-restricted parse of the VCF and each distinct window encoded once across
+        samples (variantformer_b200.cohort, DESIGN.md section 14).  The query is filtered with VCFDataset's rules; each
+        prediction equals what create_data + predict give for that sample alone.
+        -> output_dir None: a long DataFrame (sample, gene_id, tissue (name), predicted_expression[, embeddings]) in
+        (sample, gene, tissue) order.  Else: results go through ResultWriter into output_dir, one Parquet file per slab
+        (genes_per_slab query genes x samples_per_slab samples; slab index = gene block x number of sample blocks +
+        sample block, a function of the query and the sample list only), slabs already on disk are skipped, and the
+        directory is returned.  A sample block whose variant table would pass 2^31 records or ALT bytes is computed in
+        sub-blocks (CohortVariants.blocks) and still written as one slab."""
+        from .. import ingest
+        from ..pipeline import GeneSpec, HotPath
+        from ..stage1 import CohortVariants, cre_window, gene_window
+        ds = self.model_config.dataset
+        dataset = VCFDataset(max_length=ds.max_length, max_chunks=ds.max_chunks, cre_neighbour_hood=ds.cre_neighbour_hood,
+                             gencode_v24=ds.gencode_v24, gene_cre_manifest=self.gene_cre_manifest,
+                             gene_upstream_neighbour_hood=ds.gene_upstream_neighbour_hood,
+                             gene_downstream_neighbour_hood=ds.gene_downstream_neighbour_hood, query_df=query_df,
+                             fasta_path=self.vcf_loader_config.fasta_path, vcf_path=None)
+        q = dataset.query_df
+        genes, gene_ids, tissue_names, regions = [], [], [], []
+        nb, up, down = ds.cre_neighbour_hood, ds.gene_upstream_neighbour_hood, ds.gene_downstream_neighbour_hood
+        for _, row in q.iterrows():
+            info = dataset._get_gene_info(row["gene_id"])
+            assert info["chromosome"] in ["chr" + str(i) for i in range(1, 23)], \
+                f"Chromosome {info['chromosome']} is not a valid chromosome. Sex chromosomes are not supported"
+            m, _ = dataset.cre_manifest(row["gene_id"], info)
+            labels = np.asarray([dataset.ref_cre_to_idx[x] for x in m["cre_name"]], np.int64)
+            genes.append(GeneSpec(info["chromosome"], int(info["start"]), int(info["end"]), info["strand"],
+                                  m["start_cre"].to_numpy(np.int64), m["end_cre"].to_numpy(np.int64), labels,
+                                  list(row["tissues"]), cre_chrom=list(m["chromosome"])))
+            gene_ids.append(row["gene_id"]); tissue_names.append(list(row["tissue_names"]))
+            regions += [(c, *cre_window(s, e, nb)) for c, s, e in zip(m["chromosome"], m["start_cre"], m["end_cre"])]
+            regions.append((info["chromosome"], *gene_window(info["start"], info["end"], info["strand"], up, down)))
+        names, per_sample = ingest.load_vcf_cohort(vcf_path, samples=samples, regions=regions)
+        model, _, _ = self.load_model()
+        hot = HotPath(model.engine(), dataset._genome(), max_length=ds.max_length, max_chunks=ds.max_chunks,
+                      cre_neighbour_hood=nb, gene_upstream=up, gene_downstream=down)
+        g_blocks = [(a, min(len(genes), a + genes_per_slab)) for a in range(0, len(genes), genes_per_slab)]
+        s_blocks = [(a, min(len(names), a + samples_per_slab)) for a in range(0, len(names), samples_per_slab)]
+        writer = None
+        if output_dir is not None:
+            from ..writer import ResultWriter
+            writer = ResultWriter(output_dir, hot.engine.w.D, embeddings=embeddings,
+                                  meta={"cohort": os.path.basename(vcf_path), "samples": names, "genes": gene_ids,
+                                        "tissues": [list(map(int, g.tissues)) for g in genes],
+                                        "genes_per_slab": genes_per_slab, "samples_per_slab": samples_per_slab})
+            done = writer.done()
+        frames = {}
+        try:
+            for sb, (s0, s1) in enumerate(s_blocks):
+                todo = [gb for gb in range(len(g_blocks)) if writer is None or gb * len(s_blocks) + sb not in done]
+                if not todo:
+                    continue
+                # sample sub-blocks whose variant tables fit the kernels' int32 indices (one, short of 2^31 records)
+                subs = CohortVariants.blocks(per_sample[s0:s1])
+                table = lambda a, b: CohortVariants(names[s0 + a:s0 + b], per_sample[s0 + a:s0 + b], hot.engine.device)
+                kept = table(*subs[0]) if len(subs) == 1 else None
+                for gb in todo:
+                    g0, g1 = g_blocks[gb]
+                    parts = [hot.predict_cohort(genes[g0:g1], kept if kept is not None else table(a, b),
+                                                min_gene_len=1000, gene_names=gene_ids[g0:g1]) for a, b in subs]
+                    pred = np.concatenate([p for p, _ in parts]); emb = np.concatenate([e for _, e in parts])
+                    del parts
+                    rows = [(k, names[s0 + s], gene_ids[g0 + k], int(t), tn)
+                            for s in range(s1 - s0) for k in range(g1 - g0)
+                            for t, tn in zip(genes[g0 + k].tissues, tissue_names[g0 + k])]
+                    pred = pred.reshape(-1); emb = emb.reshape(len(rows), -1)
+                    if writer is not None:
+                        writer.submit(gb * len(s_blocks) + sb, [r[:4] for r in rows], pred, emb)
+                    else:
+                        frames[(sb, gb)] = (rows, pred, emb)
+        finally:
+            if writer is not None:
+                writer.close()
+        if writer is not None:
+            return output_dir
+        # (sample, gene, tissue) order: sample blocks outer, then sample, gene block, gene, tissue
+        out = []
+        for sb, (s0, s1) in enumerate(s_blocks):
+            parts = [frames[(sb, gb)] for gb in range(len(g_blocks))]
+            per_s = [[] for _ in range(s1 - s0)]
+            for (g0, g1), (rows, pred, emb) in zip(g_blocks, parts):
+                n = len(rows) // (s1 - s0)
+                for s in range(s1 - s0):
+                    per_s[s].append((rows[s * n:(s + 1) * n], pred[s * n:(s + 1) * n], emb[s * n:(s + 1) * n]))
+            for lst in per_s:
+                for rows, pred, emb in lst:
+                    d = {"sample": [r[1] for r in rows], "gene_id": [r[2] for r in rows], "tissue": [r[4] for r in rows],
+                         "predicted_expression": pred}
+                    if embeddings:
+                        d["embeddings"] = list(emb)
+                    out.append(pd.DataFrame(d))
+        return pd.concat(out, ignore_index=True)
+
     def format_output(self, df, predictions):
         pred_exp, embd = [], []
         for p in predictions:

@@ -133,6 +133,87 @@ class SampleVariants:
         return base + int(np.searchsorted(p, w0, "left")), base + int(np.searchsorted(p, w1, "left"))
 
 
+INT32_LIMIT = 2 ** 31 - 1
+
+
+class CohortVariants:
+    """Many samples' variants in one device table: every sample's records concatenated sample-major, then by chromosome,
+    then by position, in the six arrays of SampleVariants.dev.  A row (window, sample) of vf_encode_windows points at its
+    sample's records through var_lo / var_hi (window_ranges), so one encode batch may mix samples.  The kernels index
+    records and ALT bytes with int32: a table past 2^31 of either is refused (split the samples: `blocks`)."""
+
+    def __init__(self, names, per_sample, device="cuda"):
+        self.names = list(names)
+        assert len(self.names) == len(per_sample)
+        self.chroms = list(dict.fromkeys(c for d in per_sample for c in d))
+        self.chrom_idx = {c: i for i, c in enumerate(self.chroms)}
+        n_rec, n_alt = self.sizes(per_sample)
+        if n_rec > INT32_LIMIT or n_alt > INT32_LIMIT:
+            raise ValueError(f"{n_rec} records / {n_alt} ALT bytes do not fit int32 indices: split the samples "
+                             "(CohortVariants.blocks)")
+        keys, pos, rl, al, gt, alts = [], [], [], [], [], []
+        nc = len(self.chroms)
+        self.n_records = np.zeros(len(self.names), np.int64)
+        for s, d in enumerate(per_sample):
+            for c in self.chroms:
+                if c not in d:
+                    continue
+                v = d[c]
+                p = np.asarray(v["pos"], np.int64)
+                assert (np.diff(p) >= 0).all(), "variants must be sorted by position"
+                keys.append((s * nc + self.chrom_idx[c]) * (1 << 32) + p)
+                pos.append(p.astype(np.int32)); rl.append(np.asarray(v["ref_len"], np.int32))
+                gt.append(np.asarray(v["gt"], np.uint8))
+                a = [x.encode() if isinstance(x, str) else bytes(x) for x in v["alt"]]
+                al.append(np.asarray([len(x) for x in a], np.int32)); alts += a
+                self.n_records[s] += len(p)
+        cat = lambda xs, dt: np.concatenate(xs).astype(dt) if xs else np.zeros(0, dt)
+        self.key = cat(keys, np.int64)               # (segment << 32) + pos: sorted, one segment per (sample, chrom)
+        lens = cat(al, np.int32)
+        off = (np.cumsum(lens, dtype=np.int64) - lens).astype(np.int32)
+        pool = np.frombuffer(b"".join(alts), np.uint8).copy() if alts else np.zeros(0, np.uint8)
+        up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt) if len(a) else np.zeros(1, dt)).to(device)
+        self.dev = dict(pos=up(cat(pos, np.int32), np.int32), ref_len=up(cat(rl, np.int32), np.int32),
+                        alt_off=up(off, np.int32), alt_len=up(lens, np.int32), gt=up(cat(gt, np.uint8), np.uint8),
+                        alt_pool=up(pool, np.uint8))
+
+    @staticmethod
+    def sizes(per_sample):
+        """(records, ALT bytes) of a list of per-sample dicts."""
+        n_rec = sum(len(v["pos"]) for d in per_sample for v in d.values())
+        n_alt = sum(len(a) for d in per_sample for v in d.values() for a in v["alt"])
+        return n_rec, n_alt
+
+    @staticmethod
+    def blocks(per_sample, limit=None):
+        """Consecutive sample ranges [a, b) whose tables fit int32 indices (records and ALT bytes <= limit; a single
+        sample past it stays alone, and CohortVariants refuses it as SampleVariants' int32 arrays cannot hold it)."""
+        limit = INT32_LIMIT if limit is None else limit
+        out, a = [], 0
+        while a < len(per_sample):
+            b, rec, alt = a, 0, 0
+            while b < len(per_sample):
+                r, x = CohortVariants.sizes([per_sample[b]])
+                if b > a and (rec + r > limit or alt + x > limit):
+                    break
+                rec += r; alt += x; b += 1
+            out.append((a, b))
+            a = b
+        return out
+
+    def window_ranges(self, sample_idx, chroms, w0, w1):
+        """Vectorised var_lo / var_hi (int64 numpy) of rows (sample_idx[i], chroms[i], [w0[i], w1[i])) into the
+        concatenated arrays: the records of that sample and chromosome with pos in [w0, w1)."""
+        s = np.asarray(sample_idx, np.int64)
+        names, inv = np.unique(np.asarray(chroms, dtype=object).astype(str), return_inverse=True)
+        c = np.asarray([self.chrom_idx.get(x, -1) for x in names], np.int64)[inv.reshape(-1)]
+        seg = (s * len(self.chroms) + np.maximum(c, 0)) * (1 << 32)
+        lo = np.searchsorted(self.key, seg + np.asarray(w0, np.int64), "left")
+        hi = np.searchsorted(self.key, seg + np.asarray(w1, np.int64), "left")
+        hi = np.where(c < 0, lo, hi)                 # a chromosome no sample has a record on
+        return lo, hi
+
+
 def cre_window(start, end, nb):
     return max(0, int(start) - nb), int(end) + nb
 
