@@ -195,6 +195,14 @@ class HotPath:
         from .cohort import predict_cohort
         return predict_cohort(self, genes, cohort, sample_idx, to_host=to_host, **kw)
 
+    def cre_knockout(self, genes, knockouts=None, variants: SampleVariants = None, embeddings=False, to_host=True, **kw):
+        """In-silico CRE knockout (knockout.cre_knockout): knockouts[i] = list of index arrays into gene i's CRE arrays
+        (manifest rows), None = every CRE singly.  -> (pred [sum T], emb [sum T, D]) of the baseline, bit-identical to
+        predict(genes, variants), and per gene the knockout predictions [K_g, T_g] (+ per gene [K_g, T_g, D] embeddings
+        when `embeddings`), each bit-identical to predict on the gene with those rows removed."""
+        from .knockout import cre_knockout
+        return cre_knockout(self, genes, knockouts, variants, embeddings=embeddings, to_host=to_host, **kw)
+
     @staticmethod
     def _raise_on_stage1_error(err):
         """The encode kernel flags windows it could not build (their tokens are then all padding): never hand out

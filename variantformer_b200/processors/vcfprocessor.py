@@ -203,6 +203,74 @@ class VCFProcessor:
                     out.append(pd.DataFrame(d))
         return pd.concat(out, ignore_index=True)
 
+    def cre_knockout(self, vcf_path: str, query_df: pd.DataFrame, knockouts: pd.DataFrame = None):
+        """In-silico CRE knockout (DESIGN.md section 15): every query row predicted with one CRE, or a set of CREs,
+        removed from its gene's manifest, each distinct window encoded once.  A knockout's prediction equals what
+        create_data + predict give with those rows deleted from the manifest.  The query is filtered with VCFDataset's
+        rules; the sample is `vcf_path` or a per-row vcf_path column (empty or missing: the reference genome).
+        knockouts: None = every CRE of every query gene singly (a gene with one CRE gets none), or a DataFrame with
+        columns gene_id, knockout (a label) and cre_index (a manifest row; one row per member of the set).  Invalid sets
+        raise a ValueError before any device work.  Writes no file.
+        -> one row per (query row, knockout, tissue), in that order (default knockouts in manifest order, user sets in
+        first-appearance order): gene_id, tissue (name), knockout (label; the manifest row for the default scan),
+        cre_indices, the manifest columns of a single-CRE knockout (null for larger sets), baseline_expression,
+        predicted_expression and delta = predicted - baseline."""
+        from .. import knockout as ko
+        from ..pipeline import GeneSpec, HotPath
+        ds = self.model_config.dataset
+        dataset = VCFDataset(max_length=ds.max_length, max_chunks=ds.max_chunks, cre_neighbour_hood=ds.cre_neighbour_hood,
+                             gencode_v24=ds.gencode_v24, gene_cre_manifest=self.gene_cre_manifest,
+                             gene_upstream_neighbour_hood=ds.gene_upstream_neighbour_hood,
+                             gene_downstream_neighbour_hood=ds.gene_downstream_neighbour_hood, query_df=query_df,
+                             fasta_path=self.vcf_loader_config.fasta_path, vcf_path=vcf_path)
+        q = dataset.query_df
+        user = ko.knockout_sets(knockouts) if knockouts is not None else None
+        genes, manifests, sets, paths = [], [], [], []
+        for _, row in q.iterrows():
+            gid = row["gene_id"]
+            info = dataset._get_gene_info(gid)
+            assert info["chromosome"] in ["chr" + str(i) for i in range(1, 23)], \
+                f"Chromosome {info['chromosome']} is not a valid chromosome. Sex chromosomes are not supported"
+            m, _ = dataset.cre_manifest(gid, info)
+            labels = np.asarray([dataset.ref_cre_to_idx[x] for x in m["cre_name"]], np.int64)
+            genes.append(GeneSpec(info["chromosome"], int(info["start"]), int(info["end"]), info["strand"],
+                                  m["start_cre"].to_numpy(np.int64), m["end_cre"].to_numpy(np.int64), labels,
+                                  list(row["tissues"]), cre_chrom=list(m["chromosome"])))
+            manifests.append(m)
+            if user is not None:
+                sets.append(user.get(gid, []))
+            elif len(m) > 1:
+                sets.append([(i, np.asarray([i], np.int64)) for i in range(len(m))])
+            else:
+                print(f"Gene {gid} has a single CRE so skipping its knockouts")
+                sets.append([])
+            p = row["vcf_path"] if "vcf_path" in q.columns else vcf_path
+            paths.append(None if p is None or (not isinstance(p, str) and pd.isna(p)) or str(p) == "" else str(p))
+        if user is not None:
+            for gid in user:
+                if gid not in set(q["gene_id"]):
+                    print(f"Gene {gid} of the knockouts is not in the query so skipping it")
+        gene_ids = list(q["gene_id"])
+        checked = ko.check_knockouts(genes, [[ix for _, ix in s] for s in sets], gene_ids,
+                                     [[lab for lab, _ in s] for s in sets])
+        sets = [[(lab, ix) for (lab, _), ix in zip(s, c)] for s, c in zip(sets, checked)]
+        model, _, _ = self.load_model()
+        hot = HotPath(model.engine(), dataset._genome(), max_length=ds.max_length, max_chunks=ds.max_chunks,
+                      cre_neighbour_hood=ds.cre_neighbour_hood, gene_upstream=ds.gene_upstream_neighbour_hood,
+                      gene_downstream=ds.gene_downstream_neighbour_hood)
+        base, kos = [None] * len(genes), [None] * len(genes)
+        for p in dict.fromkeys(paths):                       # one call per sample, in first-appearance order
+            rows = [i for i, x in enumerate(paths) if x == p]
+            pred, _, ko_pred = hot.cre_knockout([genes[i] for i in rows], [[ix for _, ix in sets[i]] for i in rows],
+                                                dataset._variants(p), min_gene_len=1000,
+                                                gene_names=[gene_ids[i] for i in rows])
+            off = np.concatenate([[0], np.cumsum([len(genes[i].tissues) for i in rows])])
+            for k, i in enumerate(rows):
+                base[i], kos[i] = pred[off[k]:off[k + 1]], ko_pred[k]
+        frames = [ko.knockout_frame(gid, list(q["tissue_names"].iloc[i]), manifests[i], sets[i], base[i], kos[i])
+                  for i, gid in enumerate(gene_ids)]
+        return pd.concat(frames, ignore_index=True)
+
     def format_output(self, df, predictions):
         pred_exp, embd = [], []
         for p in predictions:
