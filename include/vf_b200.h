@@ -211,6 +211,22 @@ int vf_encode_windows(const uint8_t* genome, const int64_t* win_base, const int3
                       const uint8_t* alt_pool, int n_win, int max_window, uint8_t* out, int64_t pitch, int32_t* out_len,
                       int32_t* err, void* stream);
 /*
+ * vf_encode_windows with ONE extra record per row (in-silico deletions, variant edits against a sample background): row w
+ * is encoded as vf_encode_windows encodes it on the table with the record {pos e_pos[w], ref_len e_ref_len[w], ALT
+ * e_alt_pool[e_alt_off[w], + e_alt_len[w]), gt 2 (hom-alt)} inserted into [var_lo[w], var_hi[w]) right after every record
+ * with pos <= e_pos[w], bit for bit: the same rule decides, in the same kernel body, whether it applies.  The extra
+ * record counts toward the 2048-record cap.  applied uint8 [n_win] = 1 iff row w's extra record was applied (it then
+ * lies in [w0, w1), no earlier applied record overlaps its position and it is not dropped by the SNP-only filter).
+ * Other arguments, outputs and errors as vf_encode_windows; n_win < 0 or a NULL array fails before any launch.
+ */
+int vf_encode_windows_edit(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
+                           const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
+                           const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
+                           const uint8_t* v_gt, const uint8_t* alt_pool, const int32_t* e_pos, const int32_t* e_ref_len,
+                           const int32_t* e_alt_off, const int32_t* e_alt_len, const uint8_t* e_alt_pool, int n_win,
+                           int max_window, uint8_t* out, int64_t pitch, int32_t* out_len, uint8_t* applied,
+                           int32_t* err, void* stream);
+/*
  * Which rows of a cohort encode to the same bytes.  Row r = one (window, sample): w0/w1/flags/var_lo/var_hi as in
  * vf_encode_windows (flags bit1 = SNP-only), the variant arrays those of vf_encode_windows (one concatenated table may
  * hold every sample's records; each row's [var_lo, var_hi) points at its sample's).  The applied records of a row are

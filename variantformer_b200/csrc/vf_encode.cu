@@ -52,17 +52,50 @@ struct AppliedScan {
     bool snp_only;
     __device__ __forceinline__ AppliedScan(int lo, int hi_, int w0, int w1_, bool snp)
         : i(lo), hi(hi_), cur(w0), w1(w1_), snp_only(snp) {}
+    // the rule for one record with a non-zero genotype that comes next in order: applies it (true) or skips it
+    __device__ __forceinline__ bool take(int pos, int rl, int al) {
+        if (pos < cur || pos + rl > w1) return false;
+        if (snp_only && !(rl == 1 && al == 1)) return false;
+        cur = pos + rl;
+        return true;
+    }
     __device__ __forceinline__ int next(const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_len,
                                         const uint8_t* v_gt) {
         for (; i < hi; ++i) {
             if (v_gt[i] == 0) continue;
-            const int pos = v_pos[i], rl = v_ref_len[i], al = v_alt_len[i];
-            if (pos < cur || pos + rl > w1) continue;
-            if (snp_only && !(rl == 1 && al == 1)) continue;
-            cur = pos + rl;
-            return i++;
+            if (take(v_pos[i], v_ref_len[i], v_alt_len[i])) return i++;
         }
         return -1;
+    }
+};
+
+// vf_encode_windows_edit: one extra hom-alt record per row, merged into the row's candidates.  It is walked right after
+// every candidate whose pos is <= its own (a VCF line placed after the records of its position) and judged by
+// AppliedScan's own rule, so a row encodes exactly as vf_encode_windows does on the table with the record inserted.
+// next() returns kExtra for it.
+constexpr int kExtra = 0x7FFFFFFF;
+
+struct MergedScan {
+    AppliedScan sc;
+    int hi, x_pos, x_rl, x_al;
+    bool pending;
+    __device__ __forceinline__ MergedScan(int lo, int hi_, int w0, int w1, bool snp, int xp, int xr, int xa,
+                                          const int32_t* v_pos)
+        : sc(lo, hi_, w0, w1, snp), hi(hi_), x_pos(xp), x_rl(xr), x_al(xa), pending(true) {
+        int a = lo, b = hi_;                               // the candidates are sorted by pos: first one past x_pos
+        while (a < b) { const int m = (a + b) >> 1; if (v_pos[m] <= xp) a = m + 1; else b = m; }
+        sc.hi = a;
+    }
+    __device__ __forceinline__ int next(const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_len,
+                                        const uint8_t* v_gt) {
+        if (pending) {
+            const int i = sc.next(v_pos, v_ref_len, v_alt_len, v_gt);
+            if (i >= 0) return i;
+            pending = false;
+            sc.hi = hi;
+            if (sc.take(x_pos, x_rl, x_al)) return kExtra;
+        }
+        return sc.next(v_pos, v_ref_len, v_alt_len, v_gt);
     }
 };
 
@@ -80,8 +113,17 @@ struct EncodeParams {
     int32_t* err;                     // device error flag (1 = pitch overflow, 2 = too many variants)
 };
 
+struct EditParams {                   // vf_encode_windows_edit: the extra record of every row (unused by the plain kernel)
+    const int32_t* pos; const int32_t* ref_len; const int32_t* alt_off; const int32_t* alt_len;   // [n_win]
+    const uint8_t* alt_pool;
+    uint8_t* applied;                 // [n_win] 1 = the row's extra record was applied
+};
+
+// kEdit = false: vf_encode_windows.  kEdit = true: the same body over MergedScan; record index kExtra reads the row's
+// extra record (hom-alt) wherever the plain kernel reads the table.
+template <bool kEdit>
 __global__ void __launch_bounds__(256)
-encode_windows_kernel(const EncodeParams p) {
+encode_windows_kernel(const EncodeParams p, const EditParams e) {
     __shared__ int32_t s_vidx[kMaxApplied];     // applied variant index
     __shared__ int32_t s_shift[kMaxApplied];    // cumulative (alt_len - ref_len) BEFORE this variant
     __shared__ int s_n, s_total;
@@ -91,20 +133,38 @@ encode_windows_kernel(const EncodeParams p) {
     if (slice0 >= w1 && !(blockIdx.x == 0)) return;
     const uint8_t fl = p.flags[w];
     const bool rc = fl & 1, snp_only = fl & 2;
+    int x_pos = 0, x_rl = 0, x_al = 0;
+    if constexpr (kEdit) { x_pos = e.pos[w]; x_rl = e.ref_len[w]; x_al = e.alt_len[w]; }
+    const auto POS = [&](int v) { return kEdit && v == kExtra ? x_pos : p.v_pos[v]; };
+    const auto RL = [&](int v) { return kEdit && v == kExtra ? x_rl : p.v_ref_len[v]; };
+    const auto AL = [&](int v) { return kEdit && v == kExtra ? x_al : p.v_alt_len[v]; };
+    const auto ALT = [&](int v, int j) { return kEdit && v == kExtra ? e.alt_pool[e.alt_off[w] + j] : p.alt_pool[p.v_alt_off[v] + j]; };
+    const auto GT = [&](int v) { return kEdit && v == kExtra ? (uint8_t)2 : p.v_gt[v]; };
     if (threadIdx.x == 0) {
         // sequential scan: which records are applied (overlap rule needs order) and where they land
         int n = 0, shift = 0, bad = 0;
-        AppliedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only);
-        for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)) >= 0;) {
-            if (n == kMaxApplied) { bad = 2; break; }
-            s_vidx[n] = i; s_shift[n] = shift; ++n;
-            shift += p.v_alt_len[i] - p.v_ref_len[i];
+        bool took = false;
+        auto scan = [&](auto& sc) {
+            for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)) >= 0;) {
+                if (n == kMaxApplied) { bad = 2; break; }
+                if (kEdit && i == kExtra) took = true;
+                s_vidx[n] = i; s_shift[n] = shift; ++n;
+                shift += AL(i) - RL(i);
+            }
+        };
+        if constexpr (kEdit) {
+            MergedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only, x_pos, x_rl, x_al, p.v_pos);
+            scan(sc);
+        } else {
+            AppliedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only);
+            scan(sc);
         }
         s_n = n; s_total = (w1 - w0) + shift;
         if (bad) atomicMax(p.err, bad);
         if (s_total > p.pitch) atomicMax(p.err, 1);
         // an overflowing window writes nothing: report length 0 (plus err = 1) so the tokenizer never reads past the row
         if (blockIdx.x == 0) p.out_len[w] = s_total > p.pitch ? 0 : s_total;
+        if constexpr (kEdit) { if (blockIdx.x == 0) e.applied[w] = took; }
     }
     __syncthreads();
     const int n = s_n, total = s_total;
@@ -116,12 +176,12 @@ encode_windows_kernel(const EncodeParams p) {
     for (int x = slice0 + threadIdx.x; x < slice1; x += blockDim.x) {
         // last applied variant with pos <= x
         int lo = 0, hi = n;
-        while (lo < hi) { const int mid = (lo + hi) >> 1; if (p.v_pos[s_vidx[mid]] <= x) lo = mid + 1; else hi = mid; }
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (POS(s_vidx[mid]) <= x) lo = mid + 1; else hi = mid; }
         int shift = 0;
         if (lo > 0) {
             const int v = s_vidx[lo - 1];
-            if (x < p.v_pos[v] + p.v_ref_len[v]) continue;              // replaced by the record's ALT
-            shift = s_shift[lo - 1] + p.v_alt_len[v] - p.v_ref_len[v];
+            if (x < POS(v) + RL(v)) continue;                           // replaced by the record's ALT
+            shift = s_shift[lo - 1] + AL(v) - RL(v);
         }
         const int o = x - w0 + shift;
         const uint8_t b = ref[x];
@@ -130,13 +190,13 @@ encode_windows_kernel(const EncodeParams p) {
     // (2) ALT bytes of the applied records that start inside this slice
     for (int k = threadIdx.x; k < n; k += blockDim.x) {
         const int v = s_vidx[k];
-        const int pos = p.v_pos[v];
+        const int pos = POS(v);
         if (pos < slice0 || pos >= slice1) continue;
-        const int al = p.v_alt_len[v], rl = p.v_ref_len[v];
+        const int al = AL(v), rl = RL(v);
         const int o0 = pos - w0 + s_shift[k];
         if (al == 1 && rl == 1) {
-            uint8_t a = p.alt_pool[p.v_alt_off[v]];
-            if (p.v_gt[v] == 1) {
+            uint8_t a = ALT(v, 0);
+            if (GT(v) == 1) {
                 uint8_t r = ref[pos];
                 if (r >= 'a' && r <= 'z') r -= 32;
                 a = iupac_het(r, a);
@@ -144,7 +204,7 @@ encode_windows_kernel(const EncodeParams p) {
             if (rc) out[total - 1 - o0] = comp_base(a); else out[o0] = a;
         } else {
             for (int j = 0; j < al; ++j) {
-                const uint8_t a = p.alt_pool[p.v_alt_off[v] + j];
+                const uint8_t a = ALT(v, j);
                 if (rc) out[total - 1 - (o0 + j)] = comp_base(a); else out[o0 + j] = a;
             }
         }
@@ -167,8 +227,37 @@ int encode_windows(const uint8_t* genome, const int64_t* win_base, const int32_t
         EncodeParams p{genome, win_base + c0, w0 + c0, w1 + c0, var_lo + c0, var_hi + c0, flags + c0, v_pos, v_ref_len,
                        v_alt_off, v_alt_len, v_gt, alt_pool, out + (size_t)c0 * pitch, pitch, out_len + c0, err};
         dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n);
-        encode_windows_kernel<<<grid, 256, 0, s>>>(p);
+        encode_windows_kernel<false><<<grid, 256, 0, s>>>(p, EditParams{});
         VF_LAUNCH_OK("encode_windows_kernel launch");
+    }
+    return 0;
+}
+
+int encode_windows_edit(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
+                        const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
+                        const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
+                        const uint8_t* v_gt, const uint8_t* alt_pool, const int32_t* e_pos, const int32_t* e_ref_len,
+                        const int32_t* e_alt_off, const int32_t* e_alt_len, const uint8_t* e_alt_pool, int n_win,
+                        int max_window, uint8_t* out, int64_t pitch, int32_t* out_len, uint8_t* applied, int32_t* err,
+                        cudaStream_t s) {
+    VF_REQUIRE(n_win >= 0, "encode_windows_edit: n_win %d < 0", n_win);
+    if (n_win == 0) return 0;
+    VF_REQUIRE(max_window > 0 && pitch >= max_window, "encode_windows_edit: pitch %lld < max window %d",
+               (long long)pitch, max_window);
+    VF_REQUIRE(genome && win_base && w0 && w1 && var_lo && var_hi && flags && v_pos && v_ref_len && v_alt_off &&
+               v_alt_len && v_gt && alt_pool, "encode_windows_edit: a window or variant array is NULL");
+    VF_REQUIRE(e_pos && e_ref_len && e_alt_off && e_alt_len && e_alt_pool,
+               "encode_windows_edit: an extra-record array is NULL");
+    VF_REQUIRE(out && out_len && applied && err, "encode_windows_edit: out, out_len, applied and err are required");
+    constexpr int kMaxWinPerLaunch = 65535;              // blockIdx.y limit, as encode_windows
+    for (int c0 = 0; c0 < n_win; c0 += kMaxWinPerLaunch) {
+        const int n = n_win - c0 < kMaxWinPerLaunch ? n_win - c0 : kMaxWinPerLaunch;
+        EncodeParams p{genome, win_base + c0, w0 + c0, w1 + c0, var_lo + c0, var_hi + c0, flags + c0, v_pos, v_ref_len,
+                       v_alt_off, v_alt_len, v_gt, alt_pool, out + (size_t)c0 * pitch, pitch, out_len + c0, err};
+        EditParams e{e_pos + c0, e_ref_len + c0, e_alt_off + c0, e_alt_len + c0, e_alt_pool, applied + c0};
+        dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n);
+        encode_windows_kernel<true><<<grid, 256, 0, s>>>(p, e);
+        VF_LAUNCH_OK("encode_windows_kernel<edit> launch");
     }
     return 0;
 }

@@ -119,6 +119,46 @@ def _check_stage1(hot, genes, t, variants, sets, min_gene_len, names):
                                "variants/window)")
 
 
+def score_items(eng, items, runs, cre_pooled, gene_pooled, rows_budget, embeddings, counters):
+    """Items (pooled CRE rows, gene rows, tissues, labels), gene-major with each gene's run of runs[g] items led by its
+    baseline, through Engine.prepare_shared + run_pooled in slabs of at most rows_budget CRE rows (cohort.slab_ranges).
+    -> per gene (pred fp32 [runs[g], T], emb fp32 [runs[g], T, D], or without `embeddings` the baseline's [T, D] only),
+    device tensors.  counters["slabs"] counts the slabs."""
+    dev = gene_pooled.device
+    base = np.zeros(len(items), bool)                       # the baseline item of each gene leads its run
+    base[np.cumsum([0] + list(runs[:-1]))] = True
+    n_rows = np.asarray([len(x[2]) for x in items], np.int64)
+    preds, embs = [], []
+    for x0, x1 in cohort.slab_ranges([len(x[0]) for x in items], rows_budget):
+        counters["slabs"] += 1
+        sl = items[x0:x1]
+        used, local = np.unique(np.concatenate([x[1] for x in sl]), return_inverse=True)
+        splits = np.cumsum([len(x[1]) for x in sl])[:-1]
+        s = eng.prepare_shared([x[0] for x in sl], np.split(local, splits), len(used), [x[2] for x in sl],
+                               [torch.from_numpy(x[3]) for x in sl])
+        out = eng.run_pooled(s, cre_pooled, gene_pooled.index_select(0, torch.from_numpy(used).to(dev)))
+        preds.append(out["pred"])
+        if embeddings:
+            embs.append(out["emb"])
+        else:                                               # only the baselines' embeddings are returned
+            r0 = np.concatenate([[0], np.cumsum(n_rows[x0:x1])])
+            rows = [np.arange(r0[j], r0[j + 1]) for j in range(x1 - x0) if base[x0 + j]]
+            if rows:
+                embs.append(out["emb"].index_select(0, torch.from_numpy(np.concatenate(rows)).to(dev)))
+    P = torch.cat(preds)
+    E = torch.cat(embs)
+    out, r, e = [], 0, 0
+    for k, x in zip(runs, np.flatnonzero(base)):
+        Tg = int(n_rows[x])
+        if embeddings:
+            out.append((P[r:r + k * Tg].view(k, Tg), E[r:r + k * Tg].view(k, Tg, -1)))
+        else:
+            out.append((P[r:r + k * Tg].view(k, Tg), E[e:e + Tg]))
+            e += Tg
+        r += k * Tg
+    return out
+
+
 @torch.no_grad()
 def cre_knockout(hot, genes, knockouts=None, variants=None, embeddings=False, to_host=True, rows_budget=ism.ROWS_BUDGET,
                  pass_rows=None, timer=None, counters=None, min_gene_len=None, gene_names=None):
@@ -178,43 +218,15 @@ def cre_knockout(hot, genes, knockouts=None, variants=None, embeddings=False, to
             gene_pooled = ism._pool(eng, eng.gene_tok, ug.to(torch.int32))
             del uc, ug
         with phase("seq2gene"):
-            base = np.zeros(len(items), bool)               # the baseline item of each gene leads its run
-            base[np.cumsum([0] + [1 + len(sets[gi]) for gi in range(a, b - 1)])] = True
-            n_rows = np.asarray([len(x[2]) for x in items], np.int64)
-            preds, embs = [], []
-            for x0, x1 in cohort.slab_ranges([len(x[0]) for x in items], rows_budget):
-                c["slabs"] += 1
-                sl = items[x0:x1]
-                used, local = np.unique(np.concatenate([x[1] for x in sl]), return_inverse=True)
-                splits = np.cumsum([len(x[1]) for x in sl])[:-1]
-                s = eng.prepare_shared([x[0] for x in sl], np.split(local, splits), len(used), [x[2] for x in sl],
-                                       [torch.from_numpy(x[3]) for x in sl])
-                out = eng.run_pooled(s, cre_pooled, gene_pooled.index_select(0, torch.from_numpy(used).to(dev)))
-                preds.append(out["pred"])
+            blocks = score_items(eng, items, [1 + len(sets[gi]) for gi in range(a, b)], cre_pooled, gene_pooled,
+                                 rows_budget, embeddings, c)
+            for gi, (p, e) in zip(range(a, b), blocks):
+                pred[t_off[gi]:t_off[gi + 1]] = p[0]
+                ko_pred[gi] = p[1:]
+                emb[t_off[gi]:t_off[gi + 1]] = e[0] if embeddings else e
                 if embeddings:
-                    embs.append(out["emb"])
-                else:                                       # only the baselines' embeddings are returned
-                    r0 = np.concatenate([[0], np.cumsum(n_rows[x0:x1])])
-                    rows = [np.arange(r0[j], r0[j + 1]) for j in range(x1 - x0) if base[x0 + j]]
-                    if rows:
-                        embs.append(out["emb"].index_select(0, torch.from_numpy(np.concatenate(rows)).to(dev)))
-            P = torch.cat(preds)
-            E = torch.cat(embs) if embs else None
-            r = e = 0
-            for gi in range(a, b):
-                K, Tg = len(sets[gi]), int(T[gi])
-                blk = P[r:r + (1 + K) * Tg].view(1 + K, Tg)
-                pred[t_off[gi]:t_off[gi + 1]] = blk[0]
-                ko_pred[gi] = blk[1:]
-                if embeddings:
-                    eb = E[r:r + (1 + K) * Tg].view(1 + K, Tg, D)
-                    emb[t_off[gi]:t_off[gi + 1]] = eb[0]
-                    ko_emb[gi] = eb[1:]
-                else:
-                    emb[t_off[gi]:t_off[gi + 1]] = E[e:e + Tg]
-                    e += Tg
-                r += (1 + K) * Tg
-            del P, E, preds, embs, cre_pooled, gene_pooled
+                    ko_emb[gi] = e[1:]
+            del blocks, cre_pooled, gene_pooled
     out = (pred, emb, ko_pred) + ((ko_emb,) if embeddings else ())
     if to_host:
         host = lambda x: x.cpu().numpy()

@@ -468,6 +468,33 @@ def encode_windows(genome, win_base, w0, w1, var_lo, var_hi, flags, variants, ma
     return out, out_len, err
 
 
+def encode_windows_edit(genome, win_base, w0, w1, var_lo, var_hi, flags, variants, e_pos, e_ref_len, e_alt_off,
+                        e_alt_len, e_alt_pool, max_window, pitch, err=None):
+    """encode_windows with one extra hom-alt record per row (vf_encode_windows_edit): row w encodes as encode_windows
+    does on the table with {e_pos[w], e_ref_len[w], e_alt_pool[e_alt_off[w], + e_alt_len[w])} inserted after every
+    record of pos <= e_pos[w].  e_* int32 [n], e_alt_pool uint8 device tensors.
+    -> (out uint8 [n, pitch], out_len int32 [n], applied uint8 [n] (1: the row's extra record was applied), err)."""
+    n = w0.numel()
+    dev = genome.device
+    for t in (w0, w1, var_lo, var_hi, e_pos, e_ref_len, e_alt_off, e_alt_len):
+        assert t.dtype == torch.int32 and t.numel() == n and t.is_contiguous()
+    assert win_base.dtype == torch.int64 and flags.dtype == torch.uint8 and e_alt_pool.dtype == torch.uint8
+    out = torch.empty((n, pitch), dtype=torch.uint8, device=dev)
+    out_len = torch.empty(n, dtype=torch.int32, device=dev)
+    applied = torch.empty(n, dtype=torch.uint8, device=dev)
+    if err is None:
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+    v = variants
+    with _timed("stage1_encode_edit", nbytes=float(n) * max_window * 2):  # window bytes read + written (upper bound)
+        check(_lib.lib().vf_encode_windows_edit(ptr(genome), ptr(win_base), ptr(w0), ptr(w1), ptr(var_lo), ptr(var_hi),
+                                                ptr(flags), ptr(v["pos"]), ptr(v["ref_len"]), ptr(v["alt_off"]),
+                                                ptr(v["alt_len"]), ptr(v["gt"]), ptr(v["alt_pool"]), ptr(e_pos),
+                                                ptr(e_ref_len), ptr(e_alt_off), ptr(e_alt_len), ptr(e_alt_pool), n,
+                                                int(max_window), ptr(out), int(pitch), ptr(out_len), ptr(applied),
+                                                ptr(err), stream()))
+    return out, out_len, applied, err
+
+
 def _genotype_rows(w0, w1, var_lo, var_hi, flags, variants):
     n = w0.numel()
     for t in (w0, w1, var_lo, var_hi):

@@ -203,6 +203,15 @@ class HotPath:
         from .knockout import cre_knockout
         return cre_knockout(self, genes, knockouts, variants, embeddings=embeddings, to_host=to_host, **kw)
 
+    def deletion_scan(self, genes, deletions, variants: SampleVariants = None, embeddings=False, to_host=True, **kw):
+        """In-silico deletions (deletion.deletion_scan): deletions[i] = int64 [n, 2] 1-based inclusive spans [a, b] for
+        gene i, on the chromosomes kw["chroms"][i] (default: the gene's).  -> (pred [sum T], emb [sum T, D]) of the
+        baseline, bit-identical to predict(genes, variants), per gene the deletion predictions [n, T] (+ per gene
+        [n, T, D] embeddings when `embeddings`), each bit-identical to predict on the gene with the deletion's VCF record
+        added to the background, and per gene the applied flags dict(cre=bool [n, C] in batch order, gene=bool [n])."""
+        from .deletion import deletion_scan
+        return deletion_scan(self, genes, deletions, variants, embeddings=embeddings, to_host=to_host, **kw)
+
     @staticmethod
     def _raise_on_stage1_error(err):
         """The encode kernel flags windows it could not build (their tokens are then all padding): never hand out

@@ -271,6 +271,75 @@ class VCFProcessor:
                   for i, gid in enumerate(gene_ids)]
         return pd.concat(frames, ignore_index=True)
 
+    def deletion_scan(self, vcf_path: str, query_df: pd.DataFrame, deletions: pd.DataFrame = None):
+        """In-silico genomic deletions (DESIGN.md section 16): every query row predicted with a span of the genome
+        deleted, each window the deletion does not change encoded once.  A deletion [start, end] (1-based, inclusive)
+        gives what create_data + predict give on the sample's VCF with one more line: POS = start - 1, REF = the
+        reference bases start - 1 .. end, ALT = the anchor base, GT 1/1.  The query is filtered with VCFDataset's rules;
+        the sample is `vcf_path` or a per-row vcf_path column (empty or missing: the reference genome).
+        deletions: None = every CRE's own bases deleted singly, on its manifest chromosome ([start_cre + 1, end_cre]),
+        or a DataFrame with columns gene_id, chromosome, start, end and optionally label (deletion.tiles builds tilings).
+        Invalid spans raise a ValueError before the model is loaded.  Writes no file.
+        -> one row per (query row, deletion, tissue), in that order (default deletions in manifest order, user ones in
+        first-appearance order), columns deletion.FRAME_COLUMNS: deletion (label; the manifest row for the default
+        scan), chromosome, del_start, del_end, width, cre_windows_changed / gene_window_changed / changed (windows whose
+        bytes the deletion changed), the deleted CRE's manifest columns (default scan; null otherwise),
+        baseline_expression, predicted_expression and delta = predicted - baseline."""
+        from .. import deletion as dl
+        from ..pipeline import GeneSpec, HotPath
+        ds = self.model_config.dataset
+        dataset = VCFDataset(max_length=ds.max_length, max_chunks=ds.max_chunks, cre_neighbour_hood=ds.cre_neighbour_hood,
+                             gencode_v24=ds.gencode_v24, gene_cre_manifest=self.gene_cre_manifest,
+                             gene_upstream_neighbour_hood=ds.gene_upstream_neighbour_hood,
+                             gene_downstream_neighbour_hood=ds.gene_downstream_neighbour_hood, query_df=query_df,
+                             fasta_path=self.vcf_loader_config.fasta_path, vcf_path=vcf_path)
+        q = dataset.query_df
+        user = dl.user_deletions(deletions) if deletions is not None else None
+        genes, manifests, dels, paths = [], [], [], []
+        for _, row in q.iterrows():
+            gid = row["gene_id"]
+            info = dataset._get_gene_info(gid)
+            assert info["chromosome"] in ["chr" + str(i) for i in range(1, 23)], \
+                f"Chromosome {info['chromosome']} is not a valid chromosome. Sex chromosomes are not supported"
+            m, _ = dataset.cre_manifest(gid, info)
+            labels = np.asarray([dataset.ref_cre_to_idx[x] for x in m["cre_name"]], np.int64)
+            genes.append(GeneSpec(info["chromosome"], int(info["start"]), int(info["end"]), info["strand"],
+                                  m["start_cre"].to_numpy(np.int64), m["end_cre"].to_numpy(np.int64), labels,
+                                  list(row["tissues"]), cre_chrom=list(m["chromosome"])))
+            manifests.append(m)
+            if user is not None:
+                dels.append(user.get(gid, ([], np.zeros((0, 2), np.int64), [])))
+            else:
+                spans, chroms = dl.default_spans(m)
+                dels.append((list(range(len(m))), spans, chroms))
+            p = row["vcf_path"] if "vcf_path" in q.columns else vcf_path
+            paths.append(None if p is None or (not isinstance(p, str) and pd.isna(p)) or str(p) == "" else str(p))
+        if user is not None:
+            for gid in user:
+                if gid not in set(q["gene_id"]):
+                    print(f"Gene {gid} of the deletions is not in the query so skipping it")
+        gene_ids = list(q["gene_id"])
+        genome = dataset._genome()
+        dl.check_deletions(genes, [d[1] for d in dels], [d[2] for d in dels],
+                           {k: v[1] for k, v in genome.offsets.items()}, gene_ids)
+        model, _, _ = self.load_model()
+        hot = HotPath(model.engine(), genome, max_length=ds.max_length, max_chunks=ds.max_chunks,
+                      cre_neighbour_hood=ds.cre_neighbour_hood, gene_upstream=ds.gene_upstream_neighbour_hood,
+                      gene_downstream=ds.gene_downstream_neighbour_hood)
+        base, dpred, applied = [None] * len(genes), [None] * len(genes), [None] * len(genes)
+        for p in dict.fromkeys(paths):                       # one call per sample, in first-appearance order
+            rows = [i for i, x in enumerate(paths) if x == p]
+            pred, _, d_pred, app = hot.deletion_scan([genes[i] for i in rows], [dels[i][1] for i in rows],
+                                                     dataset._variants(p), chroms=[dels[i][2] for i in rows],
+                                                     min_gene_len=1000, gene_names=[gene_ids[i] for i in rows])
+            off = np.concatenate([[0], np.cumsum([len(genes[i].tissues) for i in rows])])
+            for k, i in enumerate(rows):
+                base[i], dpred[i], applied[i] = pred[off[k]:off[k + 1]], d_pred[k], app[k]
+        frames = [dl.deletion_frame(gid, list(q["tissue_names"].iloc[i]), dels[i][0], dels[i][1], dels[i][2],
+                                    applied[i], base[i], dpred[i], manifests[i] if user is None else None)
+                  for i, gid in enumerate(gene_ids)]
+        return pd.concat(frames, ignore_index=True)
+
     def format_output(self, df, predictions):
         pred_exp, embd = [], []
         for p in predictions:
