@@ -200,7 +200,8 @@ int vf_forest_predict(const float* x, int ldx, int n_rows, int d, const int32_t*
  * variants var_lo[w]..var_hi[w] (sorted by position; gt 0 skip / 1 het / 2 hom-alt): het SNP -> IUPAC code,
  * hom SNP -> ALT, indel/MNP -> REF span replaced by ALT, overlapping or window-straddling records skipped;
  * flags bit0 = reverse-complement the result, bit1 = SNP-only filter.
- * out: uint8 [n_win, pitch]; out_len int32 [n_win]; err: device int32 flag (1 pitch overflow, 2 >2048 records).
+ * out: uint8 [n_win, pitch]; out_len int32 [n_win]; err: device int32 flag (1 pitch overflow, 2 >2048 records;
+ * vf_encode_windows_edits also 4: a row's extra records are not sorted by pos).
  * Any n_win: batches of more than 65535 windows are launched in chunks of 65535.
  * Replaces the `samtools faidx | bcftools consensus -H I -e 'ALT~"<.*>"'` subprocess pair per window
  * (utils/data_process.py:17-101, :367-467) and utils/functions.py:129-172 (reverse_complement).
@@ -226,6 +227,24 @@ int vf_encode_windows_edit(const uint8_t* genome, const int64_t* win_base, const
                            const int32_t* e_alt_off, const int32_t* e_alt_len, const uint8_t* e_alt_pool, int n_win,
                            int max_window, uint8_t* out, int64_t pitch, int32_t* out_len, uint8_t* applied,
                            int32_t* err, void* stream);
+/*
+ * vf_encode_windows with a LIST of extra records per row (variant sets: haplotypes, pairs, edits against a sample
+ * background), in CSR form: row w owns the records [e_off[w], e_off[w + 1]) (e_off int32 [n_win + 1], nondecreasing,
+ * ranges disjoint), each {pos e_pos, ref_len e_ref_len, ALT e_alt_pool[e_alt_off, + e_alt_len), gt e_gt (0 skip, 1 het,
+ * 2 hom-alt)}, sorted by pos within the row.  Row w is encoded as vf_encode_windows encodes it on the table with each of
+ * its records inserted right after every background record with pos <= its own (records of one pos in list order), bit
+ * for bit, in the same kernel body.  Extras count toward the 2048-record cap.  applied uint8 [e_off[n_win]] = 1 iff that
+ * extra record was applied.  A row whose records are not sorted by pos sets *err to 4 and writes length 0.
+ * vf_encode_windows_edit is the one-record case: row w's list is record w, gt 2.  Other arguments, outputs and errors
+ * as vf_encode_windows; n_win < 0 or a NULL array fails before any launch.
+ */
+int vf_encode_windows_edits(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
+                            const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
+                            const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
+                            const uint8_t* v_gt, const uint8_t* alt_pool, const int32_t* e_off, const int32_t* e_pos,
+                            const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
+                            const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_win, int max_window, uint8_t* out,
+                            int64_t pitch, int32_t* out_len, uint8_t* applied, int32_t* err, void* stream);
 /*
  * Which rows of a cohort encode to the same bytes.  Row r = one (window, sample): w0/w1/flags/var_lo/var_hi as in
  * vf_encode_windows (flags bit1 = SNP-only), the variant arrays those of vf_encode_windows (one concatenated table may

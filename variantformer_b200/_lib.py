@@ -49,6 +49,7 @@ SIGNATURES = {
     "vf_forest_predict": ([_vp, _i32, _i32, _i32] + [_vp] * 9 + [_i32, _vp, _vp], _i32),
     "vf_encode_windows": ([_vp] * 13 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
     "vf_encode_windows_edit": ([_vp] * 18 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp, _vp], _i32),
+    "vf_encode_windows_edits": ([_vp] * 20 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp, _vp], _i32),
     "vf_window_genotype_keys": ([_vp] * 11 + [_i32, _vp, _vp, _vp, _vp, _vp], _i32),
     "vf_window_genotype_equal": ([_vp] * 11 + [_i32, _vp, _vp, _vp], _i32),
     "vf_mutate_windows": ([_vp, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp], _i32),

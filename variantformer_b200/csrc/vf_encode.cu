@@ -69,33 +69,42 @@ struct AppliedScan {
     }
 };
 
-// vf_encode_windows_edit: one extra hom-alt record per row, merged into the row's candidates.  It is walked right after
-// every candidate whose pos is <= its own (a VCF line placed after the records of its position) and judged by
-// AppliedScan's own rule, so a row encodes exactly as vf_encode_windows does on the table with the record inserted.
-// next() returns kExtra for it.
-constexpr int kExtra = 0x7FFFFFFF;
+// vf_encode_windows_edits / vf_encode_windows_edit: a list of extra records per row, merged into the row's candidates
+// by a two-pointer walk.  A background candidate is walked first when its pos is <= the next extra's (a VCF line placed
+// after the records of its position); every record, background or extra, is judged by AppliedScan's own rule, so a row
+// encodes exactly as vf_encode_windows does on the table with the records inserted.  next() returns extra k as the
+// tagged index extra_tag(k) (< -1; -1 ends the walk).  Extras with gt 0 are skipped like background records.
+__device__ __forceinline__ int extra_tag(int k) { return -2 - k; }
+
+struct EditParams {                   // the extra records (unused by the plain kernel)
+    const int32_t* off;               // [n_win + 1] row w owns extras [off[w], off[w + 1]); NULL: row w owns extra w
+    const int32_t* pos; const int32_t* ref_len; const int32_t* alt_off; const int32_t* alt_len;
+    const uint8_t* gt;                // NULL: every extra is hom-alt (gt 2)
+    const uint8_t* alt_pool;
+    uint8_t* applied;                 // one flag per extra: 1 = applied
+};
 
 struct MergedScan {
     AppliedScan sc;
-    int hi, x_pos, x_rl, x_al;
-    bool pending;
-    __device__ __forceinline__ MergedScan(int lo, int hi_, int w0, int w1, bool snp, int xp, int xr, int xa,
-                                          const int32_t* v_pos)
-        : sc(lo, hi_, w0, w1, snp), hi(hi_), x_pos(xp), x_rl(xr), x_al(xa), pending(true) {
-        int a = lo, b = hi_;                               // the candidates are sorted by pos: first one past x_pos
-        while (a < b) { const int m = (a + b) >> 1; if (v_pos[m] <= xp) a = m + 1; else b = m; }
-        sc.hi = a;
-    }
+    const EditParams& e;
+    int x, xe, x_pos;                 // extras [x, xe) still to walk; x_pos = the pos of extra x
+    __device__ __forceinline__ MergedScan(int lo, int hi, int w0, int w1, bool snp, const EditParams& e_, int x0, int x1)
+        : sc(lo, hi, w0, w1, snp), e(e_), x(x0), xe(x1), x_pos(x0 < x1 ? e_.pos[x0] : 0) {}
     __device__ __forceinline__ int next(const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_len,
                                         const uint8_t* v_gt) {
-        if (pending) {
-            const int i = sc.next(v_pos, v_ref_len, v_alt_len, v_gt);
-            if (i >= 0) return i;
-            pending = false;
-            sc.hi = hi;
-            if (sc.take(x_pos, x_rl, x_al)) return kExtra;
+        for (;;) {
+            if (sc.i < sc.hi && (x == xe || v_pos[sc.i] <= x_pos)) {
+                const int i = sc.i++;
+                if (v_gt[i] != 0 && sc.take(v_pos[i], v_ref_len[i], v_alt_len[i])) return i;
+            } else if (x < xe) {
+                const int k = x++;
+                const int p = x_pos;
+                if (x < xe) x_pos = e.pos[x];
+                if ((e.gt == nullptr || e.gt[k] != 0) && sc.take(p, e.ref_len[k], e.alt_len[k])) return extra_tag(k);
+            } else {
+                return -1;
+            }
         }
-        return sc.next(v_pos, v_ref_len, v_alt_len, v_gt);
     }
 };
 
@@ -110,17 +119,11 @@ struct EncodeParams {
     const uint8_t* alt_pool;
     uint8_t* out; int64_t pitch;      // [n_win, pitch]
     int32_t* out_len;                 // [n_win]
-    int32_t* err;                     // device error flag (1 = pitch overflow, 2 = too many variants)
+    int32_t* err;                     // device error flag (1 = pitch overflow, 2 = too many variants, 4 = unsorted extras)
 };
 
-struct EditParams {                   // vf_encode_windows_edit: the extra record of every row (unused by the plain kernel)
-    const int32_t* pos; const int32_t* ref_len; const int32_t* alt_off; const int32_t* alt_len;   // [n_win]
-    const uint8_t* alt_pool;
-    uint8_t* applied;                 // [n_win] 1 = the row's extra record was applied
-};
-
-// kEdit = false: vf_encode_windows.  kEdit = true: the same body over MergedScan; record index kExtra reads the row's
-// extra record (hom-alt) wherever the plain kernel reads the table.
+// kEdit = false: vf_encode_windows.  kEdit = true: the same body over MergedScan; a tagged index (< -1) reads its extra
+// record wherever the plain kernel reads the table.
 template <bool kEdit>
 __global__ void __launch_bounds__(256)
 encode_windows_kernel(const EncodeParams p, const EditParams e) {
@@ -133,41 +136,52 @@ encode_windows_kernel(const EncodeParams p, const EditParams e) {
     if (slice0 >= w1 && !(blockIdx.x == 0)) return;
     const uint8_t fl = p.flags[w];
     const bool rc = fl & 1, snp_only = fl & 2;
-    int x_pos = 0, x_rl = 0, x_al = 0;
-    if constexpr (kEdit) { x_pos = e.pos[w]; x_rl = e.ref_len[w]; x_al = e.alt_len[w]; }
-    const auto POS = [&](int v) { return kEdit && v == kExtra ? x_pos : p.v_pos[v]; };
-    const auto RL = [&](int v) { return kEdit && v == kExtra ? x_rl : p.v_ref_len[v]; };
-    const auto AL = [&](int v) { return kEdit && v == kExtra ? x_al : p.v_alt_len[v]; };
-    const auto ALT = [&](int v, int j) { return kEdit && v == kExtra ? e.alt_pool[e.alt_off[w] + j] : p.alt_pool[p.v_alt_off[v] + j]; };
-    const auto GT = [&](int v) { return kEdit && v == kExtra ? (uint8_t)2 : p.v_gt[v]; };
+    const auto X = [](int v) { return -2 - v; };            // tagged index -> extra record
+    const auto POS = [&](int v) { return kEdit && v < 0 ? e.pos[X(v)] : p.v_pos[v]; };
+    const auto RL = [&](int v) { return kEdit && v < 0 ? e.ref_len[X(v)] : p.v_ref_len[v]; };
+    const auto AL = [&](int v) { return kEdit && v < 0 ? e.alt_len[X(v)] : p.v_alt_len[v]; };
+    const auto ALT = [&](int v, int j) { return kEdit && v < 0 ? e.alt_pool[e.alt_off[X(v)] + j] : p.alt_pool[p.v_alt_off[v] + j]; };
+    const auto GT = [&](int v) { return kEdit && v < 0 ? (e.gt ? e.gt[X(v)] : (uint8_t)2) : p.v_gt[v]; };
     if (threadIdx.x == 0) {
         // sequential scan: which records are applied (overlap rule needs order) and where they land
         int n = 0, shift = 0, bad = 0;
-        bool took = false;
         auto scan = [&](auto& sc) {
-            for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)) >= 0;) {
+            for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)), kEdit ? i != -1 : i >= 0;) {
                 if (n == kMaxApplied) { bad = 2; break; }
-                if (kEdit && i == kExtra) took = true;
+                if constexpr (kEdit) { if (i < 0 && blockIdx.x == 0) e.applied[X(i)] = 1; }
                 s_vidx[n] = i; s_shift[n] = shift; ++n;
                 shift += AL(i) - RL(i);
             }
         };
         if constexpr (kEdit) {
-            MergedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only, x_pos, x_rl, x_al, p.v_pos);
-            scan(sc);
+            const int x0 = e.off ? e.off[w] : w, x1 = e.off ? e.off[w + 1] : w + 1;
+            if (blockIdx.x == 0)
+                for (int k = x0; k < x1; ++k) e.applied[k] = 0;
+            for (int k = x0 + 1; k < x1; ++k)
+                if (e.pos[k] < e.pos[k - 1]) bad = 4;
+            if (bad) {                                       // an unsorted row is not merged: it writes nothing
+                atomicMax(p.err, bad);
+                if (blockIdx.x == 0) p.out_len[w] = 0;
+                s_n = -1;
+            } else {
+                MergedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only, e, x0, x1);
+                scan(sc);
+            }
         } else {
             AppliedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only);
             scan(sc);
         }
-        s_n = n; s_total = (w1 - w0) + shift;
-        if (bad) atomicMax(p.err, bad);
-        if (s_total > p.pitch) atomicMax(p.err, 1);
-        // an overflowing window writes nothing: report length 0 (plus err = 1) so the tokenizer never reads past the row
-        if (blockIdx.x == 0) p.out_len[w] = s_total > p.pitch ? 0 : s_total;
-        if constexpr (kEdit) { if (blockIdx.x == 0) e.applied[w] = took; }
+        if (!(kEdit && bad == 4)) {
+            s_n = n; s_total = (w1 - w0) + shift;
+            if (bad) atomicMax(p.err, bad);
+            if (s_total > p.pitch) atomicMax(p.err, 1);
+            // an overflowing window writes nothing: report length 0 (plus err = 1) so the tokenizer never reads past the row
+            if (blockIdx.x == 0) p.out_len[w] = s_total > p.pitch ? 0 : s_total;
+        }
     }
     __syncthreads();
     const int n = s_n, total = s_total;
+    if (kEdit && n < 0) return;
     if (total > p.pitch) return;
     const uint8_t* ref = p.genome + p.win_base[w];
     uint8_t* out = p.out + (size_t)w * p.pitch;
@@ -233,6 +247,35 @@ int encode_windows(const uint8_t* genome, const int64_t* win_base, const int32_t
     return 0;
 }
 
+static int encode_windows_extras(const char* what, const uint8_t* genome, const int64_t* win_base, const int32_t* w0,
+                                 const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags,
+                                 const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_off,
+                                 const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, const EditParams& e,
+                                 int n_win, int max_window, uint8_t* out, int64_t pitch, int32_t* out_len, int32_t* err,
+                                 cudaStream_t s) {
+    VF_REQUIRE(n_win >= 0, "%s: n_win %d < 0", what, n_win);
+    if (n_win == 0) return 0;
+    VF_REQUIRE(max_window > 0 && pitch >= max_window, "%s: pitch %lld < max window %d", what, (long long)pitch,
+               max_window);
+    VF_REQUIRE(genome && win_base && w0 && w1 && var_lo && var_hi && flags && v_pos && v_ref_len && v_alt_off &&
+               v_alt_len && v_gt && alt_pool, "%s: a window or variant array is NULL", what);
+    VF_REQUIRE(e.pos && e.ref_len && e.alt_off && e.alt_len && e.alt_pool, "%s: an extra-record array is NULL", what);
+    VF_REQUIRE(out && out_len && e.applied && err, "%s: out, out_len, applied and err are required", what);
+    constexpr int kMaxWinPerLaunch = 65535;              // blockIdx.y limit, as encode_windows
+    for (int c0 = 0; c0 < n_win; c0 += kMaxWinPerLaunch) {
+        const int n = n_win - c0 < kMaxWinPerLaunch ? n_win - c0 : kMaxWinPerLaunch;
+        EncodeParams p{genome, win_base + c0, w0 + c0, w1 + c0, var_lo + c0, var_hi + c0, flags + c0, v_pos, v_ref_len,
+                       v_alt_off, v_alt_len, v_gt, alt_pool, out + (size_t)c0 * pitch, pitch, out_len + c0, err};
+        EditParams ec = e;                               // CSR offsets are global: only the one-record form moves
+        if (e.off) ec.off = e.off + c0;
+        else { ec.pos += c0; ec.ref_len += c0; ec.alt_off += c0; ec.alt_len += c0; ec.applied += c0; }
+        dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n);
+        encode_windows_kernel<true><<<grid, 256, 0, s>>>(p, ec);
+        VF_LAUNCH_OK("encode_windows_kernel<edit> launch");
+    }
+    return 0;
+}
+
 int encode_windows_edit(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
                         const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
                         const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
@@ -240,26 +283,24 @@ int encode_windows_edit(const uint8_t* genome, const int64_t* win_base, const in
                         const int32_t* e_alt_off, const int32_t* e_alt_len, const uint8_t* e_alt_pool, int n_win,
                         int max_window, uint8_t* out, int64_t pitch, int32_t* out_len, uint8_t* applied, int32_t* err,
                         cudaStream_t s) {
-    VF_REQUIRE(n_win >= 0, "encode_windows_edit: n_win %d < 0", n_win);
-    if (n_win == 0) return 0;
-    VF_REQUIRE(max_window > 0 && pitch >= max_window, "encode_windows_edit: pitch %lld < max window %d",
-               (long long)pitch, max_window);
-    VF_REQUIRE(genome && win_base && w0 && w1 && var_lo && var_hi && flags && v_pos && v_ref_len && v_alt_off &&
-               v_alt_len && v_gt && alt_pool, "encode_windows_edit: a window or variant array is NULL");
-    VF_REQUIRE(e_pos && e_ref_len && e_alt_off && e_alt_len && e_alt_pool,
-               "encode_windows_edit: an extra-record array is NULL");
-    VF_REQUIRE(out && out_len && applied && err, "encode_windows_edit: out, out_len, applied and err are required");
-    constexpr int kMaxWinPerLaunch = 65535;              // blockIdx.y limit, as encode_windows
-    for (int c0 = 0; c0 < n_win; c0 += kMaxWinPerLaunch) {
-        const int n = n_win - c0 < kMaxWinPerLaunch ? n_win - c0 : kMaxWinPerLaunch;
-        EncodeParams p{genome, win_base + c0, w0 + c0, w1 + c0, var_lo + c0, var_hi + c0, flags + c0, v_pos, v_ref_len,
-                       v_alt_off, v_alt_len, v_gt, alt_pool, out + (size_t)c0 * pitch, pitch, out_len + c0, err};
-        EditParams e{e_pos + c0, e_ref_len + c0, e_alt_off + c0, e_alt_len + c0, e_alt_pool, applied + c0};
-        dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n);
-        encode_windows_kernel<true><<<grid, 256, 0, s>>>(p, e);
-        VF_LAUNCH_OK("encode_windows_kernel<edit> launch");
-    }
-    return 0;
+    const EditParams e{nullptr, e_pos, e_ref_len, e_alt_off, e_alt_len, nullptr, e_alt_pool, applied};
+    return encode_windows_extras("encode_windows_edit", genome, win_base, w0, w1, var_lo, var_hi, flags, v_pos,
+                                 v_ref_len, v_alt_off, v_alt_len, v_gt, alt_pool, e, n_win, max_window, out, pitch,
+                                 out_len, err, s);
+}
+
+int encode_windows_edits(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
+                         const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
+                         const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
+                         const uint8_t* v_gt, const uint8_t* alt_pool, const int32_t* e_off, const int32_t* e_pos,
+                         const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
+                         const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_win, int max_window, uint8_t* out,
+                         int64_t pitch, int32_t* out_len, uint8_t* applied, int32_t* err, cudaStream_t s) {
+    VF_REQUIRE(n_win <= 0 || (e_off && e_gt), "encode_windows_edits: an extra-record array is NULL");
+    const EditParams e{e_off, e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool, applied};
+    return encode_windows_extras("encode_windows_edits", genome, win_base, w0, w1, var_lo, var_hi, flags, v_pos,
+                                 v_ref_len, v_alt_off, v_alt_len, v_gt, alt_pool, e, n_win, max_window, out, pitch,
+                                 out_len, err, s);
 }
 
 // ---------------------------------------------------------------------------------

@@ -21,19 +21,16 @@ What is not recomputed:
     + one per deletion, per gene) run through Engine.prepare_shared + run_pooled in slabs of at most ism.ROWS_BUDGET CRE
     rows and passes of about PASS_ROWS token rows (knockout.score_items, cohort.plan_passes).  Results depend on
     neither split.
+The planning is variant_sets.plan's: a deletion is its one-record set.
 """
-import contextlib
-
 import numpy as np
 import pandas as pd
 import torch
 
-from . import cohort, ism, knockout, ops
-from .stage1 import FLAG_REVCOMP, cre_window, gene_window
+from . import ism, knockout, ops, variant_sets
+from .stage1 import cre_window, gene_window
 
-PASS_ROWS = cohort.PASS_ROWS
-# edited CRE windows per encode + BPE call (bounds the rows' buffers; results do not depend on the split)
-CRE_EDIT_ROWS = 16384
+PASS_ROWS = variant_sets.PASS_ROWS
 
 
 def record(spans):
@@ -118,9 +115,10 @@ def _encode_edits(hot, variants, rows, pitch):
                                    max(r[2] - r[1] for r in rows), pitch)
 
 
-def _raise(code, name):
-    raise RuntimeError(f"stage-1 kernel reported error {code} for a deletion of gene {name} (1: pitch overflow, "
-                       "2: >2048 variants/window)")
+def _encode_rows(hot, variants, rows, pitch):
+    """The planner's rows [(chrom, w0, w1, flags, (record,))] of one-record sets, through _encode_edits."""
+    return _encode_edits(hot, variants, [(ch, w0, w1, fl, r[0][1], r[0][2], r[0][3][0]) for ch, w0, w1, fl, r in rows],
+                         pitch)
 
 
 @torch.no_grad()
@@ -136,171 +134,25 @@ def deletion_scan(hot, genes, deletions, variants=None, chroms=None, embeddings=
     background.  applied: the windows whose bytes the deletion changed.  timer: optional callable(phase) -> context
     manager around the "stage1", "seq2reg" and "seq2gene" phases; counters: optional dict filled with item / window
     counts; min_gene_len: VCFDataset's gene-window length rule, a ValueError for any item, baseline or deletion, whose
-    encoded gene window is not longer (gene_names name the genes)."""
+    encoded gene window is not longer (gene_names name the genes).
+    A deletion is the one-record set of variant_sets' planner: its record (record()) with the anchor base as ALT."""
     names = gene_names if gene_names is not None else [f"{g.chrom}:{g.start}-{g.end}" for g in genes]
     dels = check_deletions(genes, deletions, chroms, {k: v[1] for k, v in hot.genome.offsets.items()}, names)
-    eng, dev = hot.engine, hot.engine.device
-    phase = timer or (lambda name: contextlib.nullcontext())
-    pass_rows = PASS_ROWS if pass_rows is None else pass_rows
-    L, CW = hot.max_length, hot.max_chunks
-    hits = [gene_hits(g, s, c, hot.nb, hot.up, hot.down) for g, (s, c) in zip(genes, dels)]
-    T = np.asarray([len(g.tissues) for g in genes], np.int64)
-    t_off = np.concatenate([[0], np.cumsum(T)])
-    pred = torch.empty(int(t_off[-1]), dtype=torch.float32, device=dev)
-    emb = torch.empty((int(t_off[-1]), eng.w.D), dtype=torch.float32, device=dev)
-    del_pred, del_emb = [None] * len(genes), [None] * len(genes)
-    applied = [dict(cre=np.zeros_like(h[0]), gene=np.zeros_like(h[1])) for h in hits]
+    dev = hot.engine.device
+    sets = []
+    for s, ch in dels:
+        pos, rl = record(s)
+        idx = [hot.genome.offsets[x][0] + int(p) for x, p in zip(ch, pos)]
+        anc = (hot.genome.seq[torch.as_tensor(idx, dtype=torch.long, device=dev)].cpu().numpy() if idx
+               else np.zeros(0, np.uint8))
+        sets.append([((x, int(p), int(r), bytes([int(y)]), 2),) for x, p, r, y in zip(ch, pos, rl, anc)])
     c = counters if counters is not None else {}
-    c.update(genes=len(genes), deletions=sum(len(s) for s, _ in dels), changed=0, items=0, windows_encoded=0,
-             windows_per_item=0, cre_windows_edited=0, gene_windows_edited=0, cre_token_rows=0, gene_token_rows=0,
-             passes=0, slabs=0)
-
-    def short(n, i):
-        return ValueError(f"Mutated sequence is less than {min_gene_len}bp for gene {names[i]}") if \
-            min_gene_len is not None and n <= min_gene_len else None
-
-    rows_per_gene = [len(g.cre_start) + CW + int(h[0].sum()) + CW * int(h[1].sum()) for g, h in zip(genes, hits)]
-    for a, b, _, _ in cohort.plan_passes(rows_per_gene, pass_rows):
-        c["passes"] += 1
-        with phase("stage1"):
-            # ---- the baseline items: each gene tokenized once ----
-            ctoks, gtoks, labels, clens, glens = [], [], [], [], []
-            for k0 in range(a, b, ism.GENE_GROUP):
-                k1 = min(b, k0 + ism.GENE_GROUP)
-                t = hot.tokenize(genes[k0:k1], variants)
-                knockout._check_stage1(hot, genes[k0:k1], t, variants, [[]] * (k1 - k0), None, names[k0:k1])
-                cl = t["cre_seq"][1].cpu().numpy().astype(np.int64)
-                glens += t["gene_seq"][1].cpu().numpy().astype(np.int64).tolist()
-                for g in genes[k0:k1]:
-                    clens.append(cl[:len(g.cre_start)]); cl = cl[len(g.cre_start):]
-                ctoks += t["cre_tok"]; gtoks += t["gene_tok"]; labels += t["labels"]
-                del t
-            for i, gi in enumerate(range(a, b)):
-                if (e := short(glens[i], gi)) is not None:
-                    raise e
-            # ---- edited windows: rows (chrom, w0, w1, flags, pos, ref_len, anchor) of every (deletion, contained window)
-            anchors = []
-            for gi in range(a, b):
-                s, ch = dels[gi]
-                pos, _ = record(s)
-                idx = [hot.genome.offsets[x][0] + int(p) for x, p in zip(ch, pos)]
-                anchors.append(hot.genome.seq[torch.as_tensor(idx, dtype=torch.long, device=dev)].cpu().numpy()
-                               if idx else np.zeros(0, np.uint8))
-            c_rows, c_owner, g_rows, g_owner = [], [], [], []
-            for gi, anc in zip(range(a, b), anchors):
-                g, (s, ch), (hc, hg) = genes[gi], dels[gi], hits[gi]
-                pos, rl = record(s)
-                fl = FLAG_REVCOMP if g.strand == "-" else 0
-                order = knockout.batch_order(g)
-                for j, k in zip(*np.nonzero(hc)):
-                    r = order[k]
-                    w0, w1 = cre_window(g.cre_start[r], g.cre_end[r], hot.nb)
-                    c_rows.append((ch[j], w0, w1, fl, int(pos[j]), int(rl[j]), int(anc[j]))); c_owner.append((gi, j, k))
-                g0, g1 = gene_window(g.start, g.end, g.strand, hot.up, hot.down)
-                for j in np.flatnonzero(hg):
-                    g_rows.append((g.chrom, g0, g1, fl, int(pos[j]), int(rl[j]), int(anc[j]))); g_owner.append((gi, j))
-            # CRE windows: the per-item path's pitch is its gene's longest CRE span + 4096 (WindowTokenizer.sequences)
-            c_pitch = {gi: knockout._pitch(max(w1 - w0 for w0, w1 in (cre_window(s_, e_, hot.nb) for s_, e_ in
-                                                                      zip(genes[gi].cre_start, genes[gi].cre_end))))
-                       for gi in range(a, b)}
-            cand_c, c_len, c_app = [torch.cat(ctoks)], [], []
-            for r0 in range(0, len(c_rows), CRE_EDIT_ROWS):
-                rows = c_rows[r0:r0 + CRE_EDIT_ROWS]
-                pitch = max(c_pitch[o[0]] for o in c_owner[r0:r0 + CRE_EDIT_ROWS])
-                seq, lens, app, err = _encode_edits(hot, variants, rows, pitch)
-                if int(err.item()):
-                    _raise(int(err.item()), names[c_owner[r0][0]])
-                tok, _, _ = hot.tok.tokenize_fixed(seq, lens, seq.shape[1], typical_len=max(r[2] - r[1] for r in rows))
-                cand_c.append(tok.to(cand_c[0].dtype))
-                c_len.append(lens.cpu().numpy().astype(np.int64)); c_app.append(app.cpu().numpy().astype(bool))
-                del seq, tok
-            c_len = np.concatenate(c_len) if c_len else np.zeros(0, np.int64)
-            c_app = np.concatenate(c_app) if c_app else np.zeros(0, bool)
-            # gene windows: full BPE, 200-token chunks
-            cand_g, g_chunks, g_len, g_app = [torch.cat(gtoks)], [], [], []
-            cap = L * CW
-            for r0 in range(0, len(g_rows), ism.GENE_GROUP):
-                rows = g_rows[r0:r0 + ism.GENE_GROUP]
-                pitch = knockout._pitch(max(r[2] - r[1] for r in rows))
-                seq, lens, app, err = _encode_edits(hot, variants, rows, pitch)
-                if int(err.item()):
-                    _raise(int(err.item()), names[g_owner[r0][0]])
-                tok, cnt = ops.bpe_tokenize(seq, lens, seq.shape[1], hot.tok.merges, cap, cap)
-                del seq
-                G_m = np.minimum(CW, (cnt.cpu().numpy().astype(np.int64) + L - 1) // L)
-                tok = tok.view(len(rows), CW, L)
-                for j in range(len(rows)):
-                    cand_g.append(tok[j, :G_m[j]])
-                g_chunks += G_m.tolist()
-                g_len.append(lens.cpu().numpy().astype(np.int64)); g_app.append(app.cpu().numpy().astype(bool))
-                del tok
-            g_len = np.concatenate(g_len) if g_len else np.zeros(0, np.int64)
-            g_app = np.concatenate(g_app) if g_app else np.zeros(0, bool)
-            # errors the per-item path raises for a deletion item (the gene alone with the record added)
-            for (gi, j, k), n in zip(c_owner, c_len):
-                if n > c_pitch[gi]:
-                    _raise(1, names[gi])
-            for (gi, j), n in zip(g_owner, g_len):
-                g0, g1 = gene_window(genes[gi].start, genes[gi].end, genes[gi].strand, hot.up, hot.down)
-                if n > knockout._pitch(g1 - g0):
-                    _raise(1, names[gi])
-                if (e := short(n, gi)) is not None:
-                    raise e
-            # ---- every distinct token row once ----
-            uc, inv_c = torch.unique(torch.cat(cand_c), dim=0, return_inverse=True)
-            ug, inv_g = torch.unique(torch.cat(cand_g), dim=0, return_inverse=True)
-            del cand_c, cand_g
-            inv_c = inv_c.cpu().numpy().astype(np.int64); inv_g = inv_g.cpu().numpy().astype(np.int64)
-            n_cb = sum(x.shape[0] for x in ctoks); n_gb = sum(x.shape[0] for x in gtoks)
-            edit_c = {o: inv_c[n_cb + r] for r, o in enumerate(c_owner)}
-            g_start = n_gb + np.concatenate([[0], np.cumsum(g_chunks)]).astype(np.int64)
-            edit_g = {o: inv_g[g_start[r]:g_start[r + 1]] for r, o in enumerate(g_owner)}
-            for (gi, j, k), ap in zip(c_owner, c_app):
-                applied[gi]["cre"][j, k] = ap
-            for (gi, j), ap in zip(g_owner, g_app):
-                applied[gi]["gene"][j] = ap
-            # ---- items: per gene its baseline, then one per deletion ----
-            items = []
-            c0 = g0_ = 0
-            for i, gi in enumerate(range(a, b)):
-                C, G = ctoks[i].shape[0], gtoks[i].shape[0]
-                cr, gr, lab = inv_c[c0:c0 + C], inv_g[g0_:g0_ + G], labels[i].numpy().astype(np.int64)
-                c0 += C; g0_ += G
-                tis = torch.as_tensor(genes[gi].tissues, dtype=torch.long)
-                items.append((cr, gr, tis, lab))
-                hc, hg = hits[gi]
-                for j in range(len(dels[gi][0])):
-                    r = cr.copy()
-                    for k in np.flatnonzero(hc[j]):
-                        r[k] = edit_c[(gi, j, k)]
-                    items.append((r, edit_g[(gi, j)] if hg[j] else gr, tis, lab))
-                n_del = len(dels[gi][0])
-                c["windows_per_item"] += (1 + n_del) * (C + 1)
-                c["changed"] += int((applied[gi]["cre"].any(1) | applied[gi]["gene"]).sum())
-            del ctoks, gtoks
-            c["items"] += len(items)
-            c["cre_windows_edited"] += len(c_rows); c["gene_windows_edited"] += len(g_rows)
-            c["windows_encoded"] += sum(len(genes[gi].cre_start) + 1 for gi in range(a, b)) + len(c_rows) + len(g_rows)
-            c["cre_token_rows"] += int(uc.shape[0]); c["gene_token_rows"] += int(ug.shape[0])
-        with phase("seq2reg"):
-            cre_pooled = ism._pool(eng, eng.cre_tok, uc.to(torch.int32))
-            gene_pooled = ism._pool(eng, eng.gene_tok, ug.to(torch.int32))
-            del uc, ug
-        with phase("seq2gene"):
-            blocks = knockout.score_items(eng, items, [1 + len(dels[gi][0]) for gi in range(a, b)], cre_pooled,
-                                          gene_pooled, rows_budget, embeddings, c)
-            for gi, (p, e) in zip(range(a, b), blocks):
-                pred[t_off[gi]:t_off[gi + 1]] = p[0]
-                del_pred[gi] = p[1:]
-                emb[t_off[gi]:t_off[gi + 1]] = e[0] if embeddings else e
-                if embeddings:
-                    del_emb[gi] = e[1:]
-            del blocks, cre_pooled, gene_pooled
-    out = (pred, emb, del_pred) + ((del_emb,) if embeddings else ())
-    if to_host:
-        host = lambda x: x.cpu().numpy()
-        out = (host(pred), host(emb), [host(x) for x in del_pred]) + (([host(x) for x in del_emb],) if embeddings else ())
-    return out + (applied,)
+    out = variant_sets.plan(hot, genes, sets, variants, embeddings, to_host, rows_budget, pass_rows, timer, c,
+                            min_gene_len, names, encode=_encode_rows)
+    c["deletions"] = c.pop("sets")
+    for ap in out[-1]:
+        del ap["records"]
+    return out
 
 
 def tiles(chrom, start, end, width, step):

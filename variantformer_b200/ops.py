@@ -495,6 +495,46 @@ def encode_windows_edit(genome, win_base, w0, w1, var_lo, var_hi, flags, variant
     return out, out_len, applied, err
 
 
+def encode_windows_edits(genome, win_base, w0, w1, var_lo, var_hi, flags, variants, e_off, e_pos, e_ref_len, e_alt_off,
+                         e_alt_len, e_gt, e_alt_pool, max_window, pitch, err=None):
+    """encode_windows with a list of extra records per row (vf_encode_windows_edits): row w owns the records
+    [e_off[w], e_off[w + 1]) (CSR, sorted by pos within the row) and encodes as encode_windows does on the table with
+    each record inserted after every record of pos <= its own.  e_off int32 [n + 1]; e_pos / e_ref_len / e_alt_off /
+    e_alt_len int32 and e_gt uint8 (0 skip, 1 het, 2 hom) [e_off[-1]]; e_alt_pool uint8; device tensors.
+    -> (out uint8 [n, pitch], out_len int32 [n], applied uint8 [e_off[-1]] (1: that record was applied), err)."""
+    n = w0.numel()
+    dev = genome.device
+    for t in (w0, w1, var_lo, var_hi):
+        assert t.dtype == torch.int32 and t.numel() == n and t.is_contiguous()
+    assert win_base.dtype == torch.int64 and flags.dtype == torch.uint8 and e_alt_pool.dtype == torch.uint8
+    off = e_off.cpu().numpy()
+    if e_off.dtype != torch.int32 or off.shape != (n + 1,) or off[0] != 0 or (np.diff(off) < 0).any():
+        raise ValueError(f"e_off must be int32 [{n + 1}] offsets from 0, nondecreasing (got {e_off.dtype} "
+                         f"{tuple(off.shape)})")
+    m = int(off[-1])
+    for t, dt in ((e_pos, torch.int32), (e_ref_len, torch.int32), (e_alt_off, torch.int32), (e_alt_len, torch.int32),
+                  (e_gt, torch.uint8)):
+        if t.dtype != dt or t.numel() != m or not t.is_contiguous():
+            raise ValueError(f"extra-record arrays must be contiguous {dt} [{m}] (e_off[-1]), got {t.dtype} "
+                             f"[{t.numel()}]")
+    # kernels need non-NULL arrays; the tensors stay referenced here until the launch is enqueued
+    e = [e_off.to(dev)] + [t if t.numel() else torch.zeros(1, dtype=t.dtype, device=dev)
+                           for t in (e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool)]
+    out = torch.empty((n, pitch), dtype=torch.uint8, device=dev)
+    out_len = torch.empty(n, dtype=torch.int32, device=dev)
+    applied = torch.empty(max(m, 1), dtype=torch.uint8, device=dev)
+    if err is None:
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+    v = variants
+    with _timed("stage1_encode_edit", nbytes=float(n) * max_window * 2):  # window bytes read + written (upper bound)
+        check(_lib.lib().vf_encode_windows_edits(ptr(genome), ptr(win_base), ptr(w0), ptr(w1), ptr(var_lo), ptr(var_hi),
+                                                 ptr(flags), ptr(v["pos"]), ptr(v["ref_len"]), ptr(v["alt_off"]),
+                                                 ptr(v["alt_len"]), ptr(v["gt"]), ptr(v["alt_pool"]),
+                                                 *[ptr(t) for t in e], n, int(max_window), ptr(out), int(pitch),
+                                                 ptr(out_len), ptr(applied), ptr(err), stream()))
+    return out, out_len, applied[:m], err
+
+
 def _genotype_rows(w0, w1, var_lo, var_hi, flags, variants):
     n = w0.numel()
     for t in (w0, w1, var_lo, var_hi):

@@ -212,6 +212,15 @@ class HotPath:
         from .deletion import deletion_scan
         return deletion_scan(self, genes, deletions, variants, embeddings=embeddings, to_host=to_host, **kw)
 
+    def variant_sets(self, genes, sets, variants: SampleVariants = None, embeddings=False, to_host=True, **kw):
+        """In-silico variant combinations (variant_sets.scan): sets[i] = list of sets for gene i, each a list of
+        variant_sets.Record(chrom, pos (1-based), ref, alt, gt=2).  -> (pred [sum T], emb [sum T, D]) of the baseline,
+        bit-identical to predict(genes, variants), per gene the set predictions [n, T] (+ per gene [n, T, D] embeddings
+        when `embeddings`), each bit-identical to predict on the gene with the set's records added to the background,
+        and per gene dict(cre=bool [n, C] in batch order, gene=bool [n], records=per set bool [len(set)])."""
+        from .variant_sets import scan
+        return scan(self, genes, sets, variants, embeddings=embeddings, to_host=to_host, **kw)
+
     @staticmethod
     def _raise_on_stage1_error(err):
         """The encode kernel flags windows it could not build (their tokens are then all padding): never hand out

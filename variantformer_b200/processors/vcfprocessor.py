@@ -340,6 +340,116 @@ class VCFProcessor:
                   for i, gid in enumerate(gene_ids)]
         return pd.concat(frames, ignore_index=True)
 
+    def _edit_query(self, vcf_path, query_df):
+        """The query of an in-silico edit with VCFDataset's rules: -> (dataset, filtered query, GeneSpec per row, sample
+        path per row (None: the reference genome))."""
+        from ..pipeline import GeneSpec
+        ds = self.model_config.dataset
+        dataset = VCFDataset(max_length=ds.max_length, max_chunks=ds.max_chunks, cre_neighbour_hood=ds.cre_neighbour_hood,
+                             gencode_v24=ds.gencode_v24, gene_cre_manifest=self.gene_cre_manifest,
+                             gene_upstream_neighbour_hood=ds.gene_upstream_neighbour_hood,
+                             gene_downstream_neighbour_hood=ds.gene_downstream_neighbour_hood, query_df=query_df,
+                             fasta_path=self.vcf_loader_config.fasta_path, vcf_path=vcf_path)
+        q = dataset.query_df
+        genes, paths = [], []
+        for _, row in q.iterrows():
+            gid = row["gene_id"]
+            info = dataset._get_gene_info(gid)
+            assert info["chromosome"] in ["chr" + str(i) for i in range(1, 23)], \
+                f"Chromosome {info['chromosome']} is not a valid chromosome. Sex chromosomes are not supported"
+            m, _ = dataset.cre_manifest(gid, info)
+            labels = np.asarray([dataset.ref_cre_to_idx[x] for x in m["cre_name"]], np.int64)
+            genes.append(GeneSpec(info["chromosome"], int(info["start"]), int(info["end"]), info["strand"],
+                                  m["start_cre"].to_numpy(np.int64), m["end_cre"].to_numpy(np.int64), labels,
+                                  list(row["tissues"]), cre_chrom=list(m["chromosome"])))
+            p = row["vcf_path"] if "vcf_path" in q.columns else vcf_path
+            paths.append(None if p is None or (not isinstance(p, str) and pd.isna(p)) or str(p) == "" else str(p))
+        return dataset, q, genes, paths
+
+    def _run_sets(self, dataset, genes, sets, paths, gene_ids):
+        """variant_sets.scan per sample (one HotPath call per distinct path, in first-appearance order).
+        -> per query row (baseline fp32 [T], set predictions [n, T], applied)."""
+        from ..pipeline import HotPath
+        ds = self.model_config.dataset
+        model, _, _ = self.load_model()
+        hot = HotPath(model.engine(), dataset._genome(), max_length=ds.max_length, max_chunks=ds.max_chunks,
+                      cre_neighbour_hood=ds.cre_neighbour_hood, gene_upstream=ds.gene_upstream_neighbour_hood,
+                      gene_downstream=ds.gene_downstream_neighbour_hood)
+        out = [None] * len(genes)
+        for p in dict.fromkeys(paths):
+            rows = [i for i, x in enumerate(paths) if x == p]
+            pred, _, s_pred, app = hot.variant_sets([genes[i] for i in rows], [sets[i] for i in rows],
+                                                    dataset._variants(p), min_gene_len=1000,
+                                                    gene_names=[gene_ids[i] for i in rows])
+            off = np.concatenate([[0], np.cumsum([len(genes[i].tissues) for i in rows])])
+            for k, i in enumerate(rows):
+                out[i] = (pred[off[k]:off[k + 1]], s_pred[k], app[k])
+        return out
+
+    def variant_sets(self, vcf_path: str, query_df: pd.DataFrame, variants: pd.DataFrame):
+        """In-silico variant combinations (DESIGN.md section 17): every query row predicted with each set of VCF
+        records added to its sample, each window no record of the set lies in encoded once.  A set's prediction equals
+        what create_data + predict give on the sample's VCF with the set's lines added (each after the lines of its
+        POS).  The query is filtered with VCFDataset's rules; the sample is `vcf_path` or a per-row vcf_path column
+        (empty or missing: the reference genome).  variants: DataFrame with columns gene_id, set (a label), chromosome,
+        pos (1-based), ref, alt, optionally gt (1 het, 2 hom-alt; default 2) and label; one row per record.  Invalid
+        records raise a ValueError before the model is loaded.  Writes no file.
+        -> one row per (query row, set, tissue), in that order (sets in first-appearance order), columns
+        variant_sets.SET_COLUMNS: set, n_records, records_applied (records applied in at least one window),
+        cre_windows_changed / gene_window_changed / changed, baseline_expression, predicted_expression and delta."""
+        from .. import variant_sets as vs
+        user = vs.user_records(variants, sets=True)
+        dataset, q, genes, paths = self._edit_query(vcf_path, query_df)
+        gene_ids = list(q["gene_id"])
+        for gid in user:
+            if gid not in set(gene_ids):
+                print(f"Gene {gid} of the variant sets is not in the query so skipping it")
+        sets = [user.get(gid, []) for gid in gene_ids]
+        vs.check_sets(genes, [[rs for _, rs, _ in s] for s in sets], dataset._genome(), gene_ids)
+        res = self._run_sets(dataset, genes, [[rs for _, rs, _ in s] for s in sets], paths, gene_ids)
+        frames = [vs.set_frame(gid, list(q["tissue_names"].iloc[i]), [sid for sid, _, _ in sets[i]],
+                               [len(rs) for _, rs, _ in sets[i]], res[i][2], res[i][0], res[i][1])
+                  for i, gid in enumerate(gene_ids)]
+        return pd.concat(frames, ignore_index=True)
+
+    def variant_interactions(self, vcf_path: str, query_df: pd.DataFrame, variants: pd.DataFrame):
+        """Pairwise interaction scan (DESIGN.md section 17): for every query row, each of its gene's variants singly and
+        every unordered pair of them added to the sample, all in one planner call per sample.  Query and sample as
+        variant_sets; variants: DataFrame with columns gene_id, chromosome, pos (1-based), ref, alt, optionally gt
+        (default 2) and label.  Pairs whose REF spans overlap (two alleles of one site) are skipped.  Invalid records
+        raise a ValueError before the model is loaded.  Writes no file.
+        -> one row per (query row, pair, tissue), columns variant_sets.INTERACTION_COLUMNS: variant_a / variant_b
+        (labels), same_window (one window holds both), baseline_expression, expression_a / _b / _ab, delta_a / _b / _ab,
+        interaction = delta_ab - delta_a - delta_b and log2_interaction = log2((ab + 1e-10)(base + 1e-10) /
+        ((a + 1e-10)(b + 1e-10)))."""
+        from .. import variant_sets as vs
+        user = vs.user_records(variants, sets=False)
+        dataset, q, genes, paths = self._edit_query(vcf_path, query_df)
+        gene_ids = list(q["gene_id"])
+        for gid in user:
+            if gid not in set(gene_ids):
+                print(f"Gene {gid} of the variants is not in the query so skipping it")
+        scans = []
+        for gid in gene_ids:
+            recs, labels = user.get(gid, ([], []))
+            sets, _, pair_idx, overlapping = vs.pairs(recs)
+            for a, b in overlapping:
+                print(f"Variants {labels[a]} and {labels[b]} of gene {gid} overlap so skipping their pair")
+            scans.append((labels, sets, pair_idx))
+        ds = self.model_config.dataset
+        checked = vs.check_sets(genes, [s for _, s, _ in scans], dataset._genome(), gene_ids)
+        res = self._run_sets(dataset, genes, [s for _, s, _ in scans], paths, gene_ids)
+        frames = []
+        for i, gid in enumerate(gene_ids):
+            labels, sets, pair_idx = scans[i]
+            n = len(labels)
+            same = vs.shared_window(genes[i], checked[i][n:], ds.cre_neighbour_hood, ds.gene_upstream_neighbour_hood,
+                                    ds.gene_downstream_neighbour_hood)
+            base, sp, _ = res[i]
+            frames.append(vs.interaction_frame(gid, list(q["tissue_names"].iloc[i]), labels, pair_idx, same, base,
+                                               sp[:n], sp[n:]))
+        return pd.concat(frames, ignore_index=True)
+
     def format_output(self, df, predictions):
         pred_exp, embd = [], []
         for p in predictions:
