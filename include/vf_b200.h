@@ -268,6 +268,31 @@ int vf_window_genotype_equal(const int32_t* w0, const int32_t* w1, const int32_t
                              const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, int n_rows,
                              const int32_t* rep, int32_t* equal, void* stream);
 /*
+ * The same keys and comparison for rows with a list of extra records (variant sets across a cohort), the records in the
+ * CSR form of vf_encode_windows_edits (e_off int32 [n_rows + 1], e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool):
+ * a row's applied list is what vf_encode_windows_edits applies for it, background and extra records merged by the same
+ * device walk.  The hash and the comparison read record content only, so a row whose extras are all blocked keys and
+ * compares equal to its window without them, and a row with no extras gets vf_window_genotype_keys' key, count and
+ * out_len bit for bit.  vf_window_genotype_keys_edits also writes applied uint8 [e_off[n_rows]], equal to what
+ * vf_encode_windows_edits writes for the row.  A row whose extras are not sorted by pos sets *err to 4, count -1 and
+ * out_len 0, and compares equal to no other row.  Other arguments, outputs and errors as vf_window_genotype_keys /
+ * vf_window_genotype_equal; n_rows < 0 or a NULL array fails before any launch.
+ */
+int vf_window_genotype_keys_edits(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                                  const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len,
+                                  const int32_t* v_alt_off, const int32_t* v_alt_len, const uint8_t* v_gt,
+                                  const uint8_t* alt_pool, const int32_t* e_off, const int32_t* e_pos,
+                                  const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
+                                  const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_rows, unsigned long long* keys,
+                                  int32_t* count, int32_t* out_len, uint8_t* applied, int32_t* err, void* stream);
+int vf_window_genotype_equal_edits(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                                   const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len,
+                                   const int32_t* v_alt_off, const int32_t* v_alt_len, const uint8_t* v_gt,
+                                   const uint8_t* alt_pool, const int32_t* e_off, const int32_t* e_pos,
+                                   const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
+                                   const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_rows, const int32_t* rep,
+                                   int32_t* equal, void* stream);
+/*
  * Single-base substitution of encoded windows (in-silico saturation mutagenesis): row r of out = the source row
  * src[row_src[r]] (src_len[row_src[r]] bytes, as vf_encode_windows wrote it) with ONE base replaced by row_base[r].
  * row_off[r] = forward-strand offset pos0 - w0 of the base; flags[r] bit0 = the source was reverse-complemented: the base

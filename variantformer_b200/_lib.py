@@ -52,6 +52,8 @@ SIGNATURES = {
     "vf_encode_windows_edits": ([_vp] * 20 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp, _vp], _i32),
     "vf_window_genotype_keys": ([_vp] * 11 + [_i32, _vp, _vp, _vp, _vp, _vp], _i32),
     "vf_window_genotype_equal": ([_vp] * 11 + [_i32, _vp, _vp, _vp], _i32),
+    "vf_window_genotype_keys_edits": ([_vp] * 18 + [_i32, _vp, _vp, _vp, _vp, _vp, _vp], _i32),
+    "vf_window_genotype_equal_edits": ([_vp] * 18 + [_i32, _vp, _vp, _vp], _i32),
     "vf_mutate_windows": ([_vp, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
     "vf_splice_windows": ([_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
     "vf_bpe_tokenize": ([_vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _i64,

@@ -417,6 +417,145 @@ int window_genotype_equal(const int32_t* w0, const int32_t* w1, const int32_t* v
     return 0;
 }
 
+// vf_window_genotype_keys_edits / _equal_edits: the same key and comparison over MergedScan, the walk
+// vf_encode_windows_edits encodes with, so a row's list is its background and its extra records (CSR in `e`) merged by
+// the encoder's own rule.  The hash and the comparison read a record's content, not its index, so background and extra
+// records hash alike: a row whose extras are all blocked keys (and compares) equal to the same window without them, and a
+// row without extras gets the plain kernel's key, count and out_len.  (Kernels of their own: the plain ones keep their
+// code.)
+struct EditRecords {                  // record v of a merged walk: a background index (>= 0) or a tagged extra (< -1)
+    const GenotypeRows& p;
+    const EditParams& e;
+    __device__ __forceinline__ int pos(int v) const { return v < 0 ? e.pos[-2 - v] : p.v_pos[v]; }
+    __device__ __forceinline__ int ref_len(int v) const { return v < 0 ? e.ref_len[-2 - v] : p.v_ref_len[v]; }
+    __device__ __forceinline__ int alt_len(int v) const { return v < 0 ? e.alt_len[-2 - v] : p.v_alt_len[v]; }
+    __device__ __forceinline__ uint8_t gt(int v) const { return v < 0 ? e.gt[-2 - v] : p.v_gt[v]; }
+    __device__ __forceinline__ const uint8_t* alt(int v) const {
+        return v < 0 ? e.alt_pool + e.alt_off[-2 - v] : p.alt_pool + p.v_alt_off[v];
+    }
+    __device__ __forceinline__ MergedScan scan(int r) const {
+        return MergedScan(p.var_lo[r], p.var_hi[r], p.w0[r], p.w1[r], p.flags[r] & 2, e, e.off[r], e.off[r + 1]);
+    }
+    __device__ __forceinline__ bool sorted(int r) const {      // the encoder's error 4 otherwise
+        for (int k = e.off[r] + 1; k < e.off[r + 1]; ++k)
+            if (e.pos[k] < e.pos[k - 1]) return false;
+        return true;
+    }
+};
+
+__global__ void __launch_bounds__(128)
+window_genotype_keys_edits_kernel(const GenotypeRows p, const EditParams e, unsigned long long* keys, int32_t* count,
+                                  int32_t* out_len, int32_t* err) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= p.n_rows) return;
+    const EditRecords v{p, e};
+    for (int k = e.off[r]; k < e.off[r + 1]; ++k) e.applied[k] = 0;
+    if (!v.sorted(r)) {                                  // an unsorted row is not merged, as in the encoder
+        atomicMax(err, 4);
+        count[r] = -1;
+        if (out_len) out_len[r] = 0;
+        keys[2 * r] = keys[2 * r + 1] = 0ull;
+        return;
+    }
+    constexpr uint64_t kMul0 = 0x9E3779B97F4A7C15ull, kMul1 = 0xC2B2AE3D27D4EB4Full;
+    uint64_t h0 = 0x243F6A8885A308D3ull, h1 = 0x13198A2E03707344ull;
+    int n = 0, shift = 0;
+    bool bad = false;
+    MergedScan sc = v.scan(r);
+    for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)) != -1;) {
+        if (n == kMaxApplied) { bad = true; break; }     // the encoder's cap: err 2 on exactly the rows it flags
+        if (i < 0) e.applied[extra_tag(i)] = 1;          // (extra_tag is its own inverse)
+        ++n;
+        const int al = v.alt_len(i);
+        shift += al - v.ref_len(i);
+        const uint64_t a = ((uint64_t)(uint32_t)v.pos(i) << 32) | (uint32_t)v.ref_len(i);
+        const uint64_t b = ((uint64_t)v.gt(i) << 32) | (uint32_t)al;
+        h0 = mix64(mix64(h0, a, kMul0), b, kMul0);
+        h1 = mix64(mix64(h1, b, kMul1), a, kMul1);
+        const uint8_t* s = v.alt(i);
+        for (int j = 0; j < al; j += 8) {
+            uint64_t w = 0;
+            for (int k = 0; k < 8 && j + k < al; ++k) w |= (uint64_t)s[j + k] << (8 * k);
+            h0 = mix64(h0, w, kMul0);
+            h1 = mix64(h1, w ^ 0x5555555555555555ull, kMul1);
+        }
+    }
+    if (bad) atomicMax(err, 2);
+    count[r] = bad ? -1 : n;
+    if (out_len) out_len[r] = (p.w1[r] - p.w0[r]) + shift;
+    keys[2 * r] = n ? h0 : 0ull;
+    keys[2 * r + 1] = n ? h1 : 0ull;
+}
+
+__global__ void __launch_bounds__(128)
+window_genotype_equal_edits_kernel(const GenotypeRows p, const EditParams e, const int32_t* rep, int32_t* equal) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= p.n_rows) return;
+    const int q = rep[r];
+    if (q == r) { equal[r] = 1; return; }
+    const EditRecords v{p, e};
+    // a row the encoder refuses (unsorted extras) equals no other
+    int eq = p.w0[r] == p.w0[q] && p.w1[r] == p.w1[q] && ((p.flags[r] ^ p.flags[q]) & 3) == 0 && v.sorted(r) &&
+             v.sorted(q);
+    MergedScan a = v.scan(r), b = v.scan(q);
+    while (eq) {
+        const int i = a.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt);
+        const int j = b.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt);
+        if (i == -1 || j == -1) { eq = i == j; break; }
+        const int al = v.alt_len(i);
+        if (v.pos(i) != v.pos(j) || v.ref_len(i) != v.ref_len(j) || v.gt(i) != v.gt(j) || al != v.alt_len(j)) {
+            eq = 0;
+            break;
+        }
+        const uint8_t* x = v.alt(i);
+        const uint8_t* y = v.alt(j);
+        for (int k = 0; k < al; ++k)
+            if (x[k] != y[k]) { eq = 0; break; }
+    }
+    equal[r] = eq;
+}
+
+static int genotype_edits_check(const GenotypeRows& g, const EditParams& e, const char* what) {
+    if (const int rc = genotype_rows_check(g, what)) return rc;
+    VF_REQUIRE(g.n_rows == 0 || (e.off && e.pos && e.ref_len && e.alt_off && e.alt_len && e.gt && e.alt_pool),
+               "%s: an extra-record array is NULL", what);
+    return 0;
+}
+
+int window_genotype_keys_edits(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                               const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len,
+                               const int32_t* v_alt_off, const int32_t* v_alt_len, const uint8_t* v_gt,
+                               const uint8_t* alt_pool, const int32_t* e_off, const int32_t* e_pos,
+                               const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
+                               const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_rows, unsigned long long* keys,
+                               int32_t* count, int32_t* out_len, uint8_t* applied, int32_t* err, cudaStream_t s) {
+    const GenotypeRows g{w0, w1, var_lo, var_hi, flags, v_pos, v_ref_len, v_alt_off, v_alt_len, v_gt, alt_pool, n_rows};
+    const EditParams e{e_off, e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool, applied};
+    if (const int rc = genotype_edits_check(g, e, "window_genotype_keys_edits")) return rc;
+    if (n_rows == 0) return 0;
+    VF_REQUIRE(keys && count && applied && err, "window_genotype_keys_edits: keys, count, applied and err are required");
+    window_genotype_keys_edits_kernel<<<(n_rows + 127) / 128, 128, 0, s>>>(g, e, keys, count, out_len, err);
+    VF_LAUNCH_OK("window_genotype_keys_edits_kernel launch");
+    return 0;
+}
+
+int window_genotype_equal_edits(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                                const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len,
+                                const int32_t* v_alt_off, const int32_t* v_alt_len, const uint8_t* v_gt,
+                                const uint8_t* alt_pool, const int32_t* e_off, const int32_t* e_pos,
+                                const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
+                                const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_rows, const int32_t* rep,
+                                int32_t* equal, cudaStream_t s) {
+    const GenotypeRows g{w0, w1, var_lo, var_hi, flags, v_pos, v_ref_len, v_alt_off, v_alt_len, v_gt, alt_pool, n_rows};
+    const EditParams e{e_off, e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool, nullptr};
+    if (const int rc = genotype_edits_check(g, e, "window_genotype_equal_edits")) return rc;
+    if (n_rows == 0) return 0;
+    VF_REQUIRE(rep && equal, "window_genotype_equal_edits: rep and equal are required");
+    window_genotype_equal_edits_kernel<<<(n_rows + 127) / 128, 128, 0, s>>>(g, e, rep, equal);
+    VF_LAUNCH_OK("window_genotype_equal_edits_kernel launch");
+    return 0;
+}
+
 // ---------------------------------------------------------------------------------
 // splice_windows: an encoded window with ONE base replaced by an allele of k >= 0 bases (variant tables: a hom ALT of
 // any length, k = 0 deleting the base; saturation mutagenesis: k = 1).  Row r of `out` is the source row src[row_src[r]] with the base at

@@ -74,6 +74,20 @@ int window_genotype_equal(const int32_t* w0, const int32_t* w1, const int32_t* v
                           const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_off,
                           const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, int n_rows,
                           const int32_t* rep, int32_t* equal, cudaStream_t s);
+int window_genotype_keys_edits(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                               const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len,
+                               const int32_t* v_alt_off, const int32_t* v_alt_len, const uint8_t* v_gt,
+                               const uint8_t* alt_pool, const int32_t* e_off, const int32_t* e_pos,
+                               const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
+                               const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_rows, unsigned long long* keys,
+                               int32_t* count, int32_t* out_len, uint8_t* applied, int32_t* err, cudaStream_t s);
+int window_genotype_equal_edits(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
+                                const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len,
+                                const int32_t* v_alt_off, const int32_t* v_alt_len, const uint8_t* v_gt,
+                                const uint8_t* alt_pool, const int32_t* e_off, const int32_t* e_pos,
+                                const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
+                                const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_rows, const int32_t* rep,
+                                int32_t* equal, cudaStream_t s);
 int mutate_windows(const uint8_t* src, int64_t src_pitch, const int32_t* src_len, const int32_t* row_src,
                    const int32_t* row_off, const uint8_t* row_base, const uint8_t* flags, int n_rows, uint8_t* out,
                    int64_t out_pitch, int32_t* out_len, int32_t* err, cudaStream_t s);

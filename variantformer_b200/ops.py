@@ -495,6 +495,26 @@ def encode_windows_edit(genome, win_base, w0, w1, var_lo, var_hi, flags, variant
     return out, out_len, applied, err
 
 
+def _edit_records(n, dev, e_off, e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool):
+    """encode_windows_edits' host checks of the CSR extra records of n rows -> (device arrays with non-NULL stand-ins for
+    empty ones, number of records)."""
+    off = e_off.cpu().numpy()
+    if e_off.dtype != torch.int32 or off.shape != (n + 1,) or off[0] != 0 or (np.diff(off) < 0).any():
+        raise ValueError(f"e_off must be int32 [{n + 1}] offsets from 0, nondecreasing (got {e_off.dtype} "
+                         f"{tuple(off.shape)})")
+    m = int(off[-1])
+    for t, dt in ((e_pos, torch.int32), (e_ref_len, torch.int32), (e_alt_off, torch.int32), (e_alt_len, torch.int32),
+                  (e_gt, torch.uint8)):
+        if t.dtype != dt or t.numel() != m or not t.is_contiguous():
+            raise ValueError(f"extra-record arrays must be contiguous {dt} [{m}] (e_off[-1]), got {t.dtype} "
+                             f"[{t.numel()}]")
+    if e_alt_pool.dtype != torch.uint8:
+        raise ValueError(f"e_alt_pool must be uint8, got {e_alt_pool.dtype}")
+    # kernels need non-NULL arrays; the tensors stay referenced by the caller until the launch is enqueued
+    return [e_off.to(dev)] + [t if t.numel() else torch.zeros(1, dtype=t.dtype, device=dev)
+                              for t in (e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool)], m
+
+
 def encode_windows_edits(genome, win_base, w0, w1, var_lo, var_hi, flags, variants, e_off, e_pos, e_ref_len, e_alt_off,
                          e_alt_len, e_gt, e_alt_pool, max_window, pitch, err=None):
     """encode_windows with a list of extra records per row (vf_encode_windows_edits): row w owns the records
@@ -507,19 +527,7 @@ def encode_windows_edits(genome, win_base, w0, w1, var_lo, var_hi, flags, varian
     for t in (w0, w1, var_lo, var_hi):
         assert t.dtype == torch.int32 and t.numel() == n and t.is_contiguous()
     assert win_base.dtype == torch.int64 and flags.dtype == torch.uint8 and e_alt_pool.dtype == torch.uint8
-    off = e_off.cpu().numpy()
-    if e_off.dtype != torch.int32 or off.shape != (n + 1,) or off[0] != 0 or (np.diff(off) < 0).any():
-        raise ValueError(f"e_off must be int32 [{n + 1}] offsets from 0, nondecreasing (got {e_off.dtype} "
-                         f"{tuple(off.shape)})")
-    m = int(off[-1])
-    for t, dt in ((e_pos, torch.int32), (e_ref_len, torch.int32), (e_alt_off, torch.int32), (e_alt_len, torch.int32),
-                  (e_gt, torch.uint8)):
-        if t.dtype != dt or t.numel() != m or not t.is_contiguous():
-            raise ValueError(f"extra-record arrays must be contiguous {dt} [{m}] (e_off[-1]), got {t.dtype} "
-                             f"[{t.numel()}]")
-    # kernels need non-NULL arrays; the tensors stay referenced here until the launch is enqueued
-    e = [e_off.to(dev)] + [t if t.numel() else torch.zeros(1, dtype=t.dtype, device=dev)
-                           for t in (e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool)]
+    e, m = _edit_records(n, dev, e_off, e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool)
     out = torch.empty((n, pitch), dtype=torch.uint8, device=dev)
     out_len = torch.empty(n, dtype=torch.int32, device=dev)
     applied = torch.empty(max(m, 1), dtype=torch.uint8, device=dev)
@@ -576,6 +584,47 @@ def window_genotype_equal(w0, w1, var_lo, var_hi, flags, variants, rep):
     equal = torch.empty(n, dtype=torch.int32, device=w0.device)
     with _timed("stage1_keys"):
         check(_lib.lib().vf_window_genotype_equal(*args, ptr(rep), ptr(equal), stream()))
+    return equal
+
+
+def window_genotype_keys_edits(w0, w1, var_lo, var_hi, flags, variants, e_off, e_pos, e_ref_len, e_alt_off, e_alt_len,
+                               e_gt, e_alt_pool, key_bits=128, err=None):
+    """window_genotype_keys for rows with a list of extra records each, in encode_windows_edits' CSR form
+    (vf_window_genotype_keys_edits): a row's key, count and length are those of the list encode_windows_edits applies
+    for it (background and extras merged); a row without extras gets window_genotype_keys' outputs.  -> (keys, count,
+    lens, applied uint8 [e_off[-1]] (encode_windows_edits' flags for the same rows), err); err 4 (count -1, length 0)
+    for a row whose extras are not sorted by pos."""
+    n, args = _genotype_rows(w0, w1, var_lo, var_hi, flags, variants)
+    dev = w0.device
+    e, m = _edit_records(n, dev, e_off, e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool)
+    keys = torch.empty((n, 2), dtype=torch.int64, device=dev)
+    count = torch.empty(n, dtype=torch.int32, device=dev)
+    lens = torch.empty(n, dtype=torch.int32, device=dev)
+    applied = torch.empty(max(m, 1), dtype=torch.uint8, device=dev)
+    if err is None:
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+    with _timed("stage1_keys"):
+        check(_lib.lib().vf_window_genotype_keys_edits(*args[:-1], *[ptr(t) for t in e], n, ptr(keys), ptr(count),
+                                                       ptr(lens), ptr(applied), ptr(err), stream()))
+    if key_bits < 64:
+        keys[:, 0] &= (1 << key_bits) - 1
+        keys[:, 1] = 0
+    elif key_bits < 128:
+        keys[:, 1] &= (1 << (key_bits - 64)) - 1
+    return keys, count, lens, applied[:m], err
+
+
+def window_genotype_equal_edits(w0, w1, var_lo, var_hi, flags, variants, e_off, e_pos, e_ref_len, e_alt_off, e_alt_len,
+                                e_gt, e_alt_pool, rep):
+    """1 where row r applies the same record list as row rep[r], element by element, extras merged as in
+    window_genotype_keys_edits (vf_window_genotype_equal_edits).  -> int32 [n]."""
+    n, args = _genotype_rows(w0, w1, var_lo, var_hi, flags, variants)
+    assert rep.dtype == torch.int32 and rep.numel() == n
+    e, _ = _edit_records(n, w0.device, e_off, e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool)
+    equal = torch.empty(n, dtype=torch.int32, device=w0.device)
+    with _timed("stage1_keys"):
+        check(_lib.lib().vf_window_genotype_equal_edits(*args[:-1], *[ptr(t) for t in e], n, ptr(rep), ptr(equal),
+                                                        stream()))
     return equal
 
 

@@ -221,6 +221,16 @@ class HotPath:
         from .variant_sets import scan
         return scan(self, genes, sets, variants, embeddings=embeddings, to_host=to_host, **kw)
 
+    def cohort_variant_sets(self, genes, sets, cohort, sample_idx=None, embeddings=False, to_host=True, **kw):
+        """Variant sets across a cohort (cohort_sets.scan): every set of variant_sets' form in every sample of a cohort
+        (stage1.CohortVariants; sample_idx: which of its samples, default all), each distinct edited window encoded
+        once across samples.  -> (pred [S, sum T], emb [S, sum T, D]) of the baselines, row s bit-identical to
+        predict_cohort's, per gene the set predictions [S, n, T] (+ per gene [S, n, T, D] embeddings when `embeddings`),
+        and per gene dict(cre=bool [S, n, C] in batch order, gene=bool [S, n], records=per set bool [S, len(set)]);
+        sample s's entries are bit-identical to variant_sets(genes, sets, that sample's SampleVariants)."""
+        from .cohort_sets import scan
+        return scan(self, genes, sets, cohort, sample_idx, embeddings=embeddings, to_host=to_host, **kw)
+
     @staticmethod
     def _raise_on_stage1_error(err):
         """The encode kernel flags windows it could not build (their tokens are then all padding): never hand out

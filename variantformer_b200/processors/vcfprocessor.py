@@ -412,6 +412,68 @@ class VCFProcessor:
                   for i, gid in enumerate(gene_ids)]
         return pd.concat(frames, ignore_index=True)
 
+    def cohort_variant_sets(self, vcf_path: str, query_df: pd.DataFrame, variants: pd.DataFrame, samples=None,
+                            genes_per_slab=8, samples_per_slab=256):
+        """Variant sets across a cohort (DESIGN.md section 18): every query row predicted, in every sample of one
+        multi-sample VCF (samples: names, default every sample column), with each set of records added to that sample.
+        The query follows predict_cohort's rules (VCFDataset's filtering, one region-restricted parse of the VCF, sample
+        sub-blocks past the kernels' int32 limits); variants as variant_sets (gene_id, set, chromosome, pos, ref, alt,
+        optionally gt and label), invalid records raising a ValueError before the model is loaded.  A record the
+        sample's own records block is not applied in that sample (records_applied / changed say so per sample).  Each
+        row equals what variant_sets gives on that sample's VCF alone.  Computed in slabs of genes_per_slab query genes x
+        samples_per_slab samples, so device memory does not grow with the query or the cohort.  Writes no file.
+        -> one row per (sample, query row, set, tissue), in that order: sample, then variant_sets.SET_COLUMNS
+        (variant_sets.cohort_summary condenses it over the samples)."""
+        from .. import ingest
+        from .. import variant_sets as vs
+        from ..pipeline import HotPath
+        from ..stage1 import CohortVariants, cre_window, gene_window
+        user = vs.user_records(variants, sets=True)
+        dataset, q, genes, _ = self._edit_query(None, query_df)
+        gene_ids = list(q["gene_id"])
+        for gid in user:
+            if gid not in set(gene_ids):
+                print(f"Gene {gid} of the variant sets is not in the query so skipping it")
+        sets = [user.get(gid, []) for gid in gene_ids]
+        recs = [[rs for _, rs, _ in s] for s in sets]
+        vs.check_sets(genes, recs, dataset._genome(), gene_ids)
+        ds = self.model_config.dataset
+        nb, up, down = ds.cre_neighbour_hood, ds.gene_upstream_neighbour_hood, ds.gene_downstream_neighbour_hood
+        regions = []
+        for g in genes:
+            regions += [(c, *cre_window(a, b, nb)) for c, a, b in zip(g.cre_chrom, g.cre_start, g.cre_end)]
+            regions.append((g.chrom, *gene_window(g.start, g.end, g.strand, up, down)))
+        names, per_sample = ingest.load_vcf_cohort(vcf_path, samples=samples, regions=regions)
+        model, _, _ = self.load_model()
+        hot = HotPath(model.engine(), dataset._genome(), max_length=ds.max_length, max_chunks=ds.max_chunks,
+                      cre_neighbour_hood=nb, gene_upstream=up, gene_downstream=down)
+        frames = []
+        for s0 in range(0, len(names), samples_per_slab):
+            s1 = min(len(names), s0 + samples_per_slab)
+            per_s = [[] for _ in range(s1 - s0)]             # frames of each sample of the slab, in query order
+            # sample sub-blocks whose variant tables fit the kernels' int32 indices
+            for a, b in CohortVariants.blocks(per_sample[s0:s1]):
+                cv = CohortVariants(names[s0 + a:s0 + b], per_sample[s0 + a:s0 + b], hot.engine.device)
+                for g0 in range(0, len(genes), genes_per_slab):
+                    g1 = min(len(genes), g0 + genes_per_slab)
+                    pred, _, s_pred, app = hot.cohort_variant_sets(genes[g0:g1], recs[g0:g1], cv, min_gene_len=1000,
+                                                                   gene_names=gene_ids[g0:g1])
+                    off = np.concatenate([[0], np.cumsum([len(g.tissues) for g in genes[g0:g1]])])
+                    for s in range(b - a):
+                        for k, i in enumerate(range(g0, g1)):
+                            ap = dict(cre=app[k]["cre"][s], gene=app[k]["gene"][s],
+                                      records=[r[s] for r in app[k]["records"]])
+                            f = vs.set_frame(gene_ids[i], list(q["tissue_names"].iloc[i]), [sid for sid, _, _ in sets[i]],
+                                             [len(rs) for rs in recs[i]], ap, pred[s, off[k]:off[k + 1]], s_pred[k][s])
+                            f.insert(0, "sample", names[s0 + a + s])
+                            per_s[a + s].append(f)
+                    del pred, s_pred, app
+                del cv
+            frames += [f for fs in per_s for f in fs]
+        if not frames:
+            return pd.DataFrame(columns=["sample"] + vs.SET_COLUMNS)
+        return pd.concat(frames, ignore_index=True)
+
     def variant_interactions(self, vcf_path: str, query_df: pd.DataFrame, variants: pd.DataFrame):
         """Pairwise interaction scan (DESIGN.md section 17): for every query row, each of its gene's variants singly and
         every unordered pair of them added to the sample, all in one planner call per sample.  Query and sample as

@@ -439,6 +439,24 @@ def set_frame(gene_id, tissues, labels, n_records, applied, base_pred, set_pred)
         "delta": (sp - base[None, :]).reshape(-1)}, columns=SET_COLUMNS)
 
 
+SUMMARY_COLUMNS = ["gene_id", "set", "tissue", "n_samples", "n_changed", "mean_delta", "sd_delta", "min_delta",
+                   "max_delta"]
+
+
+def cohort_summary(frame):
+    """The background dependence of each set across a cohort: one row per (gene_id, set, tissue) of a frame of
+    VCFProcessor.cohort_variant_sets (columns sample + SET_COLUMNS), in first-appearance order.  n_samples, n_changed
+    (samples whose windows the set changed), and the mean, standard deviation (ddof 0), minimum and maximum of delta
+    over the samples, in float64."""
+    keys = ["gene_id", "set", "tissue"]
+    d = frame.assign(delta=frame["delta"].astype(np.float64))
+    g = d.groupby(keys, sort=False)
+    out = pd.DataFrame({"n_samples": g["sample"].size(), "n_changed": g["changed"].sum().astype(np.int64),
+                        "mean_delta": g["delta"].mean(), "sd_delta": g["delta"].std(ddof=0),
+                        "min_delta": g["delta"].min(), "max_delta": g["delta"].max()}).reset_index()
+    return out[SUMMARY_COLUMNS]
+
+
 INTERACTION_COLUMNS = ["gene_id", "tissue", "variant_a", "variant_b", "same_window", "baseline_expression",
                        "expression_a", "expression_b", "expression_ab", "delta_a", "delta_b", "delta_ab", "interaction",
                        "log2_interaction"]
