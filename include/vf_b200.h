@@ -201,7 +201,8 @@ int vf_forest_predict(const float* x, int ldx, int n_rows, int d, const int32_t*
  * hom SNP -> ALT, indel/MNP -> REF span replaced by ALT, overlapping or window-straddling records skipped;
  * flags bit0 = reverse-complement the result, bit1 = SNP-only filter.
  * out: uint8 [n_win, pitch]; out_len int32 [n_win]; err: device int32 flag (1 pitch overflow, 2 >2048 records;
- * vf_encode_windows_edits also 4: a row's extra records are not sorted by pos).
+ * vf_encode_windows_edits also 4: a row's extra records are not sorted by pos; vf_encode_windows_overrides also 8: a
+ * row's override list is malformed).
  * Any n_win: batches of more than 65535 windows are launched in chunks of 65535.
  * Replaces the `samtools faidx | bcftools consensus -H I -e 'ALT~"<.*>"'` subprocess pair per window
  * (utils/data_process.py:17-101, :367-467) and utils/functions.py:129-172 (reverse_complement).
@@ -245,6 +246,22 @@ int vf_encode_windows_edits(const uint8_t* genome, const int64_t* win_base, cons
                             const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
                             const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_win, int max_window, uint8_t* out,
                             int64_t pitch, int32_t* out_len, uint8_t* applied, int32_t* err, void* stream);
+/*
+ * vf_encode_windows with a list of GENOTYPE OVERRIDES per row (variant attribution: the sample's own records removed or
+ * re-genotyped), in CSR form: row w owns the overrides [o_off[w], o_off[w + 1]) (o_off int32 [n_win + 1],
+ * nondecreasing), each {record o_idx (an index into the variant table), new gt o_gt (0 removed, 1 het, 2 hom-alt)},
+ * indices strictly increasing within the row and inside [var_lo[w], var_hi[w]).  Row w is encoded as vf_encode_windows
+ * encodes it on the table with those records' gts replaced, bit for bit, in the same kernel body (gt 0 is the line
+ * removed: the encoder skips gt 0 records).  A row whose indices are unsorted, repeated or outside its range sets *err to
+ * 8 and writes length 0; other rows are not affected.  Other arguments, outputs and errors as vf_encode_windows;
+ * n_win < 0 or a NULL array fails before any launch.
+ */
+int vf_encode_windows_overrides(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
+                                const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
+                                const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
+                                const uint8_t* v_gt, const uint8_t* alt_pool, const int32_t* o_off, const int32_t* o_idx,
+                                const uint8_t* o_gt, int n_win, int max_window, uint8_t* out, int64_t pitch,
+                                int32_t* out_len, int32_t* err, void* stream);
 /*
  * Which rows of a cohort encode to the same bytes.  Row r = one (window, sample): w0/w1/flags/var_lo/var_hi as in
  * vf_encode_windows (flags bit1 = SNP-only), the variant arrays those of vf_encode_windows (one concatenated table may

@@ -50,6 +50,7 @@ SIGNATURES = {
     "vf_encode_windows": ([_vp] * 13 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
     "vf_encode_windows_edit": ([_vp] * 18 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp, _vp], _i32),
     "vf_encode_windows_edits": ([_vp] * 20 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp, _vp], _i32),
+    "vf_encode_windows_overrides": ([_vp] * 16 + [_i32, _i32, _vp, _i64, _vp, _vp, _vp], _i32),
     "vf_window_genotype_keys": ([_vp] * 11 + [_i32, _vp, _vp, _vp, _vp, _vp], _i32),
     "vf_window_genotype_equal": ([_vp] * 11 + [_i32, _vp, _vp, _vp], _i32),
     "vf_window_genotype_keys_edits": ([_vp] * 18 + [_i32, _vp, _vp, _vp, _vp, _vp, _vp], _i32),

@@ -138,6 +138,16 @@ int vf_encode_windows_edits(const uint8_t* genome, const int64_t* win_base, cons
                                 v_gt, alt_pool, e_off, e_pos, e_ref_len, e_alt_off, e_alt_len, e_gt, e_alt_pool, n_win,
                                 max_window, out, pitch, out_len, applied, err, ST(stream));
 }
+int vf_encode_windows_overrides(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
+                                const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
+                                const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
+                                const uint8_t* v_gt, const uint8_t* alt_pool, const int32_t* o_off, const int32_t* o_idx,
+                                const uint8_t* o_gt, int n_win, int max_window, uint8_t* out, int64_t pitch,
+                                int32_t* out_len, int32_t* err, void* stream) {
+    return encode_windows_overrides(genome, win_base, w0, w1, var_lo, var_hi, flags, v_pos, v_ref_len, v_alt_off,
+                                    v_alt_len, v_gt, alt_pool, o_off, o_idx, o_gt, n_win, max_window, out, pitch,
+                                    out_len, err, ST(stream));
+}
 int vf_window_genotype_keys(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
                             const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_off,
                             const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, int n_rows,

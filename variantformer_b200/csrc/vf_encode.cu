@@ -108,6 +108,40 @@ struct MergedScan {
     }
 };
 
+// vf_encode_windows_overrides: a list of genotype overrides per row, (record index, new gt) in CSR form, indices strictly
+// increasing within the row and inside its [var_lo, var_hi).  The walk is AppliedScan's, reading each record's gt
+// through the list by a two-pointer merge in index order (O(1) per record), so a row encodes exactly as
+// vf_encode_windows does on the table with those gts replaced (gt 0: the line removed).  next() returns the applied
+// record's table index, and `g` holds the gt it was applied with (the kernel keeps it beside the index).
+struct OverrideParams {
+    const int32_t* off;               // [n_win + 1] row w owns overrides [off[w], off[w + 1])
+    const int32_t* idx;               // record index into the variant table
+    const uint8_t* gt;                // the record's new gt (0 removed, 1 het, 2 hom-alt)
+};
+
+struct OverrideScan {
+    AppliedScan sc;
+    const int32_t* idx; const uint8_t* gt;                // the list's arrays (by value: no copy of the parameters)
+    int k, ke, k_idx;                 // overrides [k, ke) still to walk; k_idx = the record index of override k
+    uint8_t g;                        // the gt of the record next() returned
+    __device__ __forceinline__ OverrideScan(int lo, int hi, int w0, int w1, bool snp, const OverrideParams& o, int k0,
+                                            int k1)
+        : sc(lo, hi, w0, w1, snp), idx(o.idx), gt(o.gt), k(k0), ke(k1), k_idx(k0 < k1 ? o.idx[k0] : -1) {}
+    __device__ __forceinline__ int next(const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_len,
+                                        const uint8_t* v_gt) {
+        while (sc.i < sc.hi) {
+            const int i = sc.i++;
+            g = v_gt[i];
+            if (i == k_idx) {
+                g = gt[k++];
+                k_idx = k < ke ? idx[k] : -1;
+            }
+            if (g != 0 && sc.take(v_pos[i], v_ref_len[i], v_alt_len[i])) return i;
+        }
+        return -1;
+    }
+};
+
 struct EncodeParams {
     const uint8_t* genome;            // concatenated chromosomes, 1 byte/base as in the FASTA (case kept)
     const int64_t* win_base;          // [n_win] offset of the window's chromosome in `genome`
@@ -119,16 +153,27 @@ struct EncodeParams {
     const uint8_t* alt_pool;
     uint8_t* out; int64_t pitch;      // [n_win, pitch]
     int32_t* out_len;                 // [n_win]
-    int32_t* err;                     // device error flag (1 = pitch overflow, 2 = too many variants, 4 = unsorted extras)
+    int32_t* err;                     // device error flag (1 = pitch overflow, 2 = too many variants, 4 = unsorted extras,
+                                      // 8 = malformed overrides)
 };
 
-// kEdit = false: vf_encode_windows.  kEdit = true: the same body over MergedScan; a tagged index (< -1) reads its extra
-// record wherever the plain kernel reads the table.
-template <bool kEdit>
-__global__ void __launch_bounds__(256)
-encode_windows_kernel(const EncodeParams p, const EditParams e) {
+// kPlain: vf_encode_windows.  kExtras: the same body over MergedScan; a tagged index (< -1) reads its extra record
+// wherever the plain kernel reads the table.  kOverrides: the same body over OverrideScan; an applied record's gt is the
+// one it was applied with, kept in s_gt beside its index.
+enum EncodeMode { kPlain, kExtras, kOverrides };
+template <int kMode> struct EncodeExtra { using type = EditParams; };
+template <> struct EncodeExtra<kOverrides> { using type = OverrideParams; };
+
+// (Launch bounds: minimum blocks 0 is "unspecified", the bound the plain and extras modes have always had; the
+// overrides mode asks for 5 blocks per SM, which lets ptxas keep it at 40 registers without the spill its default choice
+// of 32 registers makes.)
+template <int kMode>
+__global__ void __launch_bounds__(256, kMode == kOverrides ? 5 : 0)
+encode_windows_kernel(const EncodeParams p, const typename EncodeExtra<kMode>::type e) {
+    constexpr bool kEdit = kMode == kExtras, kOvr = kMode == kOverrides;
     __shared__ int32_t s_vidx[kMaxApplied];     // applied variant index
     __shared__ int32_t s_shift[kMaxApplied];    // cumulative (alt_len - ref_len) BEFORE this variant
+    __shared__ uint8_t s_gt[kMode == kOverrides ? kMaxApplied : 1];     // kOverrides: the applied gt (unused otherwise)
     __shared__ int s_n, s_total;
     const int w = blockIdx.y;
     const int w0 = p.w0[w], w1 = p.w1[w];
@@ -137,18 +182,31 @@ encode_windows_kernel(const EncodeParams p, const EditParams e) {
     const uint8_t fl = p.flags[w];
     const bool rc = fl & 1, snp_only = fl & 2;
     const auto X = [](int v) { return -2 - v; };            // tagged index -> extra record
-    const auto POS = [&](int v) { return kEdit && v < 0 ? e.pos[X(v)] : p.v_pos[v]; };
-    const auto RL = [&](int v) { return kEdit && v < 0 ? e.ref_len[X(v)] : p.v_ref_len[v]; };
-    const auto AL = [&](int v) { return kEdit && v < 0 ? e.alt_len[X(v)] : p.v_alt_len[v]; };
-    const auto ALT = [&](int v, int j) { return kEdit && v < 0 ? e.alt_pool[e.alt_off[X(v)] + j] : p.alt_pool[p.v_alt_off[v] + j]; };
-    const auto GT = [&](int v) { return kEdit && v < 0 ? (e.gt ? e.gt[X(v)] : (uint8_t)2) : p.v_gt[v]; };
+    // (if constexpr: OverrideParams has no extra records, so only the extras mode names them)
+    const auto POS = [&](int v) { if constexpr (kEdit) return v < 0 ? e.pos[X(v)] : p.v_pos[v]; else return p.v_pos[v]; };
+    const auto RL = [&](int v) {
+        if constexpr (kEdit) return v < 0 ? e.ref_len[X(v)] : p.v_ref_len[v]; else return p.v_ref_len[v];
+    };
+    const auto AL = [&](int v) {
+        if constexpr (kEdit) return v < 0 ? e.alt_len[X(v)] : p.v_alt_len[v]; else return p.v_alt_len[v];
+    };
+    const auto ALT = [&](int v, int j) {
+        if constexpr (kEdit) return v < 0 ? e.alt_pool[e.alt_off[X(v)] + j] : p.alt_pool[p.v_alt_off[v] + j];
+        else return p.alt_pool[p.v_alt_off[v] + j];
+    };
+    const auto GT = [&](int v, int k) {                     // record v, the k-th applied
+        if constexpr (kEdit) return v < 0 ? (e.gt ? e.gt[X(v)] : (uint8_t)2) : p.v_gt[v];
+        else if constexpr (kOvr) return s_gt[k];
+        else return p.v_gt[v];
+    };
     if (threadIdx.x == 0) {
         // sequential scan: which records are applied (overlap rule needs order) and where they land
         int n = 0, shift = 0, bad = 0;
         auto scan = [&](auto& sc) {
-            for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)), kEdit ? i != -1 : i >= 0;) {
+            for (int i; (i = sc.next(p.v_pos, p.v_ref_len, p.v_alt_len, p.v_gt)), kMode != kPlain ? i != -1 : i >= 0;) {
                 if (n == kMaxApplied) { bad = 2; break; }
                 if constexpr (kEdit) { if (i < 0 && blockIdx.x == 0) e.applied[X(i)] = 1; }
+                if constexpr (kOvr) s_gt[n] = sc.g;
                 s_vidx[n] = i; s_shift[n] = shift; ++n;
                 shift += AL(i) - RL(i);
             }
@@ -167,11 +225,25 @@ encode_windows_kernel(const EncodeParams p, const EditParams e) {
                 MergedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only, e, x0, x1);
                 scan(sc);
             }
+        } else if constexpr (kOvr) {
+            const int k0 = e.off[w], k1 = e.off[w + 1], lo = p.var_lo[w], hi = p.var_hi[w];
+            for (int k = k0; k < k1; ++k) {
+                const int i = e.idx[k];
+                if (i < lo || i >= hi || (k > k0 && i <= e.idx[k - 1])) bad = 8;
+            }
+            if (bad) {                                       // a malformed list is not applied: the row writes nothing
+                atomicMax(p.err, bad);
+                if (blockIdx.x == 0) p.out_len[w] = 0;
+                s_n = -1;
+            } else {
+                OverrideScan sc(lo, hi, w0, w1, snp_only, e, k0, k1);
+                scan(sc);
+            }
         } else {
             AppliedScan sc(p.var_lo[w], p.var_hi[w], w0, w1, snp_only);
             scan(sc);
         }
-        if (!(kEdit && bad == 4)) {
+        if (!((kEdit && bad == 4) || (kOvr && bad == 8))) {
             s_n = n; s_total = (w1 - w0) + shift;
             if (bad) atomicMax(p.err, bad);
             if (s_total > p.pitch) atomicMax(p.err, 1);
@@ -181,7 +253,7 @@ encode_windows_kernel(const EncodeParams p, const EditParams e) {
     }
     __syncthreads();
     const int n = s_n, total = s_total;
-    if (kEdit && n < 0) return;
+    if ((kEdit || kOvr) && n < 0) return;
     if (total > p.pitch) return;
     const uint8_t* ref = p.genome + p.win_base[w];
     uint8_t* out = p.out + (size_t)w * p.pitch;
@@ -210,7 +282,7 @@ encode_windows_kernel(const EncodeParams p, const EditParams e) {
         const int o0 = pos - w0 + s_shift[k];
         if (al == 1 && rl == 1) {
             uint8_t a = ALT(v, 0);
-            if (GT(v) == 1) {
+            if (GT(v, k) == 1) {
                 uint8_t r = ref[pos];
                 if (r >= 'a' && r <= 'z') r -= 32;
                 a = iupac_het(r, a);
@@ -241,7 +313,7 @@ int encode_windows(const uint8_t* genome, const int64_t* win_base, const int32_t
         EncodeParams p{genome, win_base + c0, w0 + c0, w1 + c0, var_lo + c0, var_hi + c0, flags + c0, v_pos, v_ref_len,
                        v_alt_off, v_alt_len, v_gt, alt_pool, out + (size_t)c0 * pitch, pitch, out_len + c0, err};
         dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n);
-        encode_windows_kernel<false><<<grid, 256, 0, s>>>(p, EditParams{});
+        encode_windows_kernel<kPlain><<<grid, 256, 0, s>>>(p, EditParams{});
         VF_LAUNCH_OK("encode_windows_kernel launch");
     }
     return 0;
@@ -270,7 +342,7 @@ static int encode_windows_extras(const char* what, const uint8_t* genome, const 
         if (e.off) ec.off = e.off + c0;
         else { ec.pos += c0; ec.ref_len += c0; ec.alt_off += c0; ec.alt_len += c0; ec.applied += c0; }
         dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n);
-        encode_windows_kernel<true><<<grid, 256, 0, s>>>(p, ec);
+        encode_windows_kernel<kExtras><<<grid, 256, 0, s>>>(p, ec);
         VF_LAUNCH_OK("encode_windows_kernel<edit> launch");
     }
     return 0;
@@ -301,6 +373,34 @@ int encode_windows_edits(const uint8_t* genome, const int64_t* win_base, const i
     return encode_windows_extras("encode_windows_edits", genome, win_base, w0, w1, var_lo, var_hi, flags, v_pos,
                                  v_ref_len, v_alt_off, v_alt_len, v_gt, alt_pool, e, n_win, max_window, out, pitch,
                                  out_len, err, s);
+}
+
+int encode_windows_overrides(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
+                             const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
+                             const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
+                             const uint8_t* v_gt, const uint8_t* alt_pool, const int32_t* o_off, const int32_t* o_idx,
+                             const uint8_t* o_gt, int n_win, int max_window, uint8_t* out, int64_t pitch,
+                             int32_t* out_len, int32_t* err, cudaStream_t s) {
+    const char* what = "encode_windows_overrides";
+    VF_REQUIRE(n_win >= 0, "%s: n_win %d < 0", what, n_win);
+    if (n_win == 0) return 0;
+    VF_REQUIRE(max_window > 0 && pitch >= max_window, "%s: pitch %lld < max window %d", what, (long long)pitch,
+               max_window);
+    VF_REQUIRE(genome && win_base && w0 && w1 && var_lo && var_hi && flags && v_pos && v_ref_len && v_alt_off &&
+               v_alt_len && v_gt && alt_pool, "%s: a window or variant array is NULL", what);
+    VF_REQUIRE(o_off && o_idx && o_gt, "%s: an override array is NULL", what);
+    VF_REQUIRE(out && out_len && err, "%s: out, out_len and err are required", what);
+    constexpr int kMaxWinPerLaunch = 65535;              // blockIdx.y limit, as encode_windows
+    for (int c0 = 0; c0 < n_win; c0 += kMaxWinPerLaunch) {
+        const int n = n_win - c0 < kMaxWinPerLaunch ? n_win - c0 : kMaxWinPerLaunch;
+        EncodeParams p{genome, win_base + c0, w0 + c0, w1 + c0, var_lo + c0, var_hi + c0, flags + c0, v_pos, v_ref_len,
+                       v_alt_off, v_alt_len, v_gt, alt_pool, out + (size_t)c0 * pitch, pitch, out_len + c0, err};
+        const OverrideParams o{o_off + c0, o_idx, o_gt};   // CSR offsets are global
+        dim3 grid((max_window + kEncSlice - 1) / kEncSlice, n);
+        encode_windows_kernel<kOverrides><<<grid, 256, 0, s>>>(p, o);
+        VF_LAUNCH_OK("encode_windows_kernel<overrides> launch");
+    }
+    return 0;
 }
 
 // ---------------------------------------------------------------------------------

@@ -66,6 +66,12 @@ int encode_windows_edits(const uint8_t* genome, const int64_t* win_base, const i
                          const int32_t* e_ref_len, const int32_t* e_alt_off, const int32_t* e_alt_len,
                          const uint8_t* e_gt, const uint8_t* e_alt_pool, int n_win, int max_window, uint8_t* out,
                          int64_t pitch, int32_t* out_len, uint8_t* applied, int32_t* err, cudaStream_t s);
+int encode_windows_overrides(const uint8_t* genome, const int64_t* win_base, const int32_t* w0, const int32_t* w1,
+                             const int32_t* var_lo, const int32_t* var_hi, const uint8_t* flags, const int32_t* v_pos,
+                             const int32_t* v_ref_len, const int32_t* v_alt_off, const int32_t* v_alt_len,
+                             const uint8_t* v_gt, const uint8_t* alt_pool, const int32_t* o_off, const int32_t* o_idx,
+                             const uint8_t* o_gt, int n_win, int max_window, uint8_t* out, int64_t pitch,
+                             int32_t* out_len, int32_t* err, cudaStream_t s);
 int window_genotype_keys(const int32_t* w0, const int32_t* w1, const int32_t* var_lo, const int32_t* var_hi,
                          const uint8_t* flags, const int32_t* v_pos, const int32_t* v_ref_len, const int32_t* v_alt_off,
                          const int32_t* v_alt_len, const uint8_t* v_gt, const uint8_t* alt_pool, int n_rows,

@@ -543,6 +543,44 @@ def encode_windows_edits(genome, win_base, w0, w1, var_lo, var_hi, flags, varian
     return out, out_len, applied[:m], err
 
 
+def encode_windows_overrides(genome, win_base, w0, w1, var_lo, var_hi, flags, variants, o_off, o_idx, o_gt, max_window,
+                             pitch, err=None):
+    """encode_windows with a list of genotype overrides per row (vf_encode_windows_overrides): row w owns the overrides
+    [o_off[w], o_off[w + 1]) (CSR), each a record index o_idx into the variant table (strictly increasing within the row,
+    inside [var_lo[w], var_hi[w])) and its new gt o_gt (0 removed, 1 het, 2 hom-alt), and encodes as encode_windows does
+    on the table with those gts replaced.  o_off int32 [n + 1]; o_idx int32 and o_gt uint8 [o_off[-1]]; device tensors.
+    -> (out uint8 [n, pitch], out_len int32 [n], err); err 8 (length 0, that row only) for a malformed row."""
+    n = w0.numel()
+    dev = genome.device
+    for t in (w0, w1, var_lo, var_hi):
+        assert t.dtype == torch.int32 and t.numel() == n and t.is_contiguous()
+    assert win_base.dtype == torch.int64 and flags.dtype == torch.uint8
+    off = o_off.cpu().numpy()
+    if o_off.dtype != torch.int32 or off.shape != (n + 1,) or off[0] != 0 or (np.diff(off) < 0).any():
+        raise ValueError(f"o_off must be int32 [{n + 1}] offsets from 0, nondecreasing (got {o_off.dtype} "
+                         f"{tuple(off.shape)})")
+    m = int(off[-1])
+    for t, dt in ((o_idx, torch.int32), (o_gt, torch.uint8)):
+        if t.dtype != dt or t.numel() != m or not t.is_contiguous():
+            raise ValueError(f"override arrays must be contiguous {dt} [{m}] (o_off[-1]), got {t.dtype} [{t.numel()}]")
+    if m and int(o_gt.max()) > 2:
+        raise ValueError(f"o_gt must be 0, 1 or 2 (got {int(o_gt.max())})")
+    # kernels need non-NULL arrays; the tensors stay referenced by the caller until the launch is enqueued
+    o = [o_off.to(dev)] + [t if t.numel() else torch.zeros(1, dtype=t.dtype, device=dev) for t in (o_idx, o_gt)]
+    out = torch.empty((n, pitch), dtype=torch.uint8, device=dev)
+    out_len = torch.empty(n, dtype=torch.int32, device=dev)
+    if err is None:
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+    v = variants
+    with _timed("stage1_encode_overrides", nbytes=float(n) * max_window * 2):   # window bytes read + written (upper bound)
+        check(_lib.lib().vf_encode_windows_overrides(ptr(genome), ptr(win_base), ptr(w0), ptr(w1), ptr(var_lo),
+                                                     ptr(var_hi), ptr(flags), ptr(v["pos"]), ptr(v["ref_len"]),
+                                                     ptr(v["alt_off"]), ptr(v["alt_len"]), ptr(v["gt"]),
+                                                     ptr(v["alt_pool"]), *[ptr(t) for t in o], n, int(max_window),
+                                                     ptr(out), int(pitch), ptr(out_len), ptr(err), stream()))
+    return out, out_len, err
+
+
 def _genotype_rows(w0, w1, var_lo, var_hi, flags, variants):
     n = w0.numel()
     for t in (w0, w1, var_lo, var_hi):

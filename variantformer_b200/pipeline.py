@@ -221,6 +221,16 @@ class HotPath:
         from .variant_sets import scan
         return scan(self, genes, sets, variants, embeddings=embeddings, to_host=to_host, **kw)
 
+    def genotype_edits(self, genes, sets, variants: SampleVariants, embeddings=False, to_host=True, **kw):
+        """Variant attribution (variant_attribution.scan): sets[i] = list of sets for gene i, each a list of
+        variant_attribution.Edit(chrom, pos (1-based), ref, alt, gt=0) naming a record of the sample `variants` and its
+        new GT (0 removed, 1 het, 2 hom-alt).  -> (pred [sum T], emb [sum T, D]) of the baseline, bit-identical to
+        predict(genes, variants), per gene the set predictions [n, T] (+ per gene [n, T, D] embeddings when
+        `embeddings`), each bit-identical to predict with the records' GTs replaced in the sample's table, and per gene
+        the changed windows dict(cre=bool [n, C] in batch order, gene=bool [n], records=per set bool [len(set)])."""
+        from .variant_attribution import scan
+        return scan(self, genes, sets, variants, embeddings=embeddings, to_host=to_host, **kw)
+
     def cohort_variant_sets(self, genes, sets, cohort, sample_idx=None, embeddings=False, to_host=True, **kw):
         """Variant sets across a cohort (cohort_sets.scan): every set of variant_sets' form in every sample of a cohort
         (stage1.CohortVariants; sample_idx: which of its samples, default all), each distinct edited window encoded

@@ -474,6 +474,73 @@ class VCFProcessor:
             return pd.DataFrame(columns=["sample"] + vs.SET_COLUMNS)
         return pd.concat(frames, ignore_index=True)
 
+    def variant_attribution(self, vcf_path: str, query_df: pd.DataFrame, edits: pd.DataFrame = None, scope="record"):
+        """Variant attribution (DESIGN.md section 19): every query row predicted with some of its sample's own records
+        removed or re-genotyped, each window no edit lies in encoded once.  A set's prediction equals what create_data +
+        predict give on the sample's VCF with those lines removed (GT 0) or their GT rewritten.  The query is filtered
+        with VCFDataset's rules; the sample is `vcf_path` or a per-row vcf_path column.  edits: None = the default scan,
+        scope "record" (leave-one-out: each record of the sample whose REF span lies in one of the gene's windows and
+        whose GT is not 0, removed singly) or "window" (each window holding such records reverted to the reference); or
+        a DataFrame with columns gene_id, chromosome, pos (1-based), ref, alt, gt (the new GT: 0, 1 or 2) and
+        optionally set (a label; one set per row without it) and label.  Invalid edits raise a ValueError before the
+        model is loaded.  A row whose sample has no record in the gene's windows gives no rows.  Writes no file.
+        -> one row per (query row, set, tissue), in that order, columns variant_attribution.ATTRIBUTION_COLUMNS:
+        variant_sets.SET_COLUMNS (changed: a window's tokens differ from the baseline's), sample_gt and new_gt
+        (single-record sets), reference_expression (every record in the gene's windows removed) and delta =
+        predicted - baseline (a removed record contributes -delta)."""
+        from .. import variant_attribution as va
+        from ..pipeline import HotPath
+        if scope not in va.SCOPES:
+            raise ValueError(f"scope must be one of {va.SCOPES}, got {scope!r}")
+        user = va.user_edits(edits) if edits is not None else None
+        dataset, q, genes, paths = self._edit_query(vcf_path, query_df)
+        gene_ids = list(q["gene_id"])
+        if user is not None:
+            for gid in user:
+                if gid not in set(gene_ids):
+                    print(f"Gene {gid} of the edits is not in the query so skipping it")
+        ds = self.model_config.dataset
+        nb, up, down = ds.cre_neighbour_hood, ds.gene_upstream_neighbour_hood, ds.gene_downstream_neighbour_hood
+        genome = dataset._genome()
+        todo = []                                            # (row, sets incl. the all-removed one last, labels, gts)
+        for i, (g, gid, p) in enumerate(zip(genes, gene_ids, paths)):
+            v = dataset._variants(p)
+            ref = va.all_removed(g, v, nb, up, down)
+            if user is not None:
+                us = user.get(gid, [])
+                sets = va.check_edits([g], [[es for _, es, _ in us]], v, [gid])[0]
+                labels = [sid for sid, _, _ in us]
+                gts = [va.sample_gt(v, s[0]) if len(s) == 1 else None for s in sets]
+            else:
+                if not ref:
+                    continue
+                sets, labels, gts = va.default_sets(g, v, nb, up, down, scope, genome)
+            if sets:
+                todo.append((i, sets + [ref], labels, gts))
+        frames = []
+        if todo:
+            model, _, _ = self.load_model()
+            hot = HotPath(model.engine(), genome, max_length=ds.max_length, max_chunks=ds.max_chunks,
+                          cre_neighbour_hood=nb, gene_upstream=up, gene_downstream=down)
+            res = {}
+            for p in dict.fromkeys(paths[t[0]] for t in todo):   # one call per sample, in first-appearance order
+                part = [t for t in todo if paths[t[0]] == p]
+                pred, _, s_pred, app = va.run(hot, [genes[t[0]] for t in part], [t[1] for t in part],
+                                              dataset._variants(p), min_gene_len=1000,
+                                              gene_names=[gene_ids[t[0]] for t in part])
+                off = np.concatenate([[0], np.cumsum([len(genes[t[0]].tissues) for t in part])])
+                for k, t in enumerate(part):
+                    res[t[0]] = (pred[off[k]:off[k + 1]], s_pred[k], app[k])
+            for i, sets, labels, gts in todo:
+                base, sp, ap = res[i]
+                n = len(labels)
+                ap = dict(cre=ap["cre"][:n], gene=ap["gene"][:n], records=ap["records"][:n])
+                frames.append(va.attribution_frame(gene_ids[i], list(q["tissue_names"].iloc[i]), labels, sets[:n], gts,
+                                                   ap, base, sp[:n], sp[n]))
+        if not frames:
+            return pd.DataFrame(columns=va.ATTRIBUTION_COLUMNS)
+        return pd.concat(frames, ignore_index=True)
+
     def variant_interactions(self, vcf_path: str, query_df: pd.DataFrame, variants: pd.DataFrame):
         """Pairwise interaction scan (DESIGN.md section 17): for every query row, each of its gene's variants singly and
         every unordered pair of them added to the sample, all in one planner call per sample.  Query and sample as

@@ -105,6 +105,8 @@ class SampleVariants:
 
     def __init__(self, per_chrom: dict, device="cuda"):
         self.ranges, self.host_pos = {}, {}
+        # host copies of the rest of each record (variant attribution names a sample's own records by them)
+        self.host_ref_len, self.host_alt, self.host_gt = {}, {}, {}
         pos, rl, ao, al, gt, pool = [], [], [], [], [], []
         n = 0; pool_len = 0
         for chrom, v in per_chrom.items():
@@ -116,6 +118,8 @@ class SampleVariants:
             ao.append((np.cumsum(lens) - lens + pool_len).astype(np.int32)); gt.append(np.asarray(v["gt"], np.uint8))
             pool.append(np.frombuffer(b"".join(alts), np.uint8)); pool_len += int(lens.sum())
             self.ranges[chrom] = (n, n + len(p)); self.host_pos[chrom] = p; n += len(p)
+            self.host_ref_len[chrom] = rl[-1].astype(np.int64); self.host_alt[chrom] = alts
+            self.host_gt[chrom] = gt[-1].copy()
 
         def cat(xs, dt):
             return torch.from_numpy(np.concatenate(xs).astype(dt) if xs else np.zeros(0, dt)).to(device)

@@ -203,10 +203,13 @@ def scan(hot, genes, sets, variants=None, embeddings=False, to_host=True, rows_b
 
 
 def plan(hot, genes, sets, variants, embeddings, to_host, rows_budget, pass_rows, timer, counters, min_gene_len, names,
-         encode=None):
-    """The edited-window planner behind scan() and deletion.deletion_scan: sets as check_sets returns them (validated);
-    encode(hot, variants, rows, pitch) -> (out, out_len, applied per record, err) encodes rows [(chrom, w0, w1, flags,
-    records)] (default _encode_sets, looked up at call time)."""
+         encode=None, changed_by_tokens=False):
+    """The edited-window planner behind scan(), deletion.deletion_scan and variant_attribution.scan: sets as check_sets
+    returns them (validated; a record is a tuple whose first three fields are (chrom, pos0, ref_len), the rest is the
+    encoder's); encode(hot, variants, rows, pitch) -> (out, out_len, applied per record, err) encodes rows [(chrom, w0,
+    w1, flags, records)] (default _encode_sets, looked up at call time).  changed_by_tokens: a window counts as changed
+    when its token row (CRE) or chunk list (gene) differs from the baseline's, and a record as applied when a window
+    holding it changed (the encoder's applied flags are not read); otherwise the encoder's applied flags decide."""
     encode = encode if encode is not None else _encode_sets
     eng, dev = hot.engine, hot.engine.device
     phase = timer or (lambda name: contextlib.nullcontext())
@@ -341,13 +344,19 @@ def plan(hot, genes, sets, variants, embeddings, to_host, rows_budget, pass_rows
                     for k, ms in hits[gi][j].items():
                         kk = key(gi, j, k)
                         row = keys[kk][0]
-                        flags = (g_app if kk[0] else c_app)[a_off[kk[0]][row]:a_off[kk[0]][row + 1]]
-                        ap["records"][j][ms] |= flags
                         if kk[0]:
                             grow = inv_g[g_start[row]:g_start[row + 1]]
-                            ap["gene"][j] = flags.any()
                         else:
                             r[k] = inv_c[n_cb + row]
+                        if changed_by_tokens:
+                            ch = not np.array_equal(grow, gr) if kk[0] else bool(r[k] != cr[k])
+                            flags = np.full(len(ms), ch)
+                        else:
+                            flags = (g_app if kk[0] else c_app)[a_off[kk[0]][row]:a_off[kk[0]][row + 1]]
+                        ap["records"][j][ms] |= flags
+                        if kk[0]:
+                            ap["gene"][j] = flags.any()
+                        else:
                             ap["cre"][j, k] = flags.any()
                     items.append((r, grow, tis, lab))
                 n_set = len(sets[gi])
